@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- theta-rrt planning inner loop on B200: RRT expansions/s (+ LOS checks/s, Theta* expansions/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[2], SURVEY.md 8d cfg 3): batched RRT, 4096 independent
 queries per GPU on map1 (100x100), K=5001 (5000 expansions each), tol_xy=0 so every query runs all
@@ -27,6 +27,10 @@ The single JSON line carries
 line's value) and the unmodified Python sources, one process and one per core, when oracle/_ref is
 present.  Multi-GPU (torchrun, one rank per GPU): queries are sharded by rank, no data-path collective;
 a gather of the per-query summaries over NCCL closes each step ("scaling": "weak").
+
+--dump-outputs DIR writes what the last timed step of the headline workload returned (rank 0's queries) as float64
+.npy files in DIR (dump_outputs).  The inputs are seeded, so two builds run with the same arguments can be compared
+file for file.
 """
 from __future__ import annotations
 
@@ -47,6 +51,7 @@ NQ_PER_GPU = 4096
 K_RRT = 5001
 MAP_SEED = 1234
 K_PYREF = 601  # the Python reference is timed on the first 600 iterations of a query per process (about 10 s)
+DUMP_TREES = 96  # --dump-outputs: trees of 96 queries are at most 96 x K_RRT rows x 112 B = 54 MB
 WORKLOAD = ("cfg3: batched RRT, %d independent queries per GPU on map1.png (100x100), K=%d "
             "(5000 expansions each), tol_xy=0, seeded rand_conf streams")
 
@@ -340,6 +345,34 @@ def check_parity(free, starts, goals, sxy, sth, K, res, n):
             "fields": "n_nodes, status, iters, sol, parent, node_x/y/theta (bit patterns)", "result": "identical"}
 
 
+def dump_outputs(out_dir, res, first_query):
+    """What one Planner.rrt call returned, as float64 .npy files in out_dir:
+      n_nodes, sol, status, iters         [q]      every query of the call
+      queries                             [s]      ids of DUMP_TREES queries drawn with default_rng(0), ascending
+      node_x, node_y, node_theta, parent  [rows]   tree rows 0 .. n_nodes-1 of those queries, concatenated in the
+      u, u_nan                            [rows,5] order of `queries` (rows past n_nodes are never written)
+    u holds 0 where the kernel returns NaN (the root row, icc and rad of a straight edge) and u_nan is 1 there, so that
+    equal outputs compare equal without NaN-aware comparisons.  The per-query arrays take 32 B a query; a B200 cannot
+    hold the outputs of enough queries to take them past 16 MB."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    out = {k: getattr(res, k).cpu().numpy().astype(np.float64) for k in ("n_nodes", "sol", "status", "iters")}
+    nq = len(out["n_nodes"])
+    pick = np.sort(np.random.default_rng(0).choice(nq, size=min(DUMP_TREES, nq), replace=False))
+    idx = torch.from_numpy(pick).to(res.node_x.device)
+    n = out["n_nodes"][pick].astype(np.int64)
+    for k in ("node_x", "node_y", "node_theta", "parent", "u"):
+        a = getattr(res, k)[idx].cpu().numpy()
+        out[k] = np.concatenate([a[j, :n[j]] for j in range(len(pick))]).astype(np.float64)
+    out["u_nan"] = np.isnan(out["u"]).astype(np.float64)
+    out["u"][out["u_nan"] == 1] = 0.0
+    out["queries"] = (first_query + pick).astype(np.float64)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+    mb = sum(v.nbytes for v in out.values()) / 2**20
+    print(f"bench: {len(out)} output arrays ({mb:.1f} MiB) written to {out_dir}", file=sys.stderr)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -354,7 +387,12 @@ def main():
     ap.add_argument("--skip-secondary", action="store_true")
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-python-ref", action="store_true", help="do not time the Python reference (about 30 s of CPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -433,6 +471,8 @@ def main():
     parity = None
     if rank == 0 and not args.skip_cpu:
         parity = check_parity(free, starts, goals, sxy, sth, K, keep["res"], min(64, hi - lo))
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, keep["res"], lo)
 
     # ---- roofline of the fused kernel (this rank's launch)
     alg_bytes = 16 * int(counters[0]) + 16 * iters_total + (28 + 40) * n_nodes_total

@@ -21,7 +21,7 @@ def pytest_configure(config):
         from theta_rrt_b200 import _lib
         _lib.SO_PATH = os.path.abspath(so)
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "reference: needs the read-only reference tree at /root/reference")
+    config.addinivalue_line("markers", "reference: needs the unmodified eshira/theta-rrt sources (directory in THETA_RRT_REFERENCE)")
 
 
 def pytest_collection_modifyitems(config, items):
@@ -30,12 +30,13 @@ def pytest_collection_modifyitems(config, items):
         has_gpu = torch.cuda.is_available()
     except Exception:
         has_gpu = False
-    have_ref = os.path.isfile("/root/reference/search.py")
+    from oracle import live_reference
+    have_ref = live_reference.available()
     for item in items:
         if "gpu" in item.keywords and not has_gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))
         if "reference" in item.keywords and not have_ref:
-            item.add_marker(pytest.mark.skip(reason="reference tree not present"))
+            item.add_marker(pytest.mark.skip(reason="eshira/theta-rrt sources not found (set THETA_RRT_REFERENCE)"))
 
 
 @pytest.fixture(scope="session")

@@ -64,3 +64,40 @@ def test_reference_arm_line_without_python_reference(monkeypatch, capsys):
     assert line["value"] > 0 and line["e2e"]["value"] == line["value"]
     bench.run_reference_arm(args, rank=1, world=2)  # other ranks print nothing
     assert capsys.readouterr().out == ""
+
+
+def test_dump_outputs_writes_valid_tree_rows_of_a_fixed_sample(tmp_path):
+    import torch
+    from theta_rrt_b200.planner import RrtResult
+    nq, K = 300, 9
+    rng = np.random.default_rng(1)
+    n = rng.integers(1, K + 1, nq)
+    f = lambda *s: torch.from_numpy(rng.normal(size=s))  # noqa: E731
+    i = lambda *s: torch.from_numpy(rng.integers(-1, K, size=s).astype(np.int32))  # noqa: E731
+    res = RrtResult(K=K, node_x=f(nq, K), node_y=f(nq, K), node_theta=f(nq, K), parent=i(nq, K),
+                    n_nodes=torch.from_numpy(n.astype(np.int32)), sol=i(nq), status=i(nq), iters=i(nq), u=f(nq, K, 5))
+    res.u[:, 0] = float("nan")  # root rows
+    res.u[::3, 1:, 1:4] = float("nan")  # straight edges
+    bench.dump_outputs(str(tmp_path / "a"), res, 1000)
+    bench.dump_outputs(str(tmp_path / "b"), res, 1000)
+    names = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert names == sorted(k + ".npy" for k in ("n_nodes", "sol", "status", "iters", "queries", "node_x", "node_y", "node_theta",
+                                                "parent", "u", "u_nan"))
+    d = {p[:-4]: np.load(tmp_path / "a" / p) for p in names}
+    assert all(v.dtype == np.float64 and np.array_equal(v, np.load(tmp_path / "b" / (k + ".npy"))) for k, v in d.items())
+    assert np.array_equal(d["n_nodes"], n) and np.array_equal(d["status"], res.status.numpy())
+    q = d["queries"].astype(np.int64) - 1000
+    assert len(q) == bench.DUMP_TREES and np.all(np.diff(q) > 0)
+    rows = np.concatenate([np.stack([np.full(n[j], j), np.arange(n[j])], 1) for j in q])
+    assert len(d["node_x"]) == len(rows) == n[q].sum() and d["u"].shape == d["u_nan"].shape == (len(rows), 5)
+    for k in ("node_x", "node_y", "node_theta", "parent"):
+        assert np.array_equal(d[k], getattr(res, k).numpy()[rows[:, 0], rows[:, 1]]), k
+    u = res.u.numpy()[rows[:, 0], rows[:, 1]]
+    assert d["u_nan"].sum() > 0 and np.array_equal(d["u_nan"] == 1, np.isnan(u))
+    assert np.array_equal(d["u"], np.where(np.isnan(u), 0.0, u))
+
+
+def test_bench_rejects_zero_steps_and_dump_of_the_reference_arm():
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "x"]):
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True)
+        assert p.returncode == 2 and "error" in p.stderr, extra
