@@ -30,8 +30,6 @@ def run(label, **kw):
 
 run("rows  (one thread per ray)", layout="rows")
 run("tiles default", layout="tiles")
-# (the lanes / rays-per-warp / refill / cooperative-tail knobs are compile-time now: -DTRRT_LOS_LANES, -DTRRT_LOS_RPW,
-#  -DTRRT_LOS_REFILL, -DTRRT_LOS_COOP; build a variant with profiles/tools/variant_bench.py to sweep them)
 # sorted by length (what a caller could do for the rows kernel): upper bound on what refill can recover
 px = np.maximum(np.abs(seg[:, 2] - seg[:, 0]), np.abs(seg[:, 3] - seg[:, 1]))
 d_seg = torch.from_numpy(np.ascontiguousarray(seg[np.argsort(px)])).to(dev); ref = None

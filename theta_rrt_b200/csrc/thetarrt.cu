@@ -3,7 +3,6 @@
 // Kernels (one section each):
 //   pack_grid_kernel      byte image -> bit-packed occupancy grid
 //   los_batch_kernel      K4: search.lineofsight for independent segments, one thread per ray
-//   los_group_kernel<G>       same, G lanes per ray (optional)
 //   tile_grid_kernel / los_tiled_kernel  K4b: the same test, 8 pixels per step over 8x16-pixel strips, per-lane refill (trrt_los.cuh)
 //   nearest_tile_kernel   K1: fp64 argmin over SoA tree; query sets in registers, node slices per warp
 //                             (the last CTA of a query group folds the per-column partials, lowest-index ties)
@@ -123,49 +122,6 @@ __global__ void __launch_bounds__(256) los_batch_kernel(const uint32_t *__restri
         }
     }
     out[i] = ok ? 1 : 0;
-}
-
-// K4, group version: G lanes share one segment.  Lane l tests pixels l, l+G, l+2G, ... of the line; the minor-axis
-// offset of pixel i is floor((2*dmin*i + dmaj - 1) / (2*dmaj)) (DESIGN.md 8.1), advanced by G pixels per step with
-// a quotient/remainder pair, so there is one division per segment, not per pixel.  Rays in a batch differ wildly in
-// length and most are blocked after a few pixels: with one thread per ray a warp runs at ~8 active lanes, with 8
-// lanes per ray the early exit frees all 8 at once.
-template <int G>
-__global__ void __launch_bounds__(256) los_group_kernel(const uint32_t *__restrict__ bits, int H, int W, int wpr, const int32_t *__restrict__ map_id,
-                                                        const int4 *__restrict__ seg, int64_t n, uint8_t *__restrict__ out) {
-    const Group<G> g;
-    const int64_t i = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) / G;
-    if (i >= n) return; // whole groups leave together
-    const int4 s4 = __ldg(seg + i);
-    int x0 = s4.x, y0 = s4.y, x1 = s4.z, y1 = s4.w;
-    const uint32_t *gm = bits + (map_id ? (size_t)__ldg(map_id + i) * H * wpr : 0);
-    bool ok = x0 >= 0 && y0 >= 0 && x1 >= 0 && y1 >= 0 && x0 < H && x1 < H && y0 < W && y1 < W; // search.py:17-24
-    if (ok) {
-        const int adx = abs(x1 - x0), ady = abs(y1 - y0);
-        const bool low = ady < adx; // search.py:47
-        if (low ? (x0 > x1) : (y0 > y1)) { int t = x0; x0 = x1; x1 = t; t = y0; y0 = y1; y1 = t; }
-        const unsigned dmaj = low ? adx : ady, dmin = low ? ady : adx;
-        const int step = low ? ((y1 < y0) ? -1 : 1) : ((x1 < x0) ? -1 : 1);
-        const int a0 = low ? x0 : y0, b0 = low ? y0 : x0;
-        const unsigned den = dmaj ? 2u * dmaj : 1u;
-        const unsigned num0 = 2u * dmin * (unsigned)g.gl + dmaj - (dmaj ? 1u : 0u);
-        unsigned sm = num0 / den, rem = num0 - sm * den;
-        const unsigned inc = 2u * dmin * (unsigned)G, q = inc / den, r = inc - q * den;
-        for (unsigned base = 0;; base += G) {
-            const unsigned k = base + (unsigned)g.gl;
-            bool blocked = false;
-            if (k <= dmaj) {
-                const int a = a0 + (int)k, b = b0 + step * (int)sm;
-                const int px = low ? a : b, py = low ? b : a;
-                blocked = !((__ldg(gm + (size_t)py * wpr + (px >> 5)) >> (px & 31)) & 1u);
-            }
-            if (g.any(blocked)) { ok = false; break; }
-            if (base + G > dmaj) break;
-            sm += q; rem += r;
-            if (rem >= den) { rem -= den; sm++; }
-        }
-    }
-    if (g.gl == 0) out[i] = ok ? 1 : 0;
 }
 
 // ===========================================================================
@@ -537,27 +493,19 @@ __device__ __forceinline__ bool hless(double f1, unsigned c1, double f2, unsigne
 // The open list is a G-ary heap (G = lanes of the group): node i has children G*i+1 .. G*i+G.  A pop descends
 // log_G(size) levels (3 for the 2 800 entries of the map2 query with G = 32) and at each level the G children are
 // read with one coalesced load and reduced with shuffles, instead of the ~12 dependent compare-and-swap rounds one
-// lane would spend in a binary heap.  Pushes climb at most the same levels (leader only).  The top three levels
-// (1 + G + G*G entries, 12.7 KB per query for G = 32) live in SHARED memory as SoA (f[], cell[]); deeper levels spill
-// to the global workspace.  Level boundaries coincide with the shared/global boundary, so one level of children is
-// entirely on one side.  Any correct min-heap on the total order (f, cell) pops in the reference's PriorityQueue
-// order (search.py:231,249).
-#ifndef TRRT_THETA_SMEM_HEAP
-#define TRRT_THETA_SMEM_HEAP 0 /* measured on B200: L1-resident global heap 241 ms vs shared top levels 292 ms (2048 map2 queries) */
-#endif
+// lane would spend in a binary heap.  Pushes climb at most the same levels (leader only).  The whole heap lives in the
+// query slot's part of the global workspace, one 16-byte entry per position; its top levels stay resident in L1.
+// Keeping the top three levels (1 + G + G*G entries) in shared memory instead was measured slower on B200: 292 ms
+// vs 241 ms for 2048 map2 queries.  Any correct min-heap on the total order (f, cell) pops in the reference's
+// PriorityQueue order (search.py:231,249).
 template <int G>
 struct Heap {
-    static constexpr int SCAP = TRRT_THETA_SMEM_HEAP ? 1 + G + G * G : 0;
-    double *sf;    // shared
-    unsigned *sc;  // shared
-    HeapEnt *gh;   // global, indexed by heap position (the first SCAP slots are unused)
+    HeapEnt *gh; // indexed by heap position
     __device__ __forceinline__ void get(int i, double &f, unsigned &c) const {
-        if (SCAP > 0 && i < SCAP) { f = sf[i]; c = sc[i]; }
-        else { HeapEnt e = gh[i]; f = e.f; c = e.c; }
+        HeapEnt e = gh[i]; f = e.f; c = e.c;
     }
     __device__ __forceinline__ void put(int i, double f, unsigned c) const {
-        if (SCAP > 0 && i < SCAP) { sf[i] = f; sc[i] = c; }
-        else { HeapEnt e; e.f = f; e.c = c; e.pad = 0; gh[i] = e; }
+        HeapEnt e; e.f = f; e.c = c; e.pad = 0; gh[i] = e;
     }
 };
 
@@ -629,15 +577,8 @@ __global__ void __launch_bounds__(128) theta_kernel(const ThetaDev a) {
     const bool lead = g.gl == 0;
     const int W = a.W, H = a.H;
     Cell *cells = a.cells + (size_t)slot * H * W;
-    extern __shared__ __align__(16) unsigned char theta_smem[];
     Heap<G> heap;
-    {
-        constexpr int groups = 128 / G, SC = Heap<G>::SCAP;
-        const int gi = threadIdx.x / G;
-        heap.sf = reinterpret_cast<double *>(theta_smem) + gi * SC;
-        heap.sc = reinterpret_cast<unsigned *>(reinterpret_cast<double *>(theta_smem) + groups * SC) + gi * SC;
-        heap.gh = a.heap + (size_t)slot * a.heap_cap;
-    }
+    heap.gh = a.heap + (size_t)slot * a.heap_cap;
     const int base_lane = (threadIdx.x & 31) & ~(G - 1);
     // neighbour j = node - delta_j, delta in itertools.product([-1,0,1], repeat=2) minus (0,0)  (search.py:187-189)
     const int j = g.gl & 7;
@@ -891,21 +832,11 @@ int trrt_los_batch(const uint32_t *d_bits, int n_maps, int H, int W, const int32
     if (n < 0 || !d_bits || (n > 0 && (!d_seg || !d_out))) return TRRT_ERR_INVALID_ARGUMENT;
     if (n == 0) return TRRT_OK;
     if (((uintptr_t)d_seg & 15) != 0) return TRRT_ERR_INVALID_ARGUMENT;
-    // lanes per segment: 1 = one thread per ray (literal Bresenham).  Measured on the cfg-4 rays (2^20 rays of 1..512 px,
-    // 88% blocked): 1 lane 232 us, 8 lanes 231 us, 16 lanes 208 us, 32 lanes 253 us; short clear rays (Theta*) favour 1.
-    // Experiment builds pick another width with -DTRRT_LOS_LANES=n; the library itself reads no environment.
-#ifndef TRRT_LOS_LANES
-#define TRRT_LOS_LANES 1
-#endif
-    const int wpr = (W + 31) / 32;
-    cudaStream_t st = (cudaStream_t)stream;
-    const int4 *sg = (const int4 *)d_seg;
-    const unsigned blocks = (unsigned)((n * TRRT_LOS_LANES + 255) / 256);
-#if TRRT_LOS_LANES > 1
-    los_group_kernel<TRRT_LOS_LANES><<<blocks, 256, 0, st>>>(d_bits, H, W, wpr, d_map_id, sg, n, d_out);
-#else
-    los_batch_kernel<<<blocks, 256, 0, st>>>(d_bits, H, W, wpr, d_map_id, sg, n, d_out); // one thread per segment
-#endif
+    // One thread per ray (literal Bresenham).  G lanes per ray were measured on the cfg-4 rays (2^20 rays of 1..512 px,
+    // 88% blocked): 1 lane 232 us, 8 lanes 231 us, 16 lanes 208 us, 32 lanes 253 us; short clear rays (Theta*) favour 1,
+    // and this rows layout is only the comparison arm of the strip kernel (trrt_los_batch_tiled).
+    const unsigned blocks = (unsigned)((n + 255) / 256);
+    los_batch_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(d_bits, H, W, (W + 31) / 32, d_map_id, (const int4 *)d_seg, n, d_out);
     CUDA_TRY(cudaGetLastError());
     return TRRT_OK;
 }
@@ -940,25 +871,15 @@ int trrt_los_batch_tiled(const uint64_t *d_tiles, int n_maps, int H, int W, cons
     // 256 segments per warp when that still gives every SM 24 warps, never fewer than 64.  Measured on the cfg-4 rays:
     // rpw 96 .. 256 -> 73 .. 71 us; refill threshold 6 / 8 / 12 idle lanes -> 72.6 / 70.6 / 70.8 us; cooperative tail
     // from 4 / 8 / 16 remaining rays -> 72.4 / 70.6 / 70.7 us, without it 87 us.
-    // (experiment builds override these with -D; the library itself reads no environment)
-#ifndef TRRT_LOS_REFILL
-#define TRRT_LOS_REFILL 8
-#endif
-#ifndef TRRT_LOS_COOP
-#define TRRT_LOS_COOP 8
-#endif
-    const int refill_min = TRRT_LOS_REFILL, coop_max = TRRT_LOS_COOP;
+    const int refill_min = 8, coop_max = 8;
     const long long target_warps = (long long)sm_count() * 24;
     long long rpw = ((n + target_warps - 1) / target_warps + 31) / 32 * 32;
     if (rpw < 64) rpw = 64;
     if (rpw > 256) rpw = 256;
-#ifdef TRRT_LOS_RPW
-    rpw = TRRT_LOS_RPW;
-#endif
     const long long warps = (n + rpw - 1) / rpw;
-    const unsigned blocks = (unsigned)((warps + TRRT_LOS_WARPS - 1) / TRRT_LOS_WARPS);
-    los_tiled_kernel<<<blocks, TRRT_LOS_WARPS * 32, 0, (cudaStream_t)stream>>>((const uint4 *)d_tiles, H, (W + 7) / 8, d_map_id, (const int4 *)d_seg,
-                                                                               (long long)n, (int)rpw, refill_min, coop_max, d_out);
+    const unsigned blocks = (unsigned)((warps + LOS_WARPS - 1) / LOS_WARPS);
+    los_tiled_kernel<<<blocks, LOS_WARPS * 32, 0, (cudaStream_t)stream>>>((const uint4 *)d_tiles, H, (W + 7) / 8, d_map_id, (const int4 *)d_seg,
+                                                                          (long long)n, (int)rpw, refill_min, coop_max, d_out);
     CUDA_TRY(cudaGetLastError());
     return TRRT_OK;
 }
@@ -1099,7 +1020,7 @@ int trrt_rrt_batch(const trrt_rrt_args *args, void *stream) {
         }
     } else if (A.schedule == 0) { // speculative window of G iterations, persistent groups
         const size_t smem = 0;
-        threads = TRRT_SPEC_THREADS;
+        threads = SPEC_THREADS;
         blocks = (A.n_queries * G + threads - 1) / threads;
         CUDA_TRY(cudaMemsetAsync(d.next_query, 0, sizeof(unsigned long long), st));
         const void *fn = nullptr;
@@ -1277,15 +1198,10 @@ int trrt_theta_batch(const trrt_theta_args *args, void *stream) {
     CUDA_TRY(cudaMemsetAsync(w, 0, 256 + theta_cells_bytes(&A), st));
     const int threads = 128;
     int64_t blocks = ((int64_t)A.n_slots * G + threads - 1) / threads;
-    // shared memory: the top three heap levels of every group of the CTA, 12 bytes per entry
-    const size_t smem = TRRT_THETA_SMEM_HEAP ? (size_t)(threads / G) * (size_t)(1 + G + G * G) * 12 : 0;
     switch (G) {
-    case 8: theta_kernel<8><<<(unsigned)blocks, threads, smem, st>>>(d); break;
-    case 16: theta_kernel<16><<<(unsigned)blocks, threads, smem, st>>>(d); break;
-    default:
-        CUDA_TRY(cudaFuncSetAttribute(theta_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        theta_kernel<32><<<(unsigned)blocks, threads, smem, st>>>(d);
-        break;
+    case 8: theta_kernel<8><<<(unsigned)blocks, threads, 0, st>>>(d); break;
+    case 16: theta_kernel<16><<<(unsigned)blocks, threads, 0, st>>>(d); break;
+    default: theta_kernel<32><<<(unsigned)blocks, threads, 0, st>>>(d); break;
     }
     CUDA_TRY(cudaGetLastError());
     return TRRT_OK;

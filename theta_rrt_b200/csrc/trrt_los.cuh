@@ -120,13 +120,8 @@ __device__ __forceinline__ unsigned strip_block(const uint4 *__restrict__ gtn, i
     return (~rows_lo & rep & 0x08040201u) | (~rows_hi & rep & 0x80402010u);
 }
 
-#ifndef TRRT_LOS_WARPS
-#define TRRT_LOS_WARPS 4
-#endif
-#ifndef TRRT_LOS_CTAS_PER_SM
-#define TRRT_LOS_CTAS_PER_SM 8
-#endif
-__global__ void __launch_bounds__(TRRT_LOS_WARPS * 32, TRRT_LOS_CTAS_PER_SM)
+constexpr int LOS_WARPS = 4, LOS_CTAS_PER_SM = 8; // CTA shape of los_tiled_kernel, also used by its launch
+__global__ void __launch_bounds__(LOS_WARPS * 32, LOS_CTAS_PER_SM)
     los_tiled_kernel(const uint4 *__restrict__ tiles, int side, int tp, const int32_t *__restrict__ map_id, const int4 *__restrict__ seg, long long n,
                      int rays_per_warp, int refill_min, int coop_max, uint8_t *__restrict__ out) {
     const int lane = threadIdx.x & 31;

@@ -127,9 +127,6 @@ struct Expand {
     int drive;
 };
 
-#ifndef TRRT_EXPAND_INLINE
-#define TRRT_EXPAND_INLINE __forceinline__ /* one call site per kernel; measured on cfg 3: inlined 38.8 ms, as a call 39.4 ms */
-#endif
 // Everything after the nearest node is known.  GA lanes share the rays / raster; GA == 1 is one lane working
 // alone (speculative schedule) and takes the single-lane code of trrt_lane.cuh.
 template <int GA>
@@ -141,9 +138,10 @@ __device__ __forceinline__ bool ray_clear(const Group<GA> &ga, const Grid &m, lo
     return ok;
 }
 
+// Inlined: one call site per kernel; measured on cfg 3: inlined 38.8 ms, as a call 39.4 ms.
 template <int GA>
-__device__ TRRT_EXPAND_INLINE void expand_from(const Group<GA> &ga, const Grid &m, const BikeParams &P, double ox, double oy, double oth,
-                                                   double qx, double qy, double qth, double gx, double gy, double gth, Expand &e_out) {
+__device__ __forceinline__ void expand_from(const Group<GA> &ga, const Grid &m, const BikeParams &P, double ox, double oy, double oth,
+                                           double qx, double qy, double qth, double gx, double gy, double gth, Expand &e_out) {
     // results are built in locals (only the three pixel counters have their address taken by the callees), so that
     // after inlining the caller's Expand stays in registers
     Expand e;
@@ -490,9 +488,7 @@ __global__ void __launch_bounds__(128) rrt_kernel_coop(const RrtDev a) {
 //   instead of being re-expanded by a single lane while the rest of the warp (and, through the lockstep barrier, of the
 //   CTA) waits.  Lane 0 has no predecessor in its window, so every window commits at least one iteration.
 // ---------------------------------------------------------------------------
-#ifndef TRRT_SCAN_AHEAD
-#define TRRT_SCAN_AHEAD 1024
-#endif
+constexpr int SCAN_AHEAD = 1024; // prefetch distance of nearest_private, in bytes of each coordinate array
 // private fp64 nearest scan over nodes [0, n): every lane of the warp reads the same node (broadcast loads)
 __device__ __forceinline__ void nearest_private(const double *__restrict__ nx, const double *__restrict__ ny, int n, double qx, double qy,
                                                 double &bd_out, int &bi_out) {
@@ -507,10 +503,10 @@ __device__ __forceinline__ void nearest_private(const double *__restrict__ nx, c
         const int pairs = (n - i) >> 1;
         int p = 0;
         for (; p + 1 < pairs; p += 2) {
-            // the tree streams from L2 / HBM: ask for the lines TRRT_SCAN_AHEAD bytes ahead (one request per 128-byte line)
-            if ((p & 7) == 0 && p + TRRT_SCAN_AHEAD / 16 < pairs) { // never beyond the nodes that exist
-                asm volatile("prefetch.global.L1 [%0];" ::"l"(x2 + p + TRRT_SCAN_AHEAD / 16));
-                asm volatile("prefetch.global.L1 [%0];" ::"l"(y2 + p + TRRT_SCAN_AHEAD / 16));
+            // the tree streams from L2 / HBM: ask for the lines SCAN_AHEAD bytes ahead (one request per 128-byte line)
+            if ((p & 7) == 0 && p + SCAN_AHEAD / 16 < pairs) { // never beyond the nodes that exist
+                asm volatile("prefetch.global.L1 [%0];" ::"l"(x2 + p + SCAN_AHEAD / 16));
+                asm volatile("prefetch.global.L1 [%0];" ::"l"(y2 + p + SCAN_AHEAD / 16));
             }
             const double2 xa = x2[p], ya = y2[p], xb = x2[p + 1], yb = y2[p + 1];
             const int b = i + 2 * p;
@@ -534,16 +530,15 @@ __device__ __forceinline__ void nearest_private(const double *__restrict__ nx, c
 // long-scoreboard stalls sit on those loads, and the CTA barrier then waits for the slowest scan).  Here the warp
 // copies the tree tile by tile with cp.async (LDGSTS, 512 coalesced bytes per instruction), two tiles in flight, and
 // all lanes read the tile from shared memory (conflict-free broadcast) while the next one is landing.
-#ifndef TRRT_TILE_PAIRS
-#define TRRT_TILE_PAIRS 32 /* double2 pairs of x (and of y) per tile = 64 nodes (one copy instruction per lane and array); 2 tiles x 2 arrays
-                             x 512 B per warp.  Multiple of 32.  Measured (cfg 3): 32 -> 63.7 ms, 64 -> 65.6 ms (less shared memory, more L1) */
-#endif
+// TILE_PAIRS: double2 pairs of x (and of y) per tile = 64 nodes (one copy instruction per lane and array); 2 tiles x 2
+// arrays x 512 B per warp.  Multiple of 32.  Measured (cfg 3): 32 -> 63.7 ms, 64 -> 65.6 ms (less shared memory, more L1).
+constexpr int TILE_PAIRS = 32;
 __device__ __forceinline__ void cp_async16(void *smem_dst, const void *gmem_src) {
     const unsigned d = (unsigned)__cvta_generic_to_shared(smem_dst);
     asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(d), "l"(gmem_src) : "memory");
 }
 // Nodes [lo, n) of the tree (lo = 0: the whole tree); lowest index on ties inside the range.
-__device__ __forceinline__ void nearest_staged(double2 *tile /* [2][2][TRRT_TILE_PAIRS] of this warp */, const double *__restrict__ nx,
+__device__ __forceinline__ void nearest_staged(double2 *tile /* [2][2][TILE_PAIRS] of this warp */, const double *__restrict__ nx,
                                                const double *__restrict__ ny, int lo, int n, double qx, double qy, double &bd_out, int &bi_out) {
     const int lane = threadIdx.x & 31;
     double bd = INFINITY;
@@ -555,12 +550,12 @@ __device__ __forceinline__ void nearest_staged(double2 *tile /* [2][2][TRRT_TILE
         const double2 *x2 = reinterpret_cast<const double2 *>(nx + i);
         const double2 *y2 = reinterpret_cast<const double2 *>(ny + i);
         const int pairs = (n - i) >> 1;
-        const int tiles = (pairs + TRRT_TILE_PAIRS - 1) / TRRT_TILE_PAIRS;
+        const int tiles = (pairs + TILE_PAIRS - 1) / TILE_PAIRS;
         auto issue = [&](int t) { // lanes copy pairs lane, lane + 32 of tile t (only pairs that exist)
-            double2 *bx = tile + (t & 1) * 2 * TRRT_TILE_PAIRS, *by = bx + TRRT_TILE_PAIRS;
-            const int p0 = t * TRRT_TILE_PAIRS;
+            double2 *bx = tile + (t & 1) * 2 * TILE_PAIRS, *by = bx + TILE_PAIRS;
+            const int p0 = t * TILE_PAIRS;
 #pragma unroll
-            for (int k = 0; k < TRRT_TILE_PAIRS / 32; k++) {
+            for (int k = 0; k < TILE_PAIRS / 32; k++) {
                 const int p = p0 + lane + 32 * k;
                 if (p < pairs) { cp_async16(bx + lane + 32 * k, x2 + p); cp_async16(by + lane + 32 * k, y2 + p); }
             }
@@ -571,9 +566,9 @@ __device__ __forceinline__ void nearest_staged(double2 *tile /* [2][2][TRRT_TILE
             if (t + 1 < tiles) { issue(t + 1); asm volatile("cp.async.wait_group 1;" ::: "memory"); }
             else asm volatile("cp.async.wait_group 0;" ::: "memory");
             __syncwarp(); // every lane's part of tile t has landed
-            const double2 *bx = tile + (t & 1) * 2 * TRRT_TILE_PAIRS, *by = bx + TRRT_TILE_PAIRS;
-            const int p0 = t * TRRT_TILE_PAIRS;
-            const int cnt = pairs - p0 < TRRT_TILE_PAIRS ? pairs - p0 : TRRT_TILE_PAIRS;
+            const double2 *bx = tile + (t & 1) * 2 * TILE_PAIRS, *by = bx + TILE_PAIRS;
+            const int p0 = t * TILE_PAIRS;
+            const int cnt = pairs - p0 < TILE_PAIRS ? pairs - p0 : TILE_PAIRS;
             int p = 0;
             for (; p + 1 < cnt; p += 2) {
                 const double2 xa = bx[p], ya = by[p], xb = bx[p + 1], yb = by[p + 1];
@@ -595,26 +590,16 @@ __device__ __forceinline__ void nearest_staged(double2 *tile /* [2][2][TRRT_TILE
     bd_out = bd; bi_out = bi;
 }
 
+// CTA shape of rrt_kernel_spec, also read by its launch: 2 CTAs of 14 warps = 28 warps per SM at 72 registers, so the
+// 4 096 queries of cfg 3 are resident at once (4 144 warps), no second wave.  Measured on B200 (cfg 3): 448 x 2 39.4 ms,
+// 384 x 2 43.9 ms, 512 x 2 (64 registers) 42.4 ms, 768 x 1 43.0 ms; see profiles/r2/NOTES.md.
+constexpr int SPEC_THREADS = 448, SPEC_BLOCKS_PER_SM = 2;
+
 // Lockstep: the expansion code (steer, libm, rays, raster: ~40 KB of SASS) is far larger than an SM's instruction
 // cache, and with warps spread over it the instruction fetches of a GPC saturate its shared cache (ncu: gcc
 // instruction requests at 85% of peak, SM i-cache hit rate 68%, half of all stall samples "no instruction").
 // So the warps of a CTA enter the expansion together: one CTA barrier per window, placed after the (tiny-code)
 // nearest scan; the first warp through a code line fetches it for the others (SM i-cache hit rate 89%, gcc at 47%).
-// A CTA is TRRT_SPEC_THREADS wide.
-#ifndef TRRT_PARAMS_SMEM
-#define TRRT_PARAMS_SMEM 1 /* parameter block in shared memory instead of a per-thread stack copy: 1712 -> 1312 bytes of stack */
-#endif
-#ifndef TRRT_SPEC_LOCKSTEP
-#define TRRT_SPEC_LOCKSTEP 1
-#endif
-#ifndef TRRT_SPEC_THREADS
-#define TRRT_SPEC_THREADS 448 /* 2 CTAs of 14 warps = 28 warps per SM at 72 registers: the 4 096 queries of cfg 3 are resident at once
-                                 (4 144 warps), no second wave.  Measured on B200 (cfg 3): 448 x 2 39.4 ms, 384 x 2 43.9 ms, 512 x 2 (64
-                                 registers) 42.4 ms, 768 x 1 43.0 ms; see profiles/r2/NOTES.md */
-#endif
-#ifndef TRRT_SPEC_BLOCKS_PER_SM
-#define TRRT_SPEC_BLOCKS_PER_SM 2
-#endif
 
 #ifdef TRRT_PHASE_PROF
 // experiment builds only (profiles/tools/phase_prof.py): per-warp clock64 sums of the phases of a window
@@ -625,14 +610,14 @@ __device__ unsigned long long g_phase_prof[24];
 #endif
 
 template <int G>
-__global__ void __launch_bounds__(TRRT_SPEC_THREADS, TRRT_SPEC_BLOCKS_PER_SM) rrt_kernel_spec(const RrtDev a) {
+__global__ void __launch_bounds__(SPEC_THREADS, SPEC_BLOCKS_PER_SM) rrt_kernel_spec(const RrtDev a) {
     const Group<G> g;
     const Group<1> solo;
     const int K = a.K;
-    __shared__ __align__(16) double2 scan_tiles[(G == 32) ? (TRRT_SPEC_THREADS / 32) * 4 * TRRT_TILE_PAIRS : 1];
-    double2 *scan_tile = scan_tiles + ((G == 32) ? (threadIdx.x >> 5) * 4 * TRRT_TILE_PAIRS : 0);
+    __shared__ __align__(16) double2 scan_tiles[(G == 32) ? (SPEC_THREADS / 32) * 4 * TILE_PAIRS : 1];
+    double2 *scan_tile = scan_tiles + ((G == 32) ? (threadIdx.x >> 5) * 4 * TILE_PAIRS : 0);
     // pooled scan (G == 32): what every warp of the CTA needs to scan a slice of any warp's tree for that warp's samples
-    constexpr int NW = TRRT_SPEC_THREADS / 32;
+    constexpr int NW = SPEC_THREADS / 32;
     static_assert(NW <= 32, "one lane per warp of the CTA in the scan partition");
     __shared__ double2 pool_q[(G == 32) ? NW : 1][32];            // sample of lane l of warp w
     __shared__ const double *pool_x[(G == 32) ? NW : 1], *pool_y[(G == 32) ? NW : 1];
@@ -640,16 +625,12 @@ __global__ void __launch_bounds__(TRRT_SPEC_THREADS, TRRT_SPEC_BLOCKS_PER_SM) rr
     __shared__ double pool_d[(G == 32) ? 2 * NW : 1][32];         // partial minima: one slot per (warp, tree) overlap
     __shared__ int pool_i[(G == 32) ? 2 * NW : 1][32];
     const unsigned lane_lt = (1u << g.gl) - 1u;
-#if TRRT_PARAMS_SMEM
     // The parameter block is handed to non-inlined device functions by reference.  A reference into the kernel's parameter
-    // space would be copied to every thread's local stack (192 bytes); one copy per CTA in shared memory serves all of them.
+    // space would be copied to every thread's local stack (192 bytes); one copy per CTA in shared memory serves all of them
+    // (1712 -> 1312 bytes of stack).
     __shared__ BikeParams sP;
     for (int i = threadIdx.x; i < (int)(sizeof(BikeParams) / 4); i += blockDim.x) reinterpret_cast<int *>(&sP)[i] = reinterpret_cast<const int *>(&a.P)[i];
     __syncthreads();
-#define TRRT_PARAMS_REF sP
-#else
-#define TRRT_PARAMS_REF a.P
-#endif
     // persistent groups: queries differ a lot in length (27% of the cfg-3 queries end early), so each group
     // pulls the next query from a counter instead of owning a fixed one.  One loop trip = one window.
     bool have = false, drained = false;
@@ -697,7 +678,7 @@ __global__ void __launch_bounds__(TRRT_SPEC_THREADS, TRRT_SPEC_BLOCKS_PER_SM) rr
         const bool live = (pre == -1) && !q_in_tree;
         // ---------------- nearest scan.  One warp per query (G == 32): the trees of a CTA's queries differ in size, some
         // warps have no query any more, and the expansion below is entered by the whole CTA together -- so the CTA scans
-        // as a pool.  The trees are cut into tiles of 2 * TRRT_TILE_PAIRS nodes, the tiles of all trees are laid end to end
+        // as a pool.  The trees are cut into tiles of 2 * TILE_PAIRS nodes, the tiles of all trees are laid end to end
         // and every warp takes an equal share of that list (a share overlaps one tree or a few); for each overlap the warp
         // scans its slice for the 32 samples of the warp that owns the tree and leaves the partial minima in shared
         // memory; after the barrier the owner folds the partials of its tree in node order (lowest index on ties).
@@ -711,7 +692,7 @@ __global__ void __launch_bounds__(TRRT_SPEC_THREADS, TRRT_SPEC_BLOCKS_PER_SM) rr
             __syncthreads();
             TRRT_PROF(t4_ = clock64();)
             // lane v describes the tree of warp v: tiles, first tile in the list, first / last warp that scans it, first slot
-            constexpr int TN = 2 * TRRT_TILE_PAIRS;
+            constexpr int TN = 2 * TILE_PAIRS;
             const int nv = lane < NW ? pool_n[lane] : 0;
             const int tv = (nv + TN - 1) / TN;
             int cv = tv; // inclusive prefix sum of the tile counts
@@ -750,16 +731,11 @@ __global__ void __launch_bounds__(TRRT_SPEC_THREADS, TRRT_SPEC_BLOCKS_PER_SM) rr
                 }
             }
         } else if (have) nearest_private(Q.nx, Q.ny, live ? n : 0, qx, qy, bd, near);
-#if TRRT_SPEC_LOCKSTEP
         // ---------------- CTA barrier: the partial minima are complete, the expansion code is entered together; also the exit test
         TRRT_PROF(t5_ = clock64();)
         if (!__syncthreads_or(have ? 1 : 0)) break;
         TRRT_PROF(t2_ = clock64(); { const unsigned long long s_ = t5_ - t4_; pf[0] += s_; pf[1] += s_ * s_ >> 10; pf[2] += t2_ - t5_; pf[18] += t4_ - t1_; pf[19] += t1_ - t0_; pf[20]++; if (have) pf[10]++; })
         if (!have) continue;
-#else
-        if (G == 32) { if (!__syncthreads_or(have ? 1 : 0)) break; if (!have) continue; }
-        else if (!have) break; // no query left for this group
-#endif
         if (G == 32) { // fold the partial minima of this warp's tree, in node order: the first minimum wins
             const int lane = threadIdx.x & 31;
             TRRT_CHECK(part0 >= 0 && part0 + nparts <= 2 * NW);
@@ -771,7 +747,7 @@ __global__ void __launch_bounds__(TRRT_SPEC_THREADS, TRRT_SPEC_BLOCKS_PER_SM) rr
         // ---------------- phase A, part 2: everything after the nearest node
         if (live) {
             TRRT_CHECK(near >= 0 && near < n);
-            expand_from<1>(solo, Q.m, TRRT_PARAMS_REF, Q.nx[near], Q.ny[near], Q.nth[near], qx, qy, qth, Q.gx, Q.gy, Q.gth, e);
+            expand_from<1>(solo, Q.m, sP, Q.nx[near], Q.ny[near], Q.nth[near], qx, qy, qth, Q.gx, Q.gy, Q.gth, e);
             if (e.code == EX_ACCEPT) exist = tree_find_slot(Q.tab, Q.tmask, Q.nx, Q.ny, Q.nth, e.wx, e.wy, e.wth, probes, islot);
         }
         c.probe += probes;
