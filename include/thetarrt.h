@@ -65,7 +65,8 @@ typedef enum trrt_status {
     TRRT_ERR_ENDPOINT_BLOCKED = 3,        /* [astar prints + False, search.py:225-227]         */
     TRRT_ERR_REF_RAISES_DRIVE_NONE = 4,   /* [TypeError: drive() after straight steer, rrt.py:170-171,275] */
     TRRT_ERR_REF_RAISES_ARGMIN_EMPTY = 5, /* [ValueError: np.argmin([]), search.py:262]        */
-    TRRT_ERR_CAPACITY = 6                 /* heap / path / node capacity of the call exceeded  */
+    TRRT_ERR_CAPACITY = 6,                /* heap / path / node capacity of the call exceeded  */
+    TRRT_ERR_REF_RAISES_NO_NEAREST = 7    /* [TypeError: findnearest of a childless tree, main.py:79-81] */
 } trrt_status;
 
 /* outcome of one RRT loop iteration (rrt.py:141-201) */
@@ -300,6 +301,75 @@ typedef struct trrt_theta_args {
    0 when the map cannot be planned (2*H*W does not fit an int32: TRRT_ERR_MAP_TOO_LARGE from trrt_theta_batch) */
 size_t trrt_theta_workspace_bytes(trrt_theta_args *args);
 int trrt_theta_batch(const trrt_theta_args *args, void *stream);
+
+/* ---------------------------------------------------------------------------
+ * mission_batch.  Replaces the segment chain of main.py:56-84 (main.chain) for
+ * n_missions independent (map, waypoints, sample stream) missions.  Segment s
+ * of a mission runs rrt.rrt from waypoint s to s+1 with the headings of
+ * main.py:58-67 (rrt.anglebetween, rrt.standardangle); once a segment has
+ * failed, every later segment starts at the most recent rrt.findnearest node
+ * (rrt.py:117-128) and takes its heading.  Segment s draws its K-1 rand_conf
+ * samples (rrt.py:53-68) around its own end from the mission's normals at the
+ * current offset, which then advances by 3 * iterations run.
+ * A mission stops at segment s, and stop_seg = s, when the RRT status is not
+ * OK (TRRT_ERR_REF_RAISES_DRIVE_NONE: the reference raises), when a failed
+ * segment has no nearest node (TRRT_ERR_REF_RAISES_NO_NEAREST), or when its
+ * normals run out (TRRT_ERR_CAPACITY).  A route whose status is not
+ * TRRT_OK_FOUND is copied with zero segments and stop_seg = 0.  A mission that
+ * ran its whole chain has status TRRT_OK_FOUND and stop_seg = -1.
+ * Each stage s launches a stage kernel, the trrt_rrt_batch launcher over the
+ * first n_active[s] slots, and a commit kernel.  Slot i holds mission
+ * d_order[i]; callers dispatch missions in decreasing segment count, so that
+ * the missions with a segment s are the first n_active[s] slots.
+ * ------------------------------------------------------------------------- */
+typedef struct trrt_mission_args {
+    /* map */
+    const uint32_t *d_bits;
+    int32_t n_maps, H, W;
+    const int32_t *d_map_id;     /* [n_missions] or NULL */
+    trrt_params params;
+    double xystdv, anglestdv;    /* builtins.xystdv / anglestdv (main.py:31-32), rand_conf rrt.py:53-68 */
+    int64_t n_missions;
+    int32_t K;                   /* builtins.K: node capacity, K-1 iterations per segment */
+    /* routes: the d_path / d_path_len / d_status layout of trrt_theta_batch */
+    const int32_t *d_waypoints;  /* [n_missions][wp_cap][2] */
+    int32_t wp_cap;
+    const int32_t *d_n_waypoints; /* [n_missions]; more than wp_cap -> TRRT_ERR_CAPACITY */
+    const int32_t *d_route_status; /* [n_missions] trrt_status of the route search, or NULL (all OK) */
+    /* standard normals in draw order: mission m reads d_normals[d_normal_range[m][0] .. d_normal_range[m][1]) */
+    const double *d_normals;
+    const int64_t *d_normal_range; /* [n_missions][2] */
+    /* schedule */
+    const int32_t *d_order;      /* [n_missions] slot -> mission */
+    int32_t n_stages;
+    const int32_t *n_active;     /* HOST [n_stages], non-increasing: missions with a segment s */
+    /* per-segment outputs [n_missions][seg_cap]; seg_cap >= the largest segment count (else TRRT_ERR_CAPACITY) */
+    int32_t seg_cap;
+    double *d_seg_begin;         /* [..][3] x, y, theta of the segment's start */
+    double *d_seg_end;           /* [..][3] */
+    double *d_seg_solution;      /* [..][3] rrt solution node, NaN when none */
+    double *d_seg_nearest;       /* [..][3] findnearest node of a failed segment, NaN otherwise */
+    double *d_seg_mindist;       /* [..]    its distance, NaN otherwise */
+    int32_t *d_seg_n_nodes;      /* [..] len(G) */
+    int32_t *d_seg_n_edges;      /* [..] child entries of G */
+    int32_t *d_seg_iters;        /* [..] loop iterations run */
+    int32_t *d_seg_status;       /* [..] trrt_status of the segment's RRT, 255 = not run */
+    /* per-mission outputs */
+    int32_t *d_status;           /* [n_missions] trrt_status */
+    int32_t *d_stop_seg;         /* [n_missions] */
+    int32_t *d_n_seg;            /* [n_missions] segments of the route */
+    double *d_path;              /* [n_missions][path_cap][8] x, y, theta, u[5] of main.path_nodes, segment after segment */
+    int32_t *d_path_seg;         /* [n_missions][path_cap] segment of each row */
+    int32_t path_cap;
+    int32_t *d_path_len;         /* [n_missions] full length even if > path_cap */
+    /* scratch, 256-byte aligned */
+    void *d_work;
+    size_t work_bytes;           /* >= trrt_mission_workspace_bytes(n_missions, K) */
+} trrt_mission_args;
+
+/* 19 * 256 + n_missions * (104 + 68 * K + 24 * (K - 1)) + trrt_rrt_workspace_bytes(n_missions, K) */
+size_t trrt_mission_workspace_bytes(int64_t n_missions, int32_t K);
+int trrt_mission_batch(const trrt_mission_args *args, void *stream);
 
 #ifdef __cplusplus
 }

@@ -63,6 +63,24 @@ class CThetaArgs(C.Structure):
     ]
 
 
+class CMissionArgs(C.Structure):
+    """struct trrt_mission_args."""
+    _fields_ = [
+        ("d_bits", C.c_void_p), ("n_maps", C.c_int32), ("H", C.c_int32), ("W", C.c_int32), ("d_map_id", C.c_void_p),
+        ("params", CParams), ("xystdv", C.c_double), ("anglestdv", C.c_double),
+        ("n_missions", C.c_int64), ("K", C.c_int32),
+        ("d_waypoints", C.c_void_p), ("wp_cap", C.c_int32), ("d_n_waypoints", C.c_void_p), ("d_route_status", C.c_void_p),
+        ("d_normals", C.c_void_p), ("d_normal_range", C.c_void_p),
+        ("d_order", C.c_void_p), ("n_stages", C.c_int32), ("n_active", C.c_void_p),
+        ("seg_cap", C.c_int32), ("d_seg_begin", C.c_void_p), ("d_seg_end", C.c_void_p), ("d_seg_solution", C.c_void_p),
+        ("d_seg_nearest", C.c_void_p), ("d_seg_mindist", C.c_void_p), ("d_seg_n_nodes", C.c_void_p),
+        ("d_seg_n_edges", C.c_void_p), ("d_seg_iters", C.c_void_p), ("d_seg_status", C.c_void_p),
+        ("d_status", C.c_void_p), ("d_stop_seg", C.c_void_p), ("d_n_seg", C.c_void_p),
+        ("d_path", C.c_void_p), ("d_path_seg", C.c_void_p), ("path_cap", C.c_int32), ("d_path_len", C.c_void_p),
+        ("d_work", C.c_void_p), ("work_bytes", C.c_size_t),
+    ]
+
+
 # every symbol include/thetarrt.h declares: name -> (restype, argtypes)
 SIGNATURES = {
     "trrt_version": (C.c_int, []),
@@ -95,6 +113,8 @@ SIGNATURES = {
                                          C.c_void_p, C.c_void_p]),
     "trrt_theta_workspace_bytes": (C.c_size_t, [C.POINTER(CThetaArgs)]),
     "trrt_theta_batch": (C.c_int, [C.POINTER(CThetaArgs), C.c_void_p]),
+    "trrt_mission_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int32]),
+    "trrt_mission_batch": (C.c_int, [C.POINTER(CMissionArgs), C.c_void_p]),
 }
 
 _lib = None

@@ -12,6 +12,7 @@
 //   arc_pixels_kernel         pixel lists of search.getArc / getCircle / bresenham in the reference's list order
 //   clearance / anglediff batch kernels: rrt.bike_clear, rrt.front_of_bike_clear, rrt.anglediff
 //   findnearest_kernel    rrt.findnearest over the edge log
+//   mission_*_kernel      main.py missions: segment chain around trrt_rrt_batch, findnearest restarts (trrt_mission.cuh)
 //   theta_kernel<G>       K3: A* / lazy Theta*, G lanes per query, G-ary heap
 //
 // Build: nvcc -gencode arch=compute_100a,code=sm_100a -fmad=false -lineinfo
@@ -26,6 +27,7 @@
 #include "trrt_bike.cuh"
 #include "trrt_device.cuh"
 #include "trrt_los.cuh"
+#include "trrt_mission.cuh"
 #include "trrt_rrt.cuh"
 
 using namespace trrt;
@@ -416,42 +418,19 @@ __global__ void anglediff_batch_kernel(int64_t n, const double *__restrict__ in,
 }
 
 // ===========================================================================
-// rrt.findnearest (rrt.py:117-128): one block per query over the edge log.
-// The reference walks parents in tree order and children in append order with
-// a strict `<`, i.e. it returns the edge minimising (distance, parent index,
-// iteration) lexicographically.
+// rrt.findnearest (rrt.py:117-128): one block per query over the edge log
+// (findnearest_block, trrt_mission.cuh).
 // ===========================================================================
-__global__ void __launch_bounds__(128) findnearest_kernel(BikeParams P, int64_t nq, int K, const double *__restrict__ nx, const double *__restrict__ ny,
-                                                          const double *__restrict__ nth, const int32_t *__restrict__ it_near,
-                                                          const int32_t *__restrict__ it_new, const double *__restrict__ goal, int32_t *best,
-                                                          double *best_dist) {
+__global__ void __launch_bounds__(FN_THREADS) findnearest_kernel(BikeParams P, int64_t nq, int K, const double *__restrict__ nx, const double *__restrict__ ny,
+                                                                 const double *__restrict__ nth, const int32_t *__restrict__ it_near,
+                                                                 const int32_t *__restrict__ it_new, const double *__restrict__ goal, int32_t *best,
+                                                                 double *best_dist) {
     int64_t q = blockIdx.x;
-    const double gx = goal[3 * q], gy = goal[3 * q + 1], gth = goal[3 * q + 2];
-    double bd = INFINITY;
-    int bp = 0x7fffffff, bit = 0x7fffffff, bc = -1;
-    for (int it = threadIdx.x; it < K - 1; it += blockDim.x) {
-        int c = it_new[q * (int64_t)(K - 1) + it];
-        if (c < 0) continue;
-        int p = it_near[q * (int64_t)(K - 1) + it];
-        double dx = gx - nx[q * K + c], dy = gy - ny[q * K + c];
-        double d = P.weightxy * sqrt(dx * dx + dy * dy) + (1 - P.weightxy) * fabs(anglediff(nth[q * K + c], gth));
-        if (d < bd || (d == bd && (p < bp || (p == bp && it < bit)))) { bd = d; bp = p; bit = it; bc = c; }
-    }
-    __shared__ double sd[128];
-    __shared__ int sp[128], si[128], sc[128];
-    sd[threadIdx.x] = bd; sp[threadIdx.x] = bp; si[threadIdx.x] = bit; sc[threadIdx.x] = bc;
-    __syncthreads();
-    for (int off = 64; off > 0; off >>= 1) {
-        if ((int)threadIdx.x < off) {
-            int o = threadIdx.x + off;
-            if (sc[o] >= 0 && (sc[threadIdx.x] < 0 || sd[o] < sd[threadIdx.x] ||
-                               (sd[o] == sd[threadIdx.x] && (sp[o] < sp[threadIdx.x] || (sp[o] == sp[threadIdx.x] && si[o] < si[threadIdx.x]))))) {
-                sd[threadIdx.x] = sd[o]; sp[threadIdx.x] = sp[o]; si[threadIdx.x] = si[o]; sc[threadIdx.x] = sc[o];
-            }
-        }
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) { best[q] = sc[0]; best_dist[q] = sc[0] >= 0 ? sd[0] : NAN; }
+    int b;
+    double d;
+    findnearest_block(P, K, nx + q * K, ny + q * K, nth + q * K, it_near + q * (int64_t)(K - 1), it_new + q * (int64_t)(K - 1), goal[3 * q],
+                      goal[3 * q + 1], goal[3 * q + 2], b, d);
+    if (threadIdx.x == 0) { best[q] = b; best_dist[q] = d; }
 }
 
 // ===========================================================================
@@ -771,6 +750,32 @@ __global__ void __launch_bounds__(128) theta_kernel(const ThetaDev a) {
         }
         g.sync();
     }
+}
+
+// Workspace of mission_batch: per-mission state, then the per-slot rows of one stage (trrt_rrt_batch inputs and
+// outputs for up to n_missions slots), then trrt_rrt_batch's own workspace; every region starts 256-byte aligned.
+struct MissionCarve {
+    char *base;
+    size_t p;
+    template <typename T> T *take(size_t count) {
+        p = (p + 255) & ~(size_t)255;
+        T *r = base ? (T *)(base + p) : nullptr;
+        p += count * sizeof(T);
+        return r;
+    }
+};
+static size_t mission_carve(MissionDev &d, void *work, int64_t n, int K) {
+    MissionCarve c{(char *)work, 0};
+    const size_t N = (size_t)n, Kn = (size_t)K, K1 = (size_t)(K - 1);
+    d.off = c.take<int64_t>(N); d.restart = c.take<double>(3 * N); d.restarted = c.take<int32_t>(N);
+    d.q_start = c.take<double>(3 * N); d.q_goal = c.take<double>(3 * N); d.q_map = c.take<int32_t>(N);
+    d.q_sxy = c.take<int32_t>(2 * N * K1); d.q_sth = c.take<double>(N * K1);
+    d.nx = c.take<double>(N * Kn); d.ny = c.take<double>(N * Kn); d.nth = c.take<double>(N * Kn); d.u = c.take<double>(5 * N * Kn);
+    d.parent = c.take<int32_t>(N * Kn);
+    d.q_n_nodes = c.take<int32_t>(N); d.q_sol = c.take<int32_t>(N); d.q_status = c.take<int32_t>(N); d.q_iters = c.take<int32_t>(N);
+    d.it_near = c.take<int32_t>(N * K1); d.it_new = c.take<int32_t>(N * K1);
+    c.take<char>(0); // start of the RRT workspace
+    return c.p;
 }
 
 // ===========================================================================
@@ -1204,6 +1209,68 @@ int trrt_theta_batch(const trrt_theta_args *args, void *stream) {
     default: theta_kernel<32><<<(unsigned)blocks, threads, 0, st>>>(d); break;
     }
     CUDA_TRY(cudaGetLastError());
+    return TRRT_OK;
+}
+
+size_t trrt_mission_workspace_bytes(int64_t n_missions, int32_t K) {
+    if (n_missions <= 0 || K < 1) return 256;
+    const size_t n = (size_t)n_missions, k = (size_t)K;
+    return 19 * 256 + n * (104 + 68 * k + 24 * (k - 1)) + trrt_rrt_workspace_bytes(n_missions, K);
+}
+
+int trrt_mission_batch(const trrt_mission_args *args, void *stream) {
+    if (!args) return TRRT_ERR_INVALID_ARGUMENT;
+    const trrt_mission_args &A = *args;
+    int e = check_map(A.n_maps, A.H, A.W);
+    if (e) return e;
+    if (A.n_missions < 0 || A.K < 2 || A.n_stages < 0 || A.seg_cap < 0 || A.wp_cap < 1 || A.path_cap < 0) return TRRT_ERR_INVALID_ARGUMENT;
+    if (A.n_missions == 0) return TRRT_OK;
+    if (!A.d_bits || !A.d_waypoints || !A.d_n_waypoints || !A.d_normals || !A.d_normal_range || !A.d_order || (A.n_stages > 0 && !A.n_active) ||
+        !A.d_status || !A.d_stop_seg || !A.d_n_seg || !A.d_path_len || (A.path_cap > 0 && (!A.d_path || !A.d_path_seg)) || !A.d_work)
+        return TRRT_ERR_INVALID_ARGUMENT;
+    if (A.seg_cap > 0 && (!A.d_seg_begin || !A.d_seg_end || !A.d_seg_solution || !A.d_seg_nearest || !A.d_seg_mindist || !A.d_seg_n_nodes ||
+                          !A.d_seg_n_edges || !A.d_seg_iters || !A.d_seg_status))
+        return TRRT_ERR_INVALID_ARGUMENT;
+    if (A.n_stages > A.seg_cap) return TRRT_ERR_INVALID_ARGUMENT;
+    for (int s = 0; s < A.n_stages; s++) // the active missions of a stage are a prefix of the slots of the one before
+        if (A.n_active[s] < 0 || A.n_active[s] > (s ? A.n_active[s - 1] : A.n_missions)) return TRRT_ERR_INVALID_ARGUMENT;
+    if ((uintptr_t)A.d_work & 255) return TRRT_ERR_INVALID_ARGUMENT;
+    if (A.work_bytes < trrt_mission_workspace_bytes(A.n_missions, A.K)) return TRRT_ERR_WORKSPACE_TOO_SMALL;
+    MissionDev d;
+    d.H = A.H; d.W = A.W; d.map_id = A.d_map_id; d.P = to_dev(A.params); d.xystdv = A.xystdv; d.anglestdv = A.anglestdv;
+    d.n = A.n_missions; d.K = A.K; d.wp = A.d_waypoints; d.wp_cap = A.wp_cap; d.n_wp = A.d_n_waypoints; d.route_status = A.d_route_status;
+    d.normals = A.d_normals; d.nrange = A.d_normal_range; d.order = A.d_order;
+    d.seg_cap = A.seg_cap; d.seg_begin = A.d_seg_begin; d.seg_end = A.d_seg_end; d.seg_solution = A.d_seg_solution;
+    d.seg_nearest = A.d_seg_nearest; d.seg_mindist = A.d_seg_mindist; d.seg_n_nodes = A.d_seg_n_nodes; d.seg_n_edges = A.d_seg_n_edges;
+    d.seg_iters = A.d_seg_iters; d.seg_status = A.d_seg_status;
+    d.status = A.d_status; d.stop_seg = A.d_stop_seg; d.n_seg = A.d_n_seg; d.path = A.d_path; d.path_seg = A.d_path_seg;
+    d.path_cap = A.path_cap; d.path_len = A.d_path_len;
+    const size_t rrt_off = mission_carve(d, A.d_work, A.n_missions, A.K);
+    cudaStream_t st = (cudaStream_t)stream;
+    int64_t ib = (A.n_missions + MISSION_THREADS - 1) / MISSION_THREADS;
+    if (ib > (int64_t)sm_count() * 16) ib = (int64_t)sm_count() * 16;
+    mission_init_kernel<<<(unsigned)ib, MISSION_THREADS, 0, st>>>(d);
+    CUDA_TRY(cudaGetLastError());
+    trrt_rrt_args r;
+    memset(&r, 0, sizeof(r));
+    r.d_bits = A.d_bits; r.n_maps = A.n_maps; r.H = A.H; r.W = A.W; r.d_map_id = A.d_map_id ? d.q_map : nullptr; r.params = A.params;
+    r.K = A.K; r.d_start = d.q_start; r.d_goal = d.q_goal; r.d_sample_xy = d.q_sxy; r.d_sample_th = d.q_sth;
+    r.d_node_x = d.nx; r.d_node_y = d.ny; r.d_node_th = d.nth; r.d_parent = d.parent; r.d_u = d.u;
+    r.d_n_nodes = d.q_n_nodes; r.d_sol = d.q_sol; r.d_status = d.q_status; r.d_iters = d.q_iters;
+    r.d_it_near = d.it_near; r.d_it_new = d.it_new;
+    r.d_work = (char *)A.d_work + rrt_off;
+    r.work_bytes = A.work_bytes - rrt_off;
+    for (int s = 0; s < A.n_stages; s++) {
+        const int na = A.n_active[s];
+        if (na == 0) break;
+        mission_stage_kernel<<<(unsigned)na, MISSION_THREADS, 0, st>>>(d, s);
+        CUDA_TRY(cudaGetLastError());
+        r.n_queries = na; // slots are a prefix: the per-slot arrays and the RRT workspace of n_missions queries cover it
+        e = trrt_rrt_batch(&r, stream);
+        if (e) return e;
+        mission_commit_kernel<<<(unsigned)na, MISSION_THREADS, 0, st>>>(d, s);
+        CUDA_TRY(cudaGetLastError());
+    }
     return TRRT_OK;
 }
 

@@ -83,7 +83,7 @@ def chain(waypoints, debug=False):
 def plan(image, start=None, goal=None, waypoints=None, debug=False):
     """Map in, chained path out.  `waypoints` defaults to the Theta* path from `start` to `goal`
     (the computation the reference keeps commented out at main.py:48-52); with neither given, the
-    reference's own waypoint list (main.py:57) is used."""
+    reference's own waypoint list (main.py:57) is used.  plan_batch() plans many missions at once."""
     set_map(image)
     if waypoints is None:
         if start is None or goal is None:
@@ -104,6 +104,50 @@ def path_nodes(segment):
         prev = segment["camefrom"].get(node)
         node = prev[0] if prev else None
     return out[::-1]
+
+
+def _node(row):
+    return None if np.isnan(row[0]) else ((float(row[0]), float(row[1])), float(row[2]))
+
+
+def mission_records(h, m):
+    """Mission m of a host MissionResult (`Planner.missions(...).host()`) as main.plan would return it: False when
+    the route search finds no path (search.py:222-227, :307), the exception the reference raises when it raises, else
+    one record per segment with the keys of chain(); `n_nodes` / `n_edges` stand for the graph / camefrom dicts,
+    and `path` is path_nodes() of the segment (the rows that fit the result's path_cap)."""
+    status, n_seg = int(h["status"][m]), int(h["n_seg"][m])
+    if status == 4:
+        return TypeError("unsupported operand type(s) for *: 'float' and 'NoneType'")  # rrt.py:170-171, :275
+    if status == 7:
+        return TypeError("'NoneType' object is not subscriptable")  # main.py:79-81
+    if status == 5:
+        return ValueError("attempt to get argmin of an empty sequence")  # search.py:262
+    if status in (1, 2, 3):
+        return False
+    if status != 0:
+        return RuntimeError(f"mission status {status} (capacity of the call exceeded)")
+    n_rows = min(int(h["path_len"][m]), h["path"].shape[1])
+    rows, row_seg = h["path"][m, :n_rows], h["path_seg"][m, :n_rows]
+    out = []
+    for s in range(n_seg):
+        mind = float(h["mindist"][m, s])
+        out.append({"begin": _node(h["begin"][m, s]), "end": _node(h["end"][m, s]),
+                    "solution": _node(h["solution"][m, s]), "nearest": _node(h["nearest"][m, s]),
+                    "mindist": None if np.isnan(mind) else mind, "n_nodes": int(h["n_nodes"][m, s]),
+                    "n_edges": int(h["n_edges"][m, s]), "path": [_node(r) for r in rows[row_seg == s]]})
+    return out
+
+
+def plan_batch(image, starts, goals, seeds, K=None):
+    """plan() for many (start, goal, seed) missions on one map: Theta* (A* with THETASTAR=False) waypoints and the
+    segment chain of every mission in one batched device call (Planner.missions).  Mission m draws its samples like
+    plan() after np.random.seed(seeds[m]).  Returns one mission_records() entry per mission."""
+    set_map(image)
+    from . import _context
+    p = _context.current_planner()
+    sg = np.concatenate([np.asarray(starts, np.int32).reshape(-1, 2), np.asarray(goals, np.int32).reshape(-1, 2)], axis=1)
+    h = p.missions(start_goal=sg, seeds=seeds, K=K if K is not None else int(p.params.K)).host()
+    return [mission_records(h, m) for m in range(len(sg))]
 
 
 def main(argv=None):

@@ -19,7 +19,9 @@ from .grid import OccupancyGrid
 from .params import Params
 
 STATUS_NAMES = {0: "OK_FOUND", 1: "OK_NOT_FOUND", 2: "ERR_ENDPOINT_INVALID", 3: "ERR_ENDPOINT_BLOCKED",
-                4: "ERR_REF_RAISES_DRIVE_NONE", 5: "ERR_REF_RAISES_ARGMIN_EMPTY", 6: "ERR_CAPACITY"}
+                4: "ERR_REF_RAISES_DRIVE_NONE", 5: "ERR_REF_RAISES_ARGMIN_EMPTY", 6: "ERR_CAPACITY",
+                7: "ERR_REF_RAISES_NO_NEAREST"}
+SEG_NOT_RUN = 255
 IT_NEW_NODE, IT_EXISTING_NODE, IT_QRAND_BLOCKED, IT_QRAND_IN_TREE, IT_STEER_CONSTRAINT, IT_ARC_BLOCKED = range(6)
 IT_NOT_RUN = 255
 COUNTER_NAMES = ("nodes_scanned", "los_calls", "los_pixels", "arc_candidate_pixels", "arc_angle_tests",
@@ -81,6 +83,54 @@ class ThetaResult:
         return _host_dict(self)
 
 
+@dataclass
+class MissionResult:
+    """Planner.missions output.  Per segment [B, S] (S = largest segment count): begin, end, solution, nearest
+    (float64 [.., 3] = x, y, theta; NaN where the reference has None), mindist (NaN when none), n_nodes, n_edges,
+    iters, seg_status (trrt_status of the segment's RRT, SEG_NOT_RUN = 255 where no segment ran).  Per mission:
+    status (0 = the chain ran to its end; 4 / 7 = it stopped where the reference raises; otherwise the route search's
+    status), stop_seg (-1 when the chain ran to its end), n_seg, waypoints (int32 [B, wp_cap, 2], n_waypoints of them
+    valid), path (float64 [B, path_cap, 8] = x, y, theta, u[5] of main.path_nodes, segment after segment), path_seg
+    (segment of each row) and path_len (full length, also when it exceeds path_cap; rows past it are not written)."""
+    K: int
+    begin: torch.Tensor
+    end: torch.Tensor
+    solution: torch.Tensor
+    nearest: torch.Tensor
+    mindist: torch.Tensor
+    n_nodes: torch.Tensor
+    n_edges: torch.Tensor
+    iters: torch.Tensor
+    seg_status: torch.Tensor
+    status: torch.Tensor
+    stop_seg: torch.Tensor
+    n_seg: torch.Tensor
+    waypoints: torch.Tensor
+    n_waypoints: torch.Tensor
+    path: torch.Tensor
+    path_seg: torch.Tensor
+    path_len: torch.Tensor
+    route: ThetaResult | None = None
+
+    def host(self):
+        out = _host_dict(self)
+        if self.route is not None:
+            out["route"] = self.route.host()
+        return out
+
+
+def mission_schedule(n_seg):
+    """Dispatch order of trrt_mission_batch: missions by decreasing segment count (stable), so that the missions
+    with a segment s are the first n_active[s] slots.  Returns (order int32 [B], n_active int32 [max(n_seg)])."""
+    n_seg = np.asarray(n_seg, dtype=np.int64).reshape(-1)
+    if n_seg.size and n_seg.min() < 0:
+        raise ValueError("segment counts must be >= 0")
+    order = np.argsort(-n_seg, kind="stable").astype(np.int32)
+    S = int(n_seg.max()) if n_seg.size else 0
+    n_active = (n_seg[None, :] > np.arange(S)[:, None]).sum(axis=1).astype(np.int32)
+    return order, n_active
+
+
 class Planner:
     """Device-resident planner for one OccupancyGrid (one or several same-size maps)."""
 
@@ -107,7 +157,8 @@ class Planner:
                 t = t.to(dtype)
             t = t.contiguous()
         else:
-            npdt = {torch.float64: np.float64, torch.int32: np.int32, torch.uint8: np.uint8, torch.int16: np.int16}[dtype]
+            npdt = {torch.float64: np.float64, torch.int32: np.int32, torch.uint8: np.uint8, torch.int16: np.int16,
+                    torch.int64: np.int64}[dtype]
             h = torch.from_numpy(np.ascontiguousarray(np.asarray(a, dtype=npdt)))
             t = h.pin_memory().to(self.device, non_blocking=True) if h.numel() else h.to(self.device)
         if shape is not None:
@@ -571,4 +622,127 @@ class Planner:
             _lib.check(self.lib.trrt_theta_batch(C.byref(a), self._stream()), "trrt_theta_batch")
             res.extra = dict(n_slots=int(a.n_slots), heap_cap=int(a.heap_cap), workspace_bytes=int(wb))
             res._keep = (sg, mid, order)
+        return res
+
+    # ------------------------------------------------------------------ main.py missions
+    def missions(self, start_goal=None, waypoints=None, seeds=None, normals=None, normal_range=None, map_id=None, K=None,
+                 thetastar=None, path_cap=None, params=None) -> MissionResult:
+        """main.plan for a batch of missions (main.py:56-84): a route, then one RRT per consecutive waypoint pair with
+        the headings of main.chain, restarting from the rrt.findnearest node once a segment has failed.  The segment
+        chain runs on the device (trrt_mission_batch): per stage, one kernel builds every mission's start, goal and
+        samples, the fused RRT kernel runs, and one kernel commits the segment records and path rows.
+
+        Routes: `waypoints` (one (n_i, 2) integer sequence per mission), or Theta* / A* (`thetastar`, default
+        Params.THETASTAR) over `start_goal` int32 [B, 4] = (sx, sy, gx, gy).  The route lengths are read back once to
+        build the schedule; nothing else waits for the device.
+        Samples: `seeds` gives mission m the normals of np.random.RandomState(seeds[m]) in draw order, i.e. the stream
+        main.chain consumes after np.random.seed(seeds[m]) (reference parity).  Or `normals`: a float64 stream (e.g. a
+        device torch.randn tensor) with `normal_range` int64 [B, 2] = [begin, end) per mission, or a [B, L] tensor with one
+        row per mission; mission m needs 3 * (K-1) * n_seg[m] values.
+        map_id: [B] map of each mission.  path_cap: path rows kept per mission (default n_seg_max * K, which never
+        truncates)."""
+        P = params or self.params
+        K = int(K if K is not None else P.K)
+        if K < 2:
+            raise ValueError("K must be >= 2")
+        if (seeds is None) == (normals is None):
+            raise ValueError("pass exactly one of seeds and normals")
+        g = self.grid
+        with torch.cuda.device(self.device):
+            route = None
+            if waypoints is None:
+                if start_goal is None:
+                    raise ValueError("pass start_goal or waypoints")
+                route = self.theta(start_goal, thetastar=thetastar if thetastar is not None else P.THETASTAR, map_id=map_id)
+                wp, n_wp, route_status = route.path, route.path_len, route.status
+                hr = torch.stack([n_wp, route_status]).cpu().numpy()  # the one host read: segment counts for the schedule
+                n_wp_h, rs_h = hr[0].astype(np.int64), hr[1]
+                B = len(n_wp_h)
+                ok = (rs_h == 0) & (n_wp_h <= wp.shape[1])
+                n_seg = np.where(ok, np.maximum(n_wp_h - 1, 0), 0)
+            else:
+                wl = [np.asarray(w, dtype=np.int64).reshape(-1, 2) for w in waypoints]
+                B = len(wl)
+                n_wp_h = np.array([len(w) for w in wl], np.int64)
+                wp_h = np.zeros((B, max(int(n_wp_h.max()) if B else 1, 1), 2), np.int32)
+                for m, w in enumerate(wl):
+                    wp_h[m, :len(w)] = w
+                wp = self._dev(wp_h, torch.int32)
+                n_wp = self._dev(n_wp_h, torch.int32)
+                route_status = None
+                n_seg = np.maximum(n_wp_h - 1, 0)
+            order, n_active = mission_schedule(n_seg)
+            S = len(n_active)
+            need = 3 * (K - 1) * n_seg
+            if seeds is not None:
+                seeds = np.asarray(seeds).reshape(-1)
+                if len(seeds) != B:
+                    raise ValueError(f"{len(seeds)} seeds for {B} missions")
+                rng = np.zeros((B, 2), np.int64)
+                rng[:, 1] = np.cumsum(need)
+                rng[1:, 0] = rng[:-1, 1]
+                flat = np.empty(int(need.sum()), np.float64)
+                for m in range(B):
+                    if need[m]:
+                        flat[rng[m, 0]:rng[m, 1]] = np.random.RandomState(int(seeds[m])).standard_normal(int(need[m]))
+                nz = self._dev(flat, torch.float64) if flat.size else torch.zeros(1, dtype=torch.float64, device=self.device)
+            else:
+                nz = self._dev(normals, torch.float64)
+                if normal_range is None:
+                    if nz.dim() != 2 or nz.shape[0] != B:
+                        raise ValueError("normals without normal_range must be a [missions, L] array")
+                    L = nz.shape[1]
+                    rng = np.stack([np.arange(B) * L, np.arange(B) * L + L], axis=1).astype(np.int64)
+                else:
+                    rng = (normal_range.cpu().numpy() if isinstance(normal_range, torch.Tensor) else np.asarray(normal_range))
+                    rng = rng.astype(np.int64).reshape(B, 2)
+                nz = nz.reshape(-1)
+                if B and (rng.min() < 0 or rng[:, 1].max() > nz.numel() or (rng[:, 1] < rng[:, 0]).any()):
+                    raise ValueError("normal_range outside the normals")
+                short = np.nonzero(rng[:, 1] - rng[:, 0] < need)[0]
+                if len(short):
+                    m = int(short[0])
+                    raise ValueError(f"mission {m} has {int(rng[m, 1] - rng[m, 0])} normals, its {int(n_seg[m])} segments "
+                                     f"need {int(need[m])} (3 * (K-1) per segment)")
+                if nz.numel() == 0:
+                    nz = torch.zeros(1, dtype=torch.float64, device=self.device)
+            rng_d = self._dev(rng, torch.int64) if B else None
+            order_d = self._dev(order, torch.int32)
+            mid = self._map_ids(map_id, B)
+            if path_cap is None:
+                path_cap = max(S * K, 1)
+            dev = self.device
+            f64 = dict(dtype=torch.float64, device=dev)
+            i32 = dict(dtype=torch.int32, device=dev)
+            Sc = max(S, 1)
+            res = MissionResult(K=K, begin=torch.empty((B, Sc, 3), **f64), end=torch.empty((B, Sc, 3), **f64),
+                                solution=torch.empty((B, Sc, 3), **f64), nearest=torch.empty((B, Sc, 3), **f64),
+                                mindist=torch.empty((B, Sc), **f64), n_nodes=torch.empty((B, Sc), **i32),
+                                n_edges=torch.empty((B, Sc), **i32), iters=torch.empty((B, Sc), **i32),
+                                seg_status=torch.empty((B, Sc), **i32), status=torch.empty(B, **i32),
+                                stop_seg=torch.empty(B, **i32), n_seg=torch.empty(B, **i32), waypoints=wp,
+                                n_waypoints=n_wp, path=torch.empty((B, int(path_cap), 8), **f64),
+                                path_seg=torch.empty((B, int(path_cap)), **i32), path_len=torch.empty(B, **i32), route=route)
+            if B == 0:
+                return res
+            wb = self.lib.trrt_mission_workspace_bytes(B, K)
+            work = self._scratch("mission", wb)
+            ptr = lambda t: t.data_ptr() if t is not None else None  # noqa: E731
+            n_active_h = np.ascontiguousarray(n_active, dtype=np.int32)
+            a = _lib.CMissionArgs(d_bits=g.bits.data_ptr(), n_maps=g.n_maps, H=g.H, W=g.W, d_map_id=ptr(mid),
+                                  params=P.to_c(), xystdv=float(P.xystdv), anglestdv=float(P.anglestdv), n_missions=B, K=K,
+                                  d_waypoints=wp.data_ptr(), wp_cap=int(wp.shape[1]), d_n_waypoints=n_wp.data_ptr(),
+                                  d_route_status=ptr(route_status), d_normals=nz.data_ptr(), d_normal_range=rng_d.data_ptr(),
+                                  d_order=order_d.data_ptr(), n_stages=S, n_active=n_active_h.ctypes.data if S else None,
+                                  seg_cap=Sc, d_seg_begin=res.begin.data_ptr(), d_seg_end=res.end.data_ptr(),
+                                  d_seg_solution=res.solution.data_ptr(), d_seg_nearest=res.nearest.data_ptr(),
+                                  d_seg_mindist=res.mindist.data_ptr(), d_seg_n_nodes=res.n_nodes.data_ptr(),
+                                  d_seg_n_edges=res.n_edges.data_ptr(), d_seg_iters=res.iters.data_ptr(),
+                                  d_seg_status=res.seg_status.data_ptr(), d_status=res.status.data_ptr(),
+                                  d_stop_seg=res.stop_seg.data_ptr(), d_n_seg=res.n_seg.data_ptr(),
+                                  d_path=res.path.data_ptr(), d_path_seg=res.path_seg.data_ptr(), path_cap=int(path_cap),
+                                  d_path_len=res.path_len.data_ptr(), d_work=work.data_ptr(), work_bytes=work.numel())
+            _lib.check(self.lib.trrt_mission_batch(C.byref(a), self._stream()), "trrt_mission_batch")
+            res._keep = (nz, rng_d, order_d, mid)
+            res.schedule = (order, n_active)
         return res
