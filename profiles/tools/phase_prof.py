@@ -48,7 +48,7 @@ print(f"kernel {a.elapsed_time(b):.2f} ms, windows (warp x window) {W}, iteratio
 names = [("sample, publish", 19, None), ("wait at barrier 1", 18, None), ("pooled scan", 0, 1), ("wait at barrier 2", 2, None), ("expansion", 3, 4), ("pass + commit", 7, 8)]
 WR = v[20] or W  # warp-rounds (idle warps take part in the pooled scan and the barriers)
 print(f"warp-rounds {WR}, of which with a query {W}")
-tot = v[0] + v[2] + v[3] + v[5] + v[7] + v[18] + v[19]
+tot = v[0] + v[2] + v[3] + v[7] + v[18] + v[19]
 for nm, i, j in names:
     Wn = W if i in (3, 7) else WR
     mean = v[i] / Wn
@@ -58,6 +58,11 @@ for nm, i, j in names:
         line += f"  std {max(var, 0) ** 0.5:9.0f}"
     print(line)
 if v[21]: print(f"  of 'sample, publish': nearest lookup {v[21] / WR:.0f} cycles, of which the walk over the cells {v[22] / WR:.0f}")
+if v[14]:  # fp32 prefilter of the pooled scan (per lane: one sample against one slice of a tree)
+    print(f"  scan prefilter: lane-slices {v[14]}, fp32 blocks {v[15] / v[14]:.1f} per lane-slice; rechecked in fp64 {v[11] / v[14]:.2f} "
+          f"blocks per lane-slice ({100 * v[11] / max(v[15], 1):.2f}% of the blocks), {v[11] / (32 * WR):.2f} per lane-window; "
+          f"rescanned at admission (list full) {v[12] / v[14]:.4f} blocks per lane-slice; whole slice in fp64 {100 * v[13] / v[14]:.3f}% of lane-slices")
+    print(f"  of 'pooled scan', mean per lane-window: cp.async waits {v[5] / (32 * WR):.0f} cycles, fp64 rescans {v[6] / (32 * WR):.0f} cycles")
 post = (v[3] + v[7]) / W
 print(f"  after-barrier work per window: mean {post:.0f}, std {max(v[9] * 1024 / W - post * post, 0) ** 0.5:.0f}")
 print(f"  iterations committed per window: {v[17] / max(v[16], 1):.2f} of 32")

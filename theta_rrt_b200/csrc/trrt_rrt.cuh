@@ -537,20 +537,111 @@ __device__ __forceinline__ void cp_async16(void *smem_dst, const void *gmem_src)
     const unsigned d = (unsigned)__cvta_generic_to_shared(smem_dst);
     asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(d), "l"(gmem_src) : "memory");
 }
-// Nodes [lo, n) of the tree (lo = 0: the whole tree); lowest index on ties inside the range.
+#ifdef TRRT_PHASE_PROF
+// experiment builds only (profiles/tools/phase_prof.py): per-warp clock64 sums of the phases of a window
+__device__ unsigned long long g_phase_prof[24];
+#define TRRT_PROF(...) __VA_ARGS__
+#else
+#define TRRT_PROF(...)
+#endif
+
+// Packed-fp32 prefilter of the staged scan.  The fp64 scan costs 6 fp64-pipe and ~11 warp instructions per (sample, node)
+// pair.  Here each staged tile is converted once to fp32 coordinates relative to an integer origin, every lane streams it
+// against its own sample with f32x2 instructions (FADD2 x2, FMUL2, FFMA2, FMNMX3: ~2.5 instructions per pair, none on the
+// fp64 pipe) and keeps one fp32 minimum per block of SCAN_BLOCK nodes.  fp32 only filters: the blocks that can hold the fp64
+// winner are rescanned with the fp64 arithmetic of TRRT_NODE, so the result is the same bit for bit.  Those blocks are folded
+// in by (d2, index), lexicographically, so the order in which they are rescanned does not matter: the lowest index wins ties.
+//
+// Error bound, per pair (u = 2^-24, v = 2^-53).  X = x - ox exactly; fx = rn32(rn64(X)), so |fx - X| <= e1 = (u + 1.0001 v) M
+// with M the tile's largest |fx| or |fy|.  The sample s = qx - ox is an integer, exact in fp32 (|s| <= 2^24, checked), and
+// a = qx - x = s - X exactly.  dxf = rn32(s - fx) satisfies |dxf - a| <= e1 + u' |dxf| (u' = u / (1 - u)), hence
+// |dxf^2 - a^2| <= e1^2 + 2 (1 + u') e1 |dxf| + (2u' + u'^2) dxf^2, likewise for y.  With G = dxf^2 + dyf^2, |dxf| + |dyf| <=
+// sqrt(2G) and 2 e1 (1 + u') sqrt(2G) <= t G + 2 e1^2 (1 + u')^2 / t for any t > 0:
+//     |G - S| <= t G + 2.0001 u G + 2 e1^2 ((1 + u')^2 / t + 1)        (S = a^2 + b^2)
+// The scan computes F = rn32(fma(dyf, dyf, rn32(dxf^2))); fused or not, |F - G| <= 2.0001 u G.  The kernel's fp64
+// D = rn(rn(dx^2) + rn(dy^2)) with dx = rn(qx - x) satisfies |D - S| <= 4.001 v S.  With t = 2^-16 and G <= F / (1 - 2.0001 u):
+//     |F - D| <= SCAN_REL * F + SCAN_ABS * M^2,   SCAN_REL = 2^-15 (needs 1.55e-5), SCAN_ABS = 2^-30 (needs 2^-31 (1 + 2^-15)).
+// So over a block whose fp32 minimum is m, every D is >= m (1 - SCAN_REL) - c, and the node attaining m has D <= m (1 +
+// SCAN_REL) + c (c = SCAN_ABS * M^2): lower and upper bounds, computed with directed rounding so that they stay bounds.
+// tests/test_scan_prefilter.py checks this inequality on emulated pairs (random and adversarial).
+//
+// Tiles whose |fx| or |fy| exceeds SCAN_FP32_MAX, or is not finite, are not filtered: every lane then scans the whole slice in
+// fp64, and so does a lane whose sample is not exact in fp32.  Coordinates near the map (|X| up to 2^20 pixels) keep c below
+// 2^10 and F finite.
+//
+// SCAN_BLOCK: nodes per fp32 block minimum (a divisor of 2 * TILE_PAIRS).  SCAN_LIST: candidate blocks a lane keeps until the
+// end of its slice; a block admitted while the list holds SCAN_LIST live candidates is rescanned at once instead (near-equal
+// nodes in several blocks: 0.014 blocks per lane-slice on cfg 3).  Measured on B200, cfg 3 (parent fp64 scan 34.4 ms): as
+// shipped (rescans one pair at a time) 30.6 ms; with four pairs per rescan step 32.1 ms at SCAN_BLOCK 16, 31.0 ms at 8,
+// 34.3 ms at 32, 32.2 ms with SCAN_LIST 2 (profiles/r4/NOTES.md).
+constexpr int SCAN_BLOCK = 16, SCAN_LIST = 3;
+constexpr float SCAN_REL = 0x1p-15f, SCAN_ABS = 0x1p-30f, SCAN_FP32_MAX = 0x1p20f;
+static_assert(TILE_PAIRS == 32, "the conversion pass gives lane l pair l of the tile: the pair its own cp.async staged");
+static_assert(SCAN_BLOCK % 2 == 0 && (2 * TILE_PAIRS) % SCAN_BLOCK == 0, "blocks of whole pairs that tile a tile");
+
+__device__ __forceinline__ unsigned long long f32x2_pack(float lo, float hi) {
+    unsigned long long r;
+    asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
+    return r;
+}
+// F of the two nodes of a packed pair: rn(fma(dy, dy, rn(dx * dx))), dx = rn(sx - x), dy = rn(sy - y), for both halves
+__device__ __forceinline__ void f32x2_d2(unsigned long long sx2, unsigned long long sy2, unsigned long long x2, unsigned long long y2,
+                                         float &d0, float &d1) {
+    unsigned long long dx, dy, d;
+    asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(dx) : "l"(sx2), "l"(x2));
+    asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(dy) : "l"(sy2), "l"(y2));
+    asm("mul.rn.f32x2 %0, %1, %1;" : "=l"(d) : "l"(dx));
+    asm("fma.rn.f32x2 %0, %1, %1, %2;" : "=l"(d) : "l"(dy), "l"(d));
+    asm("mov.b64 {%0, %1}, %2;" : "=f"(d0), "=f"(d1) : "l"(d));
+}
+
+struct ScanStats { // counters of the phase-profile build
+    int blocks, rechecked, settled, fp64;
+    long long cyc_wait, cyc_settle; // clock64 in cp.async waits, in fp64 rescans
+};
+
+// Nodes [lo, n) of the tree (lo = 0: the whole tree); lowest index on ties inside the range.  (ox, oy): integer origin of
+// the fp32 coordinates.
 __device__ __forceinline__ void nearest_staged(double2 *tile /* [2][2][TILE_PAIRS] of this warp */, const double *__restrict__ nx,
-                                               const double *__restrict__ ny, int lo, int n, double qx, double qy, double &bd_out, int &bi_out) {
+                                               const double *__restrict__ ny, int lo, int n, double qx, double qy, double ox, double oy,
+                                               double &bd_out, int &bi_out, ScanStats &st) {
     const int lane = threadIdx.x & 31;
     double bd = INFINITY;
     int bi = 0x7fffffff;
     int i = lo;
-#define TRRT_NODE(xv, yv, idx) { double dx = qx - (xv), dy = qy - (yv); double d = dx * dx + dy * dy; if (d < bd) { bd = d; bi = (idx); } }
+    // (d2, index) lexicographic: nodes may be folded in any order, the first minimum wins
+#define TRRT_NODE(xv, yv, idx) { double dx = qx - (xv), dy = qy - (yv); double d = dx * dx + dy * dy; if (d < bd || (d == bd && (idx) < bi)) { bd = d; bi = (idx); } }
     if ((((uintptr_t)nx ^ (uintptr_t)ny) & 15) == 0) { // rows equally aligned
         if (((uintptr_t)(nx + i) & 15) != 0 && i < n) { TRRT_NODE(nx[i], ny[i], i); i++; }
         const double2 *x2 = reinterpret_cast<const double2 *>(nx + i);
         const double2 *y2 = reinterpret_cast<const double2 *>(ny + i);
         const int pairs = (n - i) >> 1;
         const int tiles = (pairs + TILE_PAIRS - 1) / TILE_PAIRS;
+        // the sample relative to the origin, exact in fp32 (else this lane rescans its slice in fp64)
+        const double sxd = qx - ox, syd = qy - oy;
+        bool all64 = !(fabs(sxd) <= 0x1p24 && fabs(syd) <= 0x1p24);
+        bool wide = false; // warp-uniform: a tile that fp32 cannot filter was seen
+        const unsigned long long sx2 = f32x2_pack((float)sxd, (float)sxd), sy2 = f32x2_pack((float)syd, (float)syd);
+        // fp64 rescan of block b, from global memory (the slice was just streamed through L2; the fp64 x of the tile in shared
+        // memory has been overwritten by the fp32 tile).
+        auto settle = [&](int b) {
+            const int q0 = b * (SCAN_BLOCK / 2), q1 = q0 + SCAN_BLOCK / 2 < pairs ? q0 + SCAN_BLOCK / 2 : pairs;
+            TRRT_CHECK(b >= 0 && q0 < pairs && i + 2 * q1 <= n);
+#pragma unroll 1
+            for (int p = q0; p < q1; p++) {
+                const double2 xa = x2[p], ya = y2[p];
+                TRRT_NODE(xa.x, ya.x, i + 2 * p); TRRT_NODE(xa.y, ya.y, i + 2 * p + 1);
+            }
+        };
+        // Candidate list.  U: running minimum of the blocks' upper bounds; an entry holds a block and its lower bound cl.  A
+        // block is admitted when cl <= U at the time it is scanned; an entry whose cl has risen above U is free again, and a
+        // block admitted to a list of live entries only is rescanned at once.  U only falls, and the winner's block has cl <=
+        // D(winner) <= final U <= U at any time: it is admitted when scanned, and then never freed.  A block never admitted,
+        // or freed, has every D > final U >= D(winner): no ties with the winner either.
+        float U = INFINITY, cl[SCAN_LIST];
+        int cb[SCAN_LIST];
+#pragma unroll
+        for (int s = 0; s < SCAN_LIST; s++) { cl[s] = INFINITY; cb[s] = 0; }
         auto issue = [&](int t) { // lanes copy pairs lane, lane + 32 of tile t (only pairs that exist)
             double2 *bx = tile + (t & 1) * 2 * TILE_PAIRS, *by = bx + TILE_PAIRS;
             const int p0 = t * TILE_PAIRS;
@@ -563,25 +654,74 @@ __device__ __forceinline__ void nearest_staged(double2 *tile /* [2][2][TILE_PAIR
         };
         if (tiles > 0) issue(0);
         for (int t = 0; t < tiles; t++) {
+            TRRT_PROF(const long long tw_ = clock64();)
             if (t + 1 < tiles) { issue(t + 1); asm volatile("cp.async.wait_group 1;" ::: "memory"); }
             else asm volatile("cp.async.wait_group 0;" ::: "memory");
-            __syncwarp(); // every lane's part of tile t has landed
-            const double2 *bx = tile + (t & 1) * 2 * TILE_PAIRS, *by = bx + TILE_PAIRS;
+            TRRT_PROF(st.cyc_wait += clock64() - tw_;)
+            // this lane's pair of tile t has landed (its own copy): convert it in place to fp32 (x0, x1, y0, y1)
+            double2 *bx = tile + (t & 1) * 2 * TILE_PAIRS;
+            const double2 *by = bx + TILE_PAIRS;
+            float4 *f4 = reinterpret_cast<float4 *>(bx);
             const int p0 = t * TILE_PAIRS;
             const int cnt = pairs - p0 < TILE_PAIRS ? pairs - p0 : TILE_PAIRS;
-            int p = 0;
-            for (; p + 1 < cnt; p += 2) {
-                const double2 xa = bx[p], ya = by[p], xb = bx[p + 1], yb = by[p + 1];
-                const int b = i + 2 * (p0 + p);
-                TRRT_NODE(xa.x, ya.x, b); TRRT_NODE(xa.y, ya.y, b + 1); TRRT_NODE(xb.x, yb.x, b + 2); TRRT_NODE(xb.y, yb.y, b + 3);
-            }
-            if (p < cnt) {
-                const double2 xa = bx[p], ya = by[p];
-                const int b = i + 2 * (p0 + p);
-                TRRT_NODE(xa.x, ya.x, b); TRRT_NODE(xa.y, ya.y, b + 1);
+            unsigned mbits = 0;
+            if (lane < cnt) {
+                const double2 xa = bx[lane], ya = by[lane];
+                const float4 f = make_float4((float)(xa.x - ox), (float)(xa.y - ox), (float)(ya.x - oy), (float)(ya.y - oy));
+                // max of |f| as bit patterns: NaN sorts above +inf above every finite value
+                mbits = max(max(__float_as_uint(fabsf(f.x)), __float_as_uint(fabsf(f.y))), max(__float_as_uint(fabsf(f.z)), __float_as_uint(fabsf(f.w))));
+                f4[lane] = f;
+            } else f4[lane] = make_float4(0x1p30f, 0x1p30f, 0x1p30f, 0x1p30f); // pads the last block: F ~ 2^61, never a candidate
+            mbits = __reduce_max_sync(0xffffffffu, mbits);
+            __syncwarp(); // the fp32 tile is complete
+            if (mbits > __float_as_uint(SCAN_FP32_MAX)) wide = true;
+            if (!wide) {
+                const float M = __uint_as_float(mbits), c = __fmul_ru(__fmul_ru(M, M), SCAN_ABS);
+                const ulonglong2 *fp = reinterpret_cast<const ulonglong2 *>(f4);
+                for (int pb = 0; pb < cnt; pb += SCAN_BLOCK / 2) {
+                    float m = INFINITY;
+#pragma unroll
+                    for (int k = 0; k < SCAN_BLOCK / 2; k++) {
+                        const ulonglong2 v = fp[pb + k];
+                        float d0, d1;
+                        f32x2_d2(sx2, sy2, v.x, v.y, d0, d1);
+                        m = fminf(m, fminf(d0, d1));
+                    }
+                    const float lb = __fmaf_rd(m, 1.0f - SCAN_REL, -c), ub = __fmaf_ru(m, 1.0f + SCAN_REL, c);
+                    U = fminf(U, ub);
+                    TRRT_PROF(st.blocks++;)
+                    if (lb <= U) {
+                        const int blk = (2 * (p0 + pb)) / SCAN_BLOCK;
+                        bool placed = false;
+#pragma unroll
+                        for (int s = 0; s < SCAN_LIST; s++)
+                            if (!placed && !(cl[s] <= U)) { cl[s] = lb; cb[s] = blk; placed = true; }
+                        if (!placed && !all64) { TRRT_PROF(const long long ts_ = clock64();) settle(blk); TRRT_PROF(st.settled++; st.cyc_settle += clock64() - ts_;) }
+                    }
+                }
             }
             __syncwarp(); // tile t may be overwritten by the copy of tile t + 2
         }
+        // exact fp64 rescan of the live candidates, or of the whole slice
+        TRRT_PROF(const long long ts_ = clock64();)
+        if (all64 || wide) {
+            TRRT_CHECK(i + 2 * pairs <= n);
+#pragma unroll 1
+            for (int p = 0; p < pairs; p++) {
+                const double2 xa = x2[p], ya = y2[p];
+                TRRT_NODE(xa.x, ya.x, i + 2 * p); TRRT_NODE(xa.y, ya.y, i + 2 * p + 1);
+            }
+            TRRT_PROF(st.fp64++;)
+        } else if (tiles > 0) { // (no tile, no block: U is still +inf and the list empty)
+#pragma unroll 1
+            for (int r = 0; r < SCAN_LIST; r++) {
+                int b = -1; // the entry of slot r, if live (one call site of settle)
+#pragma unroll
+                for (int s = 0; s < SCAN_LIST; s++) if (s == r && cl[s] <= U) b = cb[s];
+                if (b >= 0) { settle(b); TRRT_PROF(st.rechecked++;) }
+            }
+        }
+        TRRT_PROF(st.cyc_settle += clock64() - ts_;)
         i += 2 * pairs;
     }
 #pragma unroll 1
@@ -600,14 +740,6 @@ constexpr int SPEC_THREADS = 448, SPEC_BLOCKS_PER_SM = 2;
 // instruction requests at 85% of peak, SM i-cache hit rate 68%, half of all stall samples "no instruction").
 // So the warps of a CTA enter the expansion together: one CTA barrier per window, placed after the (tiny-code)
 // nearest scan; the first warp through a code line fetches it for the others (SM i-cache hit rate 89%, gcc at 47%).
-
-#ifdef TRRT_PHASE_PROF
-// experiment builds only (profiles/tools/phase_prof.py): per-warp clock64 sums of the phases of a window
-__device__ unsigned long long g_phase_prof[24];
-#define TRRT_PROF(...) __VA_ARGS__
-#else
-#define TRRT_PROF(...)
-#endif
 
 template <int G>
 __global__ void __launch_bounds__(SPEC_THREADS, SPEC_BLOCKS_PER_SM) rrt_kernel_spec(const RrtDev a) {
@@ -724,7 +856,10 @@ __global__ void __launch_bounds__(SPEC_THREADS, SPEC_BLOCKS_PER_SM) rrt_kernel_s
                     const double2 sq = pool_q[v][lane];
                     double pd = INFINITY;
                     int pi = 0x7fffffff;
-                    if (lo < hi) nearest_staged(scan_tile, pool_x[v], pool_y[v], lo, hi, sq.x, sq.y, pd, pi);
+                    ScanStats st = {0, 0, 0, 0, 0, 0}; // counted in the phase-profile build only
+                    if (lo < hi) nearest_staged(scan_tile, pool_x[v], pool_y[v], lo, hi, sq.x, sq.y,
+                                                (double)(a.W / 2), (double)(a.H / 2), pd, pi, st); // origin: the map centre
+                    TRRT_PROF(if (lo < hi) { pf[11] += st.rechecked; pf[12] += st.settled; pf[13] += st.fp64; pf[14]++; pf[15] += st.blocks; pf[5] += st.cyc_wait; pf[6] += st.cyc_settle; })
                     const int slot = b0 + (wid - k0v);
                     TRRT_CHECK(slot >= 0 && slot < 2 * NW && lo >= 0 && hi <= n_v && v < NW);
                     pool_d[slot][lane] = pd; pool_i[slot][lane] = pi;
@@ -876,7 +1011,9 @@ __global__ void __launch_bounds__(SPEC_THREADS, SPEC_BLOCKS_PER_SM) rrt_kernel_s
             have = false;
         }
     }
-    TRRT_PROF(if ((threadIdx.x & 31) == 0) for (int i_ = 0; i_ < 24; i_++) if (pf[i_]) atomicAdd(&g_phase_prof[i_], pf[i_]);)
+    // slots 5, 6, 11-15 are per lane (scan prefilter: cycles in cp.async waits and in fp64 rescans; rechecked candidates, blocks
+    // rescanned at admission, fp64 slices, slices, blocks), the others per warp
+    TRRT_PROF(for (int i_ = 0; i_ < 24; i_++) if (pf[i_] && ((threadIdx.x & 31) == 0 || (i_ == 5 || i_ == 6 || (i_ >= 11 && i_ <= 15)))) atomicAdd(&g_phase_prof[i_], pf[i_]);)
 }
 
 } // namespace trrt
