@@ -371,6 +371,57 @@ typedef struct trrt_mission_args {
 size_t trrt_mission_workspace_bytes(int64_t n_missions, int32_t K);
 int trrt_mission_batch(const trrt_mission_args *args, void *stream);
 
+/* ---------------------------------------------------------------------------
+ * legacy_normals.  Seeded sample streams of reference parity: for every seed
+ * i, d_out[d_range[i][0] .. d_range[i][1]) receives
+ * np.random.RandomState(d_seeds[i]).standard_normal(d_range[i][1] - d_range[i][0])
+ * bit for bit (numpy's legacy MT19937 with init_genrand seeding and the polar
+ * method of legacy_gauss), the stream rrt.rand_conf (rrt.py:53-68) consumes
+ * after np.random.seed(seed).  Ranges must not overlap; empty ones are skipped.
+ * numpy takes log(r2) from the host's libm, whose rounding is not correct
+ * rounding, so two steps make up one draw:
+ *   trrt_legacy_normals_draw   every normal whose libm log is forced by the
+ *       error bound of glibc (trrt_libm.h tl_log_decided); an undecided pair
+ *       leaves x2 (and x1) in its slots and appends (slot, r2) to the fixup
+ *       list: d_fix_pos[k] = slot of f*x2, or ~slot when the pair has no f*x1
+ *       slot (odd range); d_fix_r2[k] = r2.  *d_fix_count receives the number
+ *       of undecided pairs, also when it exceeds fix_cap (entries past fix_cap
+ *       are not written: draw again with a larger list).
+ *   trrt_libm_log_batch        HOST: h_out[k] = log(h_in[k]) with this
+ *       process's libm, the one numpy's legacy_gauss calls.
+ *   trrt_legacy_normals_fixup  the first n_fix <= fix_cap list entries with
+ *       d_fix_log[k] = log(d_fix_r2[k]): f = sqrt(-2 log(r2) / r2) and the
+ *       pair's slots become f*x2, f*x1.
+ * ------------------------------------------------------------------------- */
+typedef struct trrt_legacy_normals_args {
+    int64_t n_seeds;
+    const uint32_t *d_seeds;  /* [n_seeds] */
+    const int64_t *d_range;   /* [n_seeds][2] = [begin, end) into d_out */
+    double *d_out;
+    int64_t *d_fix_pos;       /* [fix_cap] */
+    double *d_fix_r2;         /* [fix_cap] */
+    int64_t fix_cap;
+    uint64_t *d_fix_count;    /* [1] */
+    void *d_work;             /* scratch, 256-byte aligned */
+    size_t work_bytes;        /* >= trrt_legacy_normals_workspace_bytes(n_seeds) */
+} trrt_legacy_normals_args;
+
+size_t trrt_legacy_normals_workspace_bytes(int64_t n_seeds);
+int trrt_legacy_normals_draw(const trrt_legacy_normals_args *args, void *stream);
+int trrt_libm_log_batch(const double *h_in, double *h_out, int64_t n);
+int trrt_legacy_normals_fixup(const trrt_legacy_normals_args *args, const double *d_fix_log, int64_t n_fix, void *stream);
+
+/* ---------------------------------------------------------------------------
+ * rand_conf_batch.  rrt.rand_conf (rrt.py:53-68, samples.stream_from_normals)
+ * for n queries of n_samples samples each, from standard normals in draw
+ * order: query q reads d_normals[q * 3 * n_samples .. (q + 1) * 3 * n_samples)
+ * around d_goal[q] = x, y, theta_deg and writes d_sample_xy [n][n_samples][2]
+ * (int32, or int16 when sample_xy_i16) and d_sample_th [n][n_samples], the
+ * sample layout of trrt_rrt_batch.  Only the map size is needed.
+ * ------------------------------------------------------------------------- */
+int trrt_rand_conf_batch(int H, int W, double xystdv, double anglestdv, int64_t n, int32_t n_samples, const double *d_goal,
+                         const double *d_normals, void *d_sample_xy, int32_t sample_xy_i16, double *d_sample_th, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -10,7 +10,10 @@ generate the seeded normals; the stage count and n_active per stage.  On map2 al
 mission (32 missions) and mission_chain over the C oracle (tests/mission_oracle.py) on one host core (64 missions).  The first 16 missions of
 each workload are checked bitwise against the oracle.
 
-    python profiles/tools/mb_missions.py [--out profiles/r3] [--reps 3]
+    python profiles/tools/mb_missions.py [--out profiles/r3] [--reps 3] [--seed-stream host|device]
+
+--seed-stream device draws the seeded normals of the end-to-end runs on the GPU (Planner.missions(seed_stream="device"),
+the same bits); host_seeded_normals_s is still numpy's time for them.
 """
 from __future__ import annotations
 
@@ -75,9 +78,9 @@ def check_oracle(h, free_of, seeds, K, n):
     return bad
 
 
-def run(torch, planner, sg, seeds, K, map_id, reps, tag):
+def run(torch, planner, sg, seeds, K, map_id, reps, tag, seed_stream="host"):
     ev = lambda: torch.cuda.Event(enable_timing=True)  # noqa: E731
-    res = planner.missions(start_goal=sg, seeds=seeds, K=K, map_id=map_id)  # warm-up (and the checked result)
+    res = planner.missions(start_goal=sg, seeds=seeds, K=K, map_id=map_id, seed_stream=seed_stream)  # warm-up (and the checked result)
     torch.cuda.synchronize()
     h = res.host()
     n_seg = h["n_seg"]
@@ -88,7 +91,7 @@ def run(torch, planner, sg, seeds, K, map_id, reps, tag):
     for _ in range(reps):
         torch.cuda.synchronize()
         t = time.perf_counter()
-        planner.missions(start_goal=sg, seeds=seeds, K=K, map_id=map_id)
+        planner.missions(start_goal=sg, seeds=seeds, K=K, map_id=map_id, seed_stream=seed_stream)
         torch.cuda.synchronize()
         e2e.append(time.perf_counter() - t)
     # Theta* alone
@@ -131,7 +134,7 @@ def run(torch, planner, sg, seeds, K, map_id, reps, tag):
         "n_active": [int(v) for v in n_active], "status_counts": {str(k): int(v) for k, v in zip(*np.unique(h["status"], return_counts=True))},
         "e2e_s": e2e, "missions_per_s_e2e": n / float(np.median(e2e)),
         "theta_s": th, "chain_s_device_normals": ch, "missions_per_s_chain": n / float(np.median(ch)),
-        "host_seeded_normals_s": gen_s, "kernel_ms_profiled": split, "tag": tag,
+        "host_seeded_normals_s": gen_s, "kernel_ms_profiled": split, "tag": tag, "seed_stream": seed_stream,
     }
 
 
@@ -139,6 +142,8 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r3"))
     ap.add_argument("--reps", type=int, default=3)
+    ap.add_argument("--seed-stream", choices=("host", "device"), default="host",
+                    help="where the seeded normals of the end-to-end runs are drawn")
     args = ap.parse_args()
     import torch
     if not torch.cuda.is_available():
@@ -153,7 +158,7 @@ def main():
     sg2 = np.concatenate([starts[:, :2], goals[:, :2]], axis=1).astype(np.int32)
     seeds2 = np.arange(4096) + 1_000_000
     p2 = Planner(OccupancyGrid(free2, device="cuda:0"), Params())
-    h2, r2 = run(torch, p2, sg2, seeds2, K, None, args.reps, "map2")
+    h2, r2 = run(torch, p2, sg2, seeds2, K, None, args.reps, "map2", args.seed_stream)
     r2["oracle_mismatches_first16"] = check_oracle(h2, lambda m: free2, seeds2, K, 16)
     # serial references on the same missions
     M.set_map(free2)
@@ -198,7 +203,7 @@ def main():
     sg5 = np.stack([a[:, 1], a[:, 0], b[:, 1], b[:, 0]], 1).astype(np.int32)
     seeds5 = np.arange(16384) + 2_000_000
     p5 = Planner(OccupancyGrid(maps5, device="cuda:0"), Params())
-    h5, r5 = run(torch, p5, sg5, seeds5, K, mid, args.reps, "cfg5")
+    h5, r5 = run(torch, p5, sg5, seeds5, K, mid, args.reps, "cfg5", args.seed_stream)
     r5["oracle_mismatches_first16"] = check_oracle(h5, lambda m: maps5[mid[m]], seeds5, K, 16)
     out["workloads"]["cfg5_16384"] = r5
     os.makedirs(args.out, exist_ok=True)

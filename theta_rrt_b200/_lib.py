@@ -81,6 +81,15 @@ class CMissionArgs(C.Structure):
     ]
 
 
+class CLegacyNormalsArgs(C.Structure):
+    """struct trrt_legacy_normals_args."""
+    _fields_ = [
+        ("n_seeds", C.c_int64), ("d_seeds", C.c_void_p), ("d_range", C.c_void_p), ("d_out", C.c_void_p),
+        ("d_fix_pos", C.c_void_p), ("d_fix_r2", C.c_void_p), ("fix_cap", C.c_int64), ("d_fix_count", C.c_void_p),
+        ("d_work", C.c_void_p), ("work_bytes", C.c_size_t),
+    ]
+
+
 # every symbol include/thetarrt.h declares: name -> (restype, argtypes)
 SIGNATURES = {
     "trrt_version": (C.c_int, []),
@@ -115,6 +124,12 @@ SIGNATURES = {
     "trrt_theta_batch": (C.c_int, [C.POINTER(CThetaArgs), C.c_void_p]),
     "trrt_mission_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int32]),
     "trrt_mission_batch": (C.c_int, [C.POINTER(CMissionArgs), C.c_void_p]),
+    "trrt_legacy_normals_workspace_bytes": (C.c_size_t, [C.c_int64]),
+    "trrt_legacy_normals_draw": (C.c_int, [C.POINTER(CLegacyNormalsArgs), C.c_void_p]),
+    "trrt_libm_log_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64]),
+    "trrt_legacy_normals_fixup": (C.c_int, [C.POINTER(CLegacyNormalsArgs), C.c_void_p, C.c_int64, C.c_void_p]),
+    "trrt_rand_conf_batch": (C.c_int, [C.c_int, C.c_int, C.c_double, C.c_double, C.c_int64, C.c_int32, C.c_void_p,
+                                       C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
 }
 
 _lib = None

@@ -14,6 +14,8 @@
 //   findnearest_kernel    rrt.findnearest over the edge log
 //   mission_*_kernel      main.py missions: segment chain around trrt_rrt_batch, findnearest restarts (trrt_mission.cuh)
 //   theta_kernel<G>       K3: A* / lazy Theta*, G lanes per query, G-ary heap
+//   legacy_normals_kernel / legacy_normals_fixup_kernel  numpy RandomState(seed).standard_normal streams (trrt_rng.cuh)
+//   rand_conf_kernel<XY>  rrt.rand_conf samples from such streams
 //
 // Build: nvcc -gencode arch=compute_100a,code=sm_100a -fmad=false -lineinfo
 // (see theta_rrt_b200/build.py).  No tensor cores: nothing here is a dense
@@ -23,11 +25,16 @@
 #include <stdint.h>
 #include <string.h>
 
+#include <algorithm>
+#include <thread>
+#include <vector>
+
 #include "../../include/thetarrt.h"
 #include "trrt_bike.cuh"
 #include "trrt_device.cuh"
 #include "trrt_los.cuh"
 #include "trrt_mission.cuh"
+#include "trrt_rng.cuh"
 #include "trrt_rrt.cuh"
 
 using namespace trrt;
@@ -1271,6 +1278,90 @@ int trrt_mission_batch(const trrt_mission_args *args, void *stream) {
         mission_commit_kernel<<<(unsigned)na, MISSION_THREADS, 0, st>>>(d, s);
         CUDA_TRY(cudaGetLastError());
     }
+    return TRRT_OK;
+}
+
+size_t trrt_legacy_normals_workspace_bytes(int64_t n_seeds) { return 256; }
+
+static int legacy_normals_check(const trrt_legacy_normals_args *args) {
+    if (!args) return TRRT_ERR_INVALID_ARGUMENT;
+    const trrt_legacy_normals_args &A = *args;
+    if (A.n_seeds < 0 || A.fix_cap < 0 || !A.d_fix_count) return TRRT_ERR_INVALID_ARGUMENT;
+    if (A.n_seeds > 0 && (!A.d_seeds || !A.d_range || !A.d_out || !A.d_work)) return TRRT_ERR_INVALID_ARGUMENT;
+    if (A.fix_cap > 0 && (!A.d_fix_pos || !A.d_fix_r2)) return TRRT_ERR_INVALID_ARGUMENT;
+    return TRRT_OK;
+}
+
+int trrt_legacy_normals_draw(const trrt_legacy_normals_args *args, void *stream) {
+    int e = legacy_normals_check(args);
+    if (e) return e;
+    const trrt_legacy_normals_args &A = *args;
+    cudaStream_t st = (cudaStream_t)stream;
+    CUDA_TRY(cudaMemsetAsync(A.d_fix_count, 0, sizeof(uint64_t), st));
+    if (A.n_seeds == 0) return TRRT_OK;
+    if ((uintptr_t)A.d_work & 255) return TRRT_ERR_INVALID_ARGUMENT;
+    if (A.work_bytes < trrt_legacy_normals_workspace_bytes(A.n_seeds)) return TRRT_ERR_WORKSPACE_TOO_SMALL;
+    CUDA_TRY(cudaMemsetAsync(A.d_work, 0, sizeof(unsigned long long), st));
+    LegacyNormalsDev d;
+    d.n = A.n_seeds; d.seeds = A.d_seeds; d.range = A.d_range; d.out = A.d_out;
+    d.fix_pos = A.d_fix_pos; d.fix_r2 = A.d_fix_r2; d.fix_cap = A.fix_cap;
+    d.fix_count = (unsigned long long *)A.d_fix_count; d.next = (unsigned long long *)A.d_work;
+    int64_t blocks = (A.n_seeds + RNG_WARPS - 1) / RNG_WARPS;
+    if (blocks > (int64_t)sm_count() * 8) blocks = (int64_t)sm_count() * 8;
+    legacy_normals_kernel<<<(unsigned)blocks, RNG_WARPS * 32, 0, st>>>(d);
+    CUDA_TRY(cudaGetLastError());
+    return TRRT_OK;
+}
+
+int trrt_libm_log_batch(const double *h_in, double *h_out, int64_t n) {
+    if (n < 0 || (n > 0 && (!h_in || !h_out))) return TRRT_ERR_INVALID_ARGUMENT;
+    // the host's own libm log, on a few threads: the values are independent
+    const int64_t per = 1 << 16;
+    int nt = (int)std::min<int64_t>((n + per - 1) / per, (int64_t)std::max(1u, std::min(16u, std::thread::hardware_concurrency())));
+    auto run = [=](int64_t lo, int64_t hi) {
+        for (int64_t i = lo; i < hi; i++) h_out[i] = log(h_in[i]);
+    };
+    if (nt <= 1) {
+        run(0, n);
+        return TRRT_OK;
+    }
+    std::vector<std::thread> th;
+    for (int t = 1; t < nt; t++) th.emplace_back(run, n * t / nt, n * (t + 1) / nt);
+    run(0, n / nt);
+    for (auto &x : th) x.join();
+    return TRRT_OK;
+}
+
+int trrt_legacy_normals_fixup(const trrt_legacy_normals_args *args, const double *d_fix_log, int64_t n_fix, void *stream) {
+    int e = legacy_normals_check(args);
+    if (e) return e;
+    const trrt_legacy_normals_args &A = *args;
+    if (n_fix < 0 || n_fix > A.fix_cap || (n_fix > 0 && !d_fix_log)) return TRRT_ERR_INVALID_ARGUMENT;
+    if (n_fix == 0) return TRRT_OK;
+    int64_t blocks = (n_fix + 255) / 256;
+    if (blocks > (int64_t)sm_count() * 16) blocks = (int64_t)sm_count() * 16;
+    legacy_normals_fixup_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(A.d_out, A.d_fix_pos, A.d_fix_r2, d_fix_log, n_fix);
+    CUDA_TRY(cudaGetLastError());
+    return TRRT_OK;
+}
+
+int trrt_rand_conf_batch(int H, int W, double xystdv, double anglestdv, int64_t n, int32_t n_samples, const double *d_goal,
+                         const double *d_normals, void *d_sample_xy, int32_t sample_xy_i16, double *d_sample_th, void *stream) {
+    if (H < 1 || W < 1 || n < 0 || n_samples < 0) return TRRT_ERR_INVALID_ARGUMENT;
+    if (sample_xy_i16 && (H > 32768 || W > 32768)) return TRRT_ERR_MAP_TOO_LARGE;
+    const int64_t total = n * (int64_t)n_samples;
+    if (total == 0) return TRRT_OK;
+    if (!d_goal || !d_normals || !d_sample_xy || !d_sample_th) return TRRT_ERR_INVALID_ARGUMENT;
+    int64_t blocks = (total + 255) / 256;
+    if (blocks > (int64_t)sm_count() * 16) blocks = (int64_t)sm_count() * 16;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (sample_xy_i16)
+        rand_conf_kernel<int16_t><<<(unsigned)blocks, 256, 0, st>>>(H, W, xystdv, anglestdv, n, n_samples, d_goal, d_normals,
+                                                                    (int16_t *)d_sample_xy, d_sample_th);
+    else
+        rand_conf_kernel<int32_t><<<(unsigned)blocks, 256, 0, st>>>(H, W, xystdv, anglestdv, n, n_samples, d_goal, d_normals,
+                                                                    (int32_t *)d_sample_xy, d_sample_th);
+    CUDA_TRY(cudaGetLastError());
     return TRRT_OK;
 }
 

@@ -1,6 +1,7 @@
 /*
  * trrt_libm.h -- deterministic fp64 sin/cos/atan2 built only from IEEE-754
- * basic operations (+ - * / fma, rint, fabs).
+ * basic operations (+ - * / fma, rint, fabs), and the double-double log of
+ * the seeded normal streams (tl_log_dd, at the end).
  *
  * Why this exists: the reference (rrt.py) routes every rotation and angle
  * through libm sin/cos/atan2 (via scipy Rotation and numpy).  CUDA's built-in
@@ -203,6 +204,115 @@ TL_ENTRY double tl_atan2(double y, double x) {
     const double ue = (TL_PI - u) - s;
     const double r = (x > 0.0) ? s + rest : u + ((ue + TL_PI_LO) - rest);
     return (y < 0.0) ? -r : r;
+}
+
+/* ---------------------------------------------------------------------------
+ * log(x) for x in (0, 1) as a double-double, and the test of whether glibc's
+ * log must round it like correct rounding does.
+ *
+ * numpy's legacy polar method (legacy_gauss) calls the host libm's log, whose
+ * results are not correctly rounded (glibc documents < 0.519 ulp).  The device
+ * generator therefore settles only the values whose glibc rounding is forced:
+ * if the exact log lies more than TL_LOG_MARGIN ulp + the error of tl_log_dd
+ * away from every rounding midpoint, any result within 0.5 + 0.019 ulp of it
+ * is the correctly rounded double, which is hi.  The rest ("undecided") are
+ * handed to the host's libm.
+ *
+ * Algorithm: x = 2^k * m with m in [c, 2c), c = RN(sqrt(1/2)) (frexp, exact);
+ * s = (m - 1) / (m + 1), |s| <= 0.17158; log(m) = 2s * F(t), t = s^2,
+ * F(t) = 1 + t/3 + t^2/5 + ... ; log(x) = k*ln2 + log(m).
+ * Error bound (relative to |log x|), derived:
+ *   - m - 1 is exact (Sterbenz), m + 1 = dh + dl exactly (TwoSum); s = sh + sl
+ *     from one division plus the exact fma remainder: |err| <= 2^-103 |s|.
+ *   - t = s^2 in double-double: <= 2^-101 |t|.
+ *   - F: 1, 1/3, 1/5 and the products with t in double-double (each step
+ *     <= 2^-104 relative); R(t) = 1/7 + t/9 + ... + t^9/25 in double Horner
+ *     with coefficients rounded to double: |R err| <= 2^-52, which enters F
+ *     as t^3 |R err| <= 0.02944^3 * 2^-52 < 2^-67.2.  Truncation after the
+ *     t^12/25 term: sum_{j>=13} t^j/(2j+1) <= t^13/27/(1-t) < 2^-70.8.
+ *     F >= 1, so F carries < 2^-67.1 relative error.
+ *   - log(m) = 2s * F, one double-double product: < 2^-67.0 relative.
+ *   - k != 0 means x < c, m in [c, 2c): |log m| <= 0.3466 <= |k ln2| / 2, so
+ *     |log x| >= |k ln2| / 2 >= |log m|; k*ln2 is formed from a 107-bit ln2
+ *     with one exact product: the sum keeps < 2^-67 + 2^-103 relative.
+ * TL_LOG_EPS = 2^-66 is the bound used (2x headroom over the derivation);
+ * tests/test_legacy_normals.py checks it against decimal at 60 digits.
+ * ------------------------------------------------------------------------- */
+#define TL_LOG_EPS 1.3552527156068805e-20   /* 2^-66 */
+#define TL_LOG_MARGIN 0.03125               /* 2^-5 ulp > glibc's 0.019-ulp excess over correct rounding */
+
+TL_FN void tl_two_sum(double a, double b, double *s, double *e) {
+    const double x = a + b, bb = x - a;
+    *e = (a - (x - bb)) + (b - bb);
+    *s = x;
+}
+TL_FN void tl_fast_two_sum(double a, double b, double *s, double *e) { /* |a| >= |b| or a = 0 */
+    const double x = a + b;
+    *e = b - (x - a);
+    *s = x;
+}
+/* (ah + al) * (bh + bl), normalised */
+TL_FN void tl_dd_mul(double ah, double al, double bh, double bl, double *ph, double *pl) {
+    const double p = ah * bh;
+    const double e = fma(ah, bh, -p) + fma(ah, bl, al * bh);
+    tl_fast_two_sum(p, e, ph, pl);
+}
+/* (ah + al) + (bh + bl), normalised */
+TL_FN void tl_dd_add(double ah, double al, double bh, double bl, double *sh, double *sl) {
+    double s, e;
+    tl_two_sum(ah, bh, &s, &e);
+    e += al + bl;
+    tl_fast_two_sum(s, e, sh, sl);
+}
+
+TL_ENTRY void tl_log_dd(double x, double *hi, double *lo) {
+    int k;
+    double m = frexp(x, &k); /* x = m * 2^k, m in [1/2, 1) */
+    if (m < 0.7071067811865476) { m *= 2.0; k -= 1; }
+    const double num = m - 1.0;
+    double dh, dl;
+    tl_two_sum(m, 1.0, &dh, &dl);
+    const double sh = num / dh;
+    const double sl = fma(-sh, dl, fma(-sh, dh, num)) / dh;
+    double th, tl;
+    tl_dd_mul(sh, sl, sh, sl, &th, &tl);
+    /* R(t) = sum_{j=3..12} t^(j-3) / (2j+1) */
+    double r = 1.0 / 25;
+    r = fma(r, th, 1.0 / 23); r = fma(r, th, 1.0 / 21); r = fma(r, th, 1.0 / 19); r = fma(r, th, 1.0 / 17);
+    r = fma(r, th, 1.0 / 15); r = fma(r, th, 1.0 / 13); r = fma(r, th, 1.0 / 11); r = fma(r, th, 1.0 / 9);
+    r = fma(r, th, 1.0 / 7);
+    double fh, fl;
+    tl_dd_mul(th, tl, r, 0.0, &fh, &fl);
+    tl_dd_add(0.2, -1.1102230246251566e-17, fh, fl, &fh, &fl);            /* 1/5 */
+    tl_dd_mul(th, tl, fh, fl, &fh, &fl);
+    tl_dd_add(0.3333333333333333, 1.850371707708594e-17, fh, fl, &fh, &fl); /* 1/3 */
+    tl_dd_mul(th, tl, fh, fl, &fh, &fl);
+    tl_dd_add(1.0, 0.0, fh, fl, &fh, &fl);
+    double lh, ll;
+    tl_dd_mul(2.0 * sh, 2.0 * sl, fh, fl, &lh, &ll);                         /* log(m) */
+    if (k != 0) {
+        const double L2H = 0.6931471805599453, L2L = 2.3190468138462996e-17; /* ln 2 */
+        const double kd = (double)k;
+        const double p = kd * L2H;
+        const double pe = fma(kd, L2H, -p) + kd * L2L;
+        tl_dd_add(p, pe, lh, ll, &lh, &ll);
+    }
+    *hi = lh;
+    *lo = ll;
+}
+
+/* 1 when hi (= RN(hi + lo)) is the double that glibc's log returns: the exact value, within TL_LOG_EPS of hi + lo,
+   is more than TL_LOG_MARGIN ulp away from the rounding midpoint on lo's side (the one on the other side is at
+   least a quarter ulp away).  hi != 0. */
+TL_FN int tl_log_decided(double hi, double lo) {
+    const double ahi = fabs(hi);
+    int e;
+    const double f = frexp(ahi, &e);
+    const double ulp = ldexp(1.0, e - 53);
+    /* toward zero from a power of two the spacing of the doubles halves */
+    const double side = (f == 0.5 && (lo < 0.0) != (hi < 0.0) && lo != 0.0) ? 0.5 * ulp : ulp;
+    const double dist = 0.5 * side - fabs(lo);
+    return dist > TL_LOG_MARGIN * ulp + 2.0 * TL_LOG_EPS * ahi;
 }
 
 #endif /* TRRT_LIBM_H */

@@ -10,6 +10,7 @@
 // s are exactly the first n_active[s] slots and no compaction is needed between stages.
 #pragma once
 #include "trrt_bike.cuh"
+#include "trrt_rng.cuh"
 
 namespace trrt {
 
@@ -168,18 +169,11 @@ __global__ void __launch_bounds__(MISSION_THREADS) mission_stage_kernel(const Mi
         for (int j = threadIdx.x; j < K - 1; j += blockDim.x) { sxy[2 * j] = 0; sxy[2 * j + 1] = 0; sth[j] = 0.0; }
         return;
     }
-    // rrt.py:53-68 (samples.stream_from_normals): x = gx + (xystdv*H)*z0, clipped to [0, H-1] and truncated; theta wrapped
     const double gx = row[3], gy = row[4], gth = standardangle(row[5]);
     const double sx = a.xystdv * (double)a.H, sy = a.xystdv * (double)a.W, hm = (double)(a.H - 1), wm = (double)(a.W - 1);
     const double *z = a.normals + off;
-    for (int j = threadIdx.x; j < K - 1; j += blockDim.x) {
-        double x = gx + sx * z[3 * j], y = gy + sy * z[3 * j + 1];
-        x = x < 0.0 ? 0.0 : (x > hm ? hm : x);
-        y = y < 0.0 ? 0.0 : (y > wm ? wm : y);
-        sxy[2 * j] = (int32_t)trunc_ll(x);
-        sxy[2 * j + 1] = (int32_t)trunc_ll(y);
-        sth[j] = standardangle(gth + a.anglestdv * z[3 * j + 2]);
-    }
+    for (int j = threadIdx.x; j < K - 1; j += blockDim.x)
+        rand_conf_sample(z + 3 * j, gx, gy, gth, sx, sy, hm, wm, a.anglestdv, sxy[2 * j], sxy[2 * j + 1], sth[j]);
 }
 
 // main.py:68-79 after rrt.rrt returned, for the mission in slot blockIdx.x: the segment record, rrt.findnearest when

@@ -138,15 +138,16 @@ def mission_records(h, m):
     return out
 
 
-def plan_batch(image, starts, goals, seeds, K=None):
+def plan_batch(image, starts, goals, seeds, K=None, seed_stream="host"):
     """plan() for many (start, goal, seed) missions on one map: Theta* (A* with THETASTAR=False) waypoints and the
     segment chain of every mission in one batched device call (Planner.missions).  Mission m draws its samples like
-    plan() after np.random.seed(seeds[m]).  Returns one mission_records() entry per mission."""
+    plan() after np.random.seed(seeds[m]), with numpy on the host (seed_stream="host") or on the device
+    (seed_stream="device", the same bits).  Returns one mission_records() entry per mission."""
     set_map(image)
     from . import _context
     p = _context.current_planner()
     sg = np.concatenate([np.asarray(starts, np.int32).reshape(-1, 2), np.asarray(goals, np.int32).reshape(-1, 2)], axis=1)
-    h = p.missions(start_goal=sg, seeds=seeds, K=K if K is not None else int(p.params.K)).host()
+    h = p.missions(start_goal=sg, seeds=seeds, K=K if K is not None else int(p.params.K), seed_stream=seed_stream).host()
     return [mission_records(h, m) for m in range(len(sg))]
 
 

@@ -9,6 +9,7 @@ There is no CPU fallback.
 from __future__ import annotations
 
 import ctypes as C
+import operator
 from dataclasses import dataclass, field
 
 import numpy as np
@@ -117,6 +118,24 @@ class MissionResult:
         if self.route is not None:
             out["route"] = self.route.host()
         return out
+
+
+SEED_STREAMS = ("host", "device")
+
+
+def legacy_seeds(seeds):
+    """Seeds of np.random.RandomState(int) as uint32 [n]; raises numpy's ValueError outside [0, 2**32)."""
+    a = np.asarray(seeds).reshape(-1)
+    if a.dtype.kind == "O" or a.dtype.kind == "b":
+        a = np.array([operator.index(v) for v in a], dtype=object)
+        if any(v < 0 or v > 0xffffffff for v in a):
+            raise ValueError("Seed must be between 0 and 2**32 - 1")
+        return a.astype(np.uint32)
+    if a.dtype.kind not in "iu":
+        raise TypeError(f"seeds must be integers, got {a.dtype}")
+    if a.size and (int(a.min()) < 0 or int(a.max()) > 0xffffffff):
+        raise ValueError("Seed must be between 0 and 2**32 - 1")
+    return a.astype(np.uint32)
 
 
 def mission_schedule(n_seg):
@@ -624,9 +643,96 @@ class Planner:
             res._keep = (sg, mid, order)
         return res
 
+    # ------------------------------------------------------------------ seeded streams
+    def legacy_normals(self, seeds, counts, fix_cap=None):
+        """np.random.RandomState(seeds[i]).standard_normal(counts[i]) for every i, bit for bit, drawn on the device
+        (trrt_legacy_normals_draw).  Returns (normals float64 [sum(counts)], ranges int64 [n, 2]): seed i's stream is
+        normals[ranges[i, 0]:ranges[i, 1]], both on the device.  Integer seeds in [0, 2**32) only (init_genrand
+        seeding).  The logs the device cannot settle (about 6 % of the pairs) come from this process's libm, the one
+        numpy calls: their count is the one host read, then the r2 values travel to pinned memory and the logs back.
+        fix_cap: room of the list of such pairs (default a sixteenth of the normals); an overflow draws once more with
+        the reported count."""
+        seeds = legacy_seeds(seeds)
+        counts = np.asarray(counts, dtype=np.int64).reshape(-1)
+        n = len(seeds)
+        if len(counts) != n:
+            raise ValueError(f"{len(counts)} counts for {n} seeds")
+        if n and counts.min() < 0:
+            raise ValueError("counts must be >= 0")
+        rng = np.zeros((n, 2), np.int64)
+        rng[:, 1] = np.cumsum(counts)
+        rng[1:, 0] = rng[:-1, 1]
+        total = int(rng[-1, 1]) if n else 0
+        dev = self.device
+        with torch.cuda.device(dev):
+            out = torch.empty(total, dtype=torch.float64, device=dev)
+            rng_d = self._dev(rng, torch.int64) if n else torch.zeros((0, 2), dtype=torch.int64, device=dev)
+            if total == 0:
+                return out, rng_d
+            seeds_d = self._dev(seeds.view(np.int32), torch.int32)
+            cap = int(fix_cap) if fix_cap is not None else total // 16 + 1024
+            count = torch.zeros(1, dtype=torch.int64, device=dev)
+            work = self._scratch("legacy_normals", self.lib.trrt_legacy_normals_workspace_bytes(n))
+            for _ in range(2):  # a second draw only when the fixup list overflowed
+                fix_pos = torch.empty(max(cap, 1), dtype=torch.int64, device=dev)
+                fix_r2 = torch.empty(max(cap, 1), dtype=torch.float64, device=dev)
+                a = _lib.CLegacyNormalsArgs(n_seeds=n, d_seeds=seeds_d.data_ptr(), d_range=rng_d.data_ptr(), d_out=out.data_ptr(),
+                                            d_fix_pos=fix_pos.data_ptr(), d_fix_r2=fix_r2.data_ptr(), fix_cap=cap,
+                                            d_fix_count=count.data_ptr(), d_work=work.data_ptr(), work_bytes=work.numel())
+                _lib.check(self.lib.trrt_legacy_normals_draw(C.byref(a), self._stream()), "trrt_legacy_normals_draw")
+                n_fix = int(count.cpu()[0])  # the one host read
+                if n_fix <= cap:
+                    break
+                cap = n_fix  # the list overflowed: once more with room for every entry
+            if n_fix:
+                h_r2, h_log = self._pinned("legacy_normals", n_fix)
+                h_r2.copy_(fix_r2[:n_fix], non_blocking=True)
+                torch.cuda.current_stream(dev).synchronize()
+                _lib.check(self.lib.trrt_libm_log_batch(h_r2.data_ptr(), h_log.data_ptr(), n_fix), "trrt_libm_log_batch")
+                d_log = h_log.to(dev, non_blocking=True)
+                _lib.check(self.lib.trrt_legacy_normals_fixup(C.byref(a), d_log.data_ptr(), n_fix, self._stream()),
+                           "trrt_legacy_normals_fixup")
+        return out, rng_d
+
+    def _pinned(self, key, n):
+        """Two grow-only pinned float64 host buffers of at least n values per key and stream.  A call that reuses them has
+        synchronised the stream first, so the copies of the previous call that read them have completed."""
+        key = (key, torch.cuda.current_stream(self.device).cuda_stream)
+        cur = getattr(self, "_pin", {}).get(key)
+        if cur is None or cur[0].numel() < n:
+            cur = tuple(torch.empty(max(int(n), 1024), dtype=torch.float64).pin_memory() for _ in range(2))
+            self.__dict__.setdefault("_pin", {})[key] = cur
+        return cur[0][:n], cur[1][:n]
+
+    def rand_conf(self, goals, seeds, K=None, xy_dtype=torch.int32, params=None):
+        """The K-1 rand_conf samples (rrt.py:53-68) of query q after np.random.seed(seeds[q]), around goals[q] float64
+        [q, 3] = (x, y, theta_deg), i.e. samples.make_stream(goal, K-1, seeds[q], ...) per query, drawn on the device
+        (legacy_normals, then trrt_rand_conf_batch).  Returns (sample_xy xy_dtype [q, K-1, 2], sample_th float64
+        [q, K-1]) on the device, the sample layout of rrt(); xy_dtype is torch.int32 or torch.int16."""
+        P = params or self.params
+        K = int(K if K is not None else P.K)
+        if K < 1:
+            raise ValueError("K must be >= 1")
+        if xy_dtype not in (torch.int32, torch.int16):
+            raise ValueError("xy_dtype must be torch.int32 or torch.int16")
+        with torch.cuda.device(self.device):
+            goals = self._dev(goals, torch.float64).reshape(-1, 3)
+            nq, S = goals.shape[0], K - 1
+            seeds = legacy_seeds(seeds)
+            if len(seeds) != nq:
+                raise ValueError(f"{len(seeds)} seeds for {nq} queries")
+            nz, _ = self.legacy_normals(seeds, np.full(nq, 3 * S, np.int64))
+            sxy = torch.empty((nq, S, 2), dtype=xy_dtype, device=self.device)
+            sth = torch.empty((nq, S), dtype=torch.float64, device=self.device)
+            g = self.grid
+            _lib.check(self.lib.trrt_rand_conf_batch(g.H, g.W, float(P.xystdv), float(P.anglestdv), nq, S, goals.data_ptr(),
+                                                     nz.data_ptr(), sxy.data_ptr(), int(xy_dtype == torch.int16),
+                                                     sth.data_ptr(), self._stream()), "trrt_rand_conf_batch")
+        return sxy, sth
+
     # ------------------------------------------------------------------ main.py missions
     def missions(self, start_goal=None, waypoints=None, seeds=None, normals=None, normal_range=None, map_id=None, K=None,
-                 thetastar=None, path_cap=None, params=None) -> MissionResult:
+                 thetastar=None, path_cap=None, params=None, seed_stream="host") -> MissionResult:
         """main.plan for a batch of missions (main.py:56-84): a route, then one RRT per consecutive waypoint pair with
         the headings of main.chain, restarting from the rrt.findnearest node once a segment has failed.  The segment
         chain runs on the device (trrt_mission_batch): per stage, one kernel builds every mission's start, goal and
@@ -636,7 +742,8 @@ class Planner:
         Params.THETASTAR) over `start_goal` int32 [B, 4] = (sx, sy, gx, gy).  The route lengths are read back once to
         build the schedule; nothing else waits for the device.
         Samples: `seeds` gives mission m the normals of np.random.RandomState(seeds[m]) in draw order, i.e. the stream
-        main.chain consumes after np.random.seed(seeds[m]) (reference parity).  Or `normals`: a float64 stream (e.g. a
+        main.chain consumes after np.random.seed(seeds[m]) (reference parity), drawn by numpy on the host
+        (seed_stream="host") or on the device (seed_stream="device", legacy_normals: the same bits).  Or `normals`: a float64 stream (e.g. a
         device torch.randn tensor) with `normal_range` int64 [B, 2] = [begin, end) per mission, or a [B, L] tensor with one
         row per mission; mission m needs 3 * (K-1) * n_seg[m] values.
         map_id: [B] map of each mission.  path_cap: path rows kept per mission (default n_seg_max * K, which never
@@ -647,6 +754,8 @@ class Planner:
             raise ValueError("K must be >= 2")
         if (seeds is None) == (normals is None):
             raise ValueError("pass exactly one of seeds and normals")
+        if seed_stream not in SEED_STREAMS:
+            raise ValueError(f"seed_stream must be one of {SEED_STREAMS}")
         g = self.grid
         with torch.cuda.device(self.device):
             route = None
@@ -678,14 +787,19 @@ class Planner:
                 seeds = np.asarray(seeds).reshape(-1)
                 if len(seeds) != B:
                     raise ValueError(f"{len(seeds)} seeds for {B} missions")
-                rng = np.zeros((B, 2), np.int64)
-                rng[:, 1] = np.cumsum(need)
-                rng[1:, 0] = rng[:-1, 1]
-                flat = np.empty(int(need.sum()), np.float64)
-                for m in range(B):
-                    if need[m]:
-                        flat[rng[m, 0]:rng[m, 1]] = np.random.RandomState(int(seeds[m])).standard_normal(int(need[m]))
-                nz = self._dev(flat, torch.float64) if flat.size else torch.zeros(1, dtype=torch.float64, device=self.device)
+                if seed_stream == "device":
+                    nz, rng_d = self.legacy_normals(seeds, need)
+                    if nz.numel() == 0:
+                        nz = torch.zeros(1, dtype=torch.float64, device=self.device)
+                else:
+                    rng = np.zeros((B, 2), np.int64)
+                    rng[:, 1] = np.cumsum(need)
+                    rng[1:, 0] = rng[:-1, 1]
+                    flat = np.empty(int(need.sum()), np.float64)
+                    for m in range(B):
+                        if need[m]:
+                            flat[rng[m, 0]:rng[m, 1]] = np.random.RandomState(int(seeds[m])).standard_normal(int(need[m]))
+                    nz = self._dev(flat, torch.float64) if flat.size else torch.zeros(1, dtype=torch.float64, device=self.device)
             else:
                 nz = self._dev(normals, torch.float64)
                 if normal_range is None:
@@ -706,7 +820,8 @@ class Planner:
                                      f"need {int(need[m])} (3 * (K-1) per segment)")
                 if nz.numel() == 0:
                     nz = torch.zeros(1, dtype=torch.float64, device=self.device)
-            rng_d = self._dev(rng, torch.int64) if B else None
+            if not (seeds is not None and seed_stream == "device"):
+                rng_d = self._dev(rng, torch.int64) if B else None
             order_d = self._dev(order, torch.int32)
             mid = self._map_ids(map_id, B)
             if path_cap is None:

@@ -15,7 +15,7 @@ import builtins
 import numpy as np
 
 from . import _context, samples
-from .planner import (IT_ARC_BLOCKED, IT_NOT_RUN, IT_QRAND_BLOCKED, IT_QRAND_IN_TREE, Planner, RrtResult)
+from .planner import (IT_ARC_BLOCKED, IT_NOT_RUN, IT_QRAND_BLOCKED, IT_QRAND_IN_TREE, SEED_STREAMS, Planner, RrtResult)
 from .samples import standardangle as _standardangle_np
 
 
@@ -153,9 +153,13 @@ def rrt(start, goal, debug=False):
     return sol, G, cameFrom
 
 
-def rrt_batch(starts, goals, seeds=None, sample_xy=None, sample_th=None, K=None, logs=False, lanes=0) -> RrtResult:
+def rrt_batch(starts, goals, seeds=None, sample_xy=None, sample_th=None, K=None, logs=False, lanes=0,
+              seed_stream="host") -> RrtResult:
     """Many independent rrt() calls in one launch.  Either pass per-query `seeds` (the stream of query q equals
-    `np.random.seed(seeds[q])` followed by K-1 rand_conf calls) or explicit sample arrays."""
+    `np.random.seed(seeds[q])` followed by K-1 rand_conf calls, drawn by numpy on the host with seed_stream="host" or
+    on the device with seed_stream="device", Planner.rand_conf: the same bits) or explicit sample arrays."""
+    if seed_stream not in SEED_STREAMS:
+        raise ValueError(f"seed_stream must be one of {SEED_STREAMS}")
     p = _context.current_planner()
     P = p.params
     K = int(K or P.K)
@@ -167,6 +171,9 @@ def rrt_batch(starts, goals, seeds=None, sample_xy=None, sample_th=None, K=None,
         if seeds is None:
             raise ValueError("pass seeds or sample arrays")
         nq = len(starts)
+        if seed_stream == "device":
+            sample_xy, sample_th = p.rand_conf(goals, seeds, K)
+            return p.rrt(starts, goals, sample_xy, sample_th, K=K, logs=logs, lanes=lanes)
         sample_xy = np.empty((nq, K - 1, 2), np.int32)
         sample_th = np.empty((nq, K - 1), np.float64)
         for q in range(nq):
