@@ -360,7 +360,7 @@ __global__ void __launch_bounds__(128) arc_pixels_kernel(int H, int W, int64_t n
         const double bx = v[0], by = v[1], lx = v[2], ly = v[3];
         const long long xc = trunc_ll(v[5]), yc = trunc_ll(v[6]), r = trunc_ll(v[7]);
         ArcTest A;
-        A.iccx = v[5]; A.iccy = v[6]; A.usteer = v[4]; A.ready = false; A.literal_ready = false;
+        A.iccx = v[5]; A.iccy = v[6]; A.usteer = v[4]; A.ready = false;
         const long long tmax = circle_tmax(r);
         for (long long base = 0; base <= tmax; base += 32) {
             const long long t = base + lane;
@@ -415,9 +415,9 @@ __global__ void clearance_batch_kernel(const uint32_t *__restrict__ bits, int H,
     const Rot R = rot_make(th);
     double bx, by;
     rot_apply(R, P.bikelength, 0.0, bx, by);
-    clear[2 * i] = los_lane(m, trunc_ll(x), trunc_ll(y), trunc_ll(bx + x), trunc_ll(by + y), nullptr) ? 1 : 0;
+    clear[2 * i] = los_lane(m, trunc_ll(x), trunc_ll(y), trunc_ll(bx + x), trunc_ll(by + y)) ? 1 : 0;
     rot_apply(R, P.bikelength * P.frontclearance, 0.0, bx, by);
-    clear[2 * i + 1] = los_lane(m, trunc_ll(x), trunc_ll(y), trunc_ll(bx + x), trunc_ll(by + y), nullptr) ? 1 : 0;
+    clear[2 * i + 1] = los_lane(m, trunc_ll(x), trunc_ll(y), trunc_ll(bx + x), trunc_ll(by + y)) ? 1 : 0;
 }
 __global__ void anglediff_batch_kernel(int64_t n, const double *__restrict__ in, double *__restrict__ out) {
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;

@@ -39,7 +39,8 @@ __device__ __forceinline__ double standardangle(double a) {
 // scipy Rotation.from_euler('z', deg, degrees=True) -> quaternion (0,0,z,w)
 __device__ __forceinline__ void quat_z(double deg, double &z, double &w) {
     double h = (deg * (TRRT_PI / 180.0)) / 2.0;
-    tl_sincos(h, &z, &w);
+    const tl_sc r = tl_sincos_v(h);
+    z = r.s; w = r.c;
 }
 
 // Rotation.from_euler('z',deg,degrees=True).as_matrix(), the entries apply() needs
@@ -52,18 +53,18 @@ __host__ __device__ __forceinline__ Rot rot_from_quat(double z, double w) {
     return R;
 }
 __host__ __device__ __forceinline__ Rot rot_make(double deg) {
-    double z, w;
     double h = (deg * (TRRT_PI / 180.0)) / 2.0;
-    tl_sincos(h, &z, &w);
-    return rot_from_quat(z, w);
+    const tl_sc r = tl_sincos_v(h);
+    return rot_from_quat(r.s, r.c);
 }
 // Rotation.apply([vx,vy,0])[:2] (the compiled backend contracts the dot products)
 __device__ __forceinline__ void rot_apply(const Rot &R, double vx, double vy, double &ox, double &oy) {
     ox = fma(R.m00, vx, R.m01 * vy);
     oy = fma(R.m10, vx, R.m00 * vy);
 }
-// Rotation.from_euler('z',deg,degrees=True).apply([vx,vy,0])[:2]
-__device__ __noinline__ void rotz(double deg, double vx, double vy, double &ox, double &oy) {
+// Rotation.from_euler('z',deg,degrees=True).apply([vx,vy,0])[:2].  Inlined (one tl_sincos_v call and six flops): as a call
+// its two results came back through the caller's stack (cfg-3 kernel, mean of 5: 28.94 ms inlined, 29.48 ms as a call).
+__device__ __forceinline__ void rotz(double deg, double vx, double vy, double &ox, double &oy) {
     Rot R = rot_make(deg);
     rot_apply(R, vx, vy, ox, oy);
 }
@@ -114,8 +115,9 @@ __device__ __forceinline__ double arclength_to_angle(double radius, double arcle
     return arclength * 360 / (TRRT_PI * 2 * radius);
 }
 
-// np.linalg.solve, 2x2 (dgesv: partial pivoting, reciprocal-pivot scaling). false = LinAlgError
-__device__ __noinline__ bool solve2(double a1, double b1, double a2, double b2, double c1, double c2, double &x1, double &x2) {
+// np.linalg.solve, 2x2 (dgesv: partial pivoting, reciprocal-pivot scaling). false = LinAlgError.  Inlined at its two call
+// sites in steer(): as a call its results came back through the caller's stack (cfg 3: 28.94 ms inlined, 29.70 ms as a call).
+__device__ __forceinline__ bool solve2(double a1, double b1, double a2, double b2, double c1, double c2, double &x1, double &x2) {
     if (fabs(a2) > fabs(a1)) {
         double t;
         t = a1; a1 = a2; a2 = t;
@@ -149,8 +151,9 @@ struct Steer {
     bool straight;                       // u = (0, None, None, 1)
 };
 
-// rrt.py:526-541
-__device__ __noinline__ void steer_straight(const BikeParams &P, double ox, double oy, double theta, double gx, double gy, Steer &o) {
+// rrt.py:526-541.  Inlined at its two call sites in steer(): as a call it took the caller's Steer by reference, which put
+// that Steer on the stack (cfg 3: 28.94 ms inlined, 38.91 ms as a call).
+__device__ __forceinline__ void steer_straight(const BikeParams &P, double ox, double oy, double theta, double gx, double gy, Steer &o) {
     double vx = gx - ox, vy = gy - oy;
     double nv = norm2(vx, vy);
     if (nv > 0.000001) {
@@ -277,8 +280,13 @@ __device__ __forceinline__ void steer(const BikeParams &P, double ox, double oy,
 
 // rrt.py:272-304 (dist = u[3], already divided by 3 by the caller, rrt.py:170)
 // bf = Rz(theta)*[bikelength,0] as computed by steer() for the same origin bike (rrt.py:277-279 recomputes it)
-__device__ __noinline__ void drive_bf(const BikeParams &P, double ox, double oy, double bfx, double bfy, double usteer, double iccx,
-                                      double iccy, double rad, double dist, double &fx, double &fy, double &fang) {
+// A call (the re-drive is the rarer branch of the expansion) whose pose comes back by value, in registers: through
+// reference parameters it came back through the caller's stack.
+struct Pose {
+    double x, y, theta;
+};
+__device__ __noinline__ Pose drive_bf(const BikeParams &P, double ox, double oy, double bfx, double bfy, double usteer, double iccx,
+                                      double iccy, double rad, double dist) {
     double angle = arclength_to_angle(rad, dist);
     double b1x, b1y;
     rot_apply(P.r180, bfx, bfy, b1x, b1y);
@@ -292,15 +300,18 @@ __device__ __noinline__ void drive_bf(const BikeParams &P, double ox, double oy,
     bfx = iccx + bfx; bfy = iccy + bfy;
     b1x = iccx + b1x; b1y = iccy + b1y;
     double px = 0.5 * (b1x + bfx), py = 0.5 * (b1y + bfy);
-    fang = -anglebetween(1, 0, bfx - px, bfy - py);
-    fx = px; fy = py;
+    Pose f;
+    f.theta = -anglebetween(1, 0, bfx - px, bfy - py);
+    f.x = px; f.y = py;
+    return f;
 }
 // rrt.py:272-304 from scratch (single-step entry point)
 __device__ __forceinline__ void drive(const BikeParams &P, double ox, double oy, double theta, double usteer, double iccx, double iccy,
                                       double rad, double dist, double &fx, double &fy, double &fang) {
     double bfx, bfy;
     rotz(theta, P.bikelength, 0.0, bfx, bfy);
-    drive_bf(P, ox, oy, bfx, bfy, usteer, iccx, iccy, rad, dist, fx, fy, fang);
+    const Pose f = drive_bf(P, ox, oy, bfx, bfy, usteer, iccx, iccy, rad, dist);
+    fx = f.x; fy = f.y; fang = f.theta;
 }
 
 // Python round(): half to even
@@ -344,10 +355,8 @@ struct ArcTest {
     // inputs of search.getArc (search.py:144-182) for the non-straight case
     double iccx, iccy, usteer;
     double u1x, u1y, u2x, u2y, n1, n2; // begin - icc, land - icc and their squared lengths
-    double beginangle, endangle, diff;
-    double sb, cb, se, ce; // quaternions of beginangle / endangle (literal path)
     int diff_lt_180;       // -1 unknown, else the outcome of `diff < 180` (search.py:170)
-    bool ready, literal_ready;
+    bool ready;
 };
 
 // The reference keeps a circle pixel when the wrapped angle differences `forwardofbegin` and
@@ -366,31 +375,32 @@ __device__ __forceinline__ int cross_sign(double v2x, double v2y, double v1x, do
     return c > 0 ? 1 : -1;
 }
 
-__device__ __noinline__ void arc_literal_prepare(ArcTest &A) {
-    A.beginangle = anglebetween(1, 0, A.u1x, A.u1y);
-    A.endangle = anglebetween(1, 0, A.u2x, A.u2y);
-    quat_z(A.beginangle, A.sb, A.cb);
-    quat_z(A.endangle, A.se, A.ce);
-    double d = (A.usteer < 0) ? anglediff_q(A.sb, A.cb, A.se, A.ce) : anglediff_q(A.se, A.ce, A.sb, A.cb);
+// The literal path (search.py:161-170).  Real calls, rare (|sin| <= 1e-9), that take the arc's vectors by value: a reference
+// to the caller's ArcTest would put it on the stack.  Each call recomputes the begin / end quaternions from (u1, u2).
+// `diff < 180` (search.py:170), the wrapped (endangle - beginangle) for a left turn, (beginangle - endangle) otherwise
+__device__ __noinline__ int arc_literal_diff_lt180(double u1x, double u1y, double u2x, double u2y, double usteer) {
+    double sb, cb, se, ce;
+    quat_z(anglebetween(1, 0, u1x, u1y), sb, cb);
+    quat_z(anglebetween(1, 0, u2x, u2y), se, ce);
+    double d = (usteer < 0) ? anglediff_q(sb, cb, se, ce) : anglediff_q(se, ce, sb, cb);
     if (d < 0) d = 360 + d;
-    A.diff = d;
-    A.literal_ready = true;
+    return d < 180 ? 1 : 0;
 }
-
-// literal evaluation of one of the two per-pixel differences (which: 0 = forwardofbegin, 1 = backwardofgoal)
-__device__ __noinline__ bool arc_literal_ge0(ArcTest &A, double vx, double vy, int which) {
-    if (!A.literal_ready) arc_literal_prepare(A);
-    double pxangle = anglebetween(1, 0, vx, vy);
-    double sp, cp;
-    quat_z(pxangle, sp, cp);
+// one of the two per-pixel differences (which: 0 = forwardofbegin, 1 = backwardofgoal) is >= 0
+__device__ __noinline__ bool arc_literal_ge0(double u1x, double u1y, double u2x, double u2y, double usteer, double vx, double vy, int which) {
+    double sb, cb, se, ce, sp, cp;
+    quat_z(anglebetween(1, 0, u1x, u1y), sb, cb);
+    quat_z(anglebetween(1, 0, u2x, u2y), se, ce);
+    quat_z(anglebetween(1, 0, vx, vy), sp, cp);
     double d;
-    if (A.usteer > 0) d = (which == 0) ? anglediff_q(sp, cp, A.sb, A.cb) : anglediff_q(A.se, A.ce, sp, cp);
-    else d = (which == 0) ? anglediff_q(A.sb, A.cb, sp, cp) : anglediff_q(sp, cp, A.se, A.ce);
+    if (usteer > 0) d = (which == 0) ? anglediff_q(sp, cp, sb, cb) : anglediff_q(se, ce, sp, cp);
+    else d = (which == 0) ? anglediff_q(sb, cb, sp, cp) : anglediff_q(sp, cp, se, ce);
     return d >= 0;
 }
 
-// does getArc keep circle pixel (px, py)?  search.py:161-181
-__device__ __noinline__ bool arc_keeps_pixel(ArcTest &A, double bx, double by, double lx, double ly, long long px, long long py) {
+// does getArc keep circle pixel (px, py)?  search.py:161-181.  Inlined: the cross products are a few dozen instructions, and
+// as a call its ArcTest was on the stack of every raster (cfg 3: 28.94 ms inlined, 31.37 ms as a call).
+__device__ __forceinline__ bool arc_keeps_pixel(ArcTest &A, double bx, double by, double lx, double ly, long long px, long long py) {
     if (!A.ready) { // lazily: only needed once a blocked circle pixel is met
         A.u1x = bx - A.iccx; A.u1y = by - A.iccy;
         A.u2x = lx - A.iccx; A.u2y = ly - A.iccy;
@@ -411,12 +421,9 @@ __device__ __noinline__ bool arc_keeps_pixel(ArcTest &A, double bx, double by, d
         sf = cross_sign(vx, vy, A.u1x, A.u1y, A.n1 * nv);
         sb = cross_sign(A.u2x, A.u2y, vx, vy, A.n2 * nv);
     }
-    const bool fob = (sf != 0) ? (sf > 0) : arc_literal_ge0(A, vx, vy, 0);
-    const bool bog = (sb != 0) ? (sb > 0) : arc_literal_ge0(A, vx, vy, 1);
-    if (A.diff_lt_180 < 0) {
-        if (!A.literal_ready) arc_literal_prepare(A);
-        A.diff_lt_180 = (A.diff < 180) ? 1 : 0;
-    }
+    const bool fob = (sf != 0) ? (sf > 0) : arc_literal_ge0(A.u1x, A.u1y, A.u2x, A.u2y, A.usteer, vx, vy, 0);
+    const bool bog = (sb != 0) ? (sb > 0) : arc_literal_ge0(A.u1x, A.u1y, A.u2x, A.u2y, A.usteer, vx, vy, 1);
+    if (A.diff_lt_180 < 0) A.diff_lt_180 = arc_literal_diff_lt180(A.u1x, A.u1y, A.u2x, A.u2y, A.usteer);
     if (A.diff_lt_180) return fob && bog;
     return fob || bog;
 }
@@ -435,7 +442,7 @@ __device__ __noinline__ bool arc_blocked_impl(const Group<G> &g, const Grid &m, 
     const T xc = (T)(sizeof(T) == 4 ? (xc_ > lim ? lim : (xc_ < -lim ? -lim : xc_)) : xc_);
     const T yc = (T)(sizeof(T) == 4 ? (yc_ > lim ? lim : (yc_ < -lim ? -lim : yc_)) : yc_);
     ArcTest A;
-    A.iccx = iccx; A.iccy = iccy; A.usteer = usteer; A.ready = false; A.literal_ready = false;
+    A.iccx = iccx; A.iccy = iccy; A.usteer = usteer; A.ready = false;
     bool hit = false;
     const T tmax = (T)circle_tmax(r_);
     const T rr = r * r;

@@ -12,8 +12,14 @@ namespace trrt {
 
 // The single-lane ray / raster functions are real calls; they take the grid BY VALUE (four words in registers): by reference the
 // caller's copy is forced into local memory (cfg 3: 35.2 -> 34.1 ms).
-// search.lineofsight (search.py:35-94) by one lane.  pixels (optional) += max(|dx|,|dy|)+1 for in-bounds rays.
-__device__ __noinline__ bool los_lane(const Grid m, long long ax, long long ay, long long bx, long long by, int *pixels) {
+// search.lineofsight (search.py:35-94) by one lane.  Its pixel count, max(|dx|,|dy|)+1 for in-bounds rays, is los_lane_pixels:
+// through a pointer parameter the caller's counter lived on its stack.
+__device__ __forceinline__ int los_lane_pixels(const Grid &m, long long ax, long long ay, long long bx, long long by) {
+    if (!m.inb(ax, ay) || !m.inb(bx, by)) return 0;
+    const long long dx = bx > ax ? bx - ax : ax - bx, dy = by > ay ? by - ay : ay - by;
+    return (int)(dx > dy ? dx : dy) + 1;
+}
+__device__ __noinline__ bool los_lane(const Grid m, long long ax, long long ay, long long bx, long long by) {
     if (!m.inb(ax, ay) || !m.inb(bx, by)) return false;
     int x0 = (int)ax, y0 = (int)ay, x1 = (int)bx, y1 = (int)by;
     const int adx = abs(x1 - x0), ady = abs(y1 - y0);
@@ -21,7 +27,6 @@ __device__ __noinline__ bool los_lane(const Grid m, long long ax, long long ay, 
     if (low ? (x0 > x1) : (y0 > y1)) { int t = x0; x0 = x1; x1 = t; t = y0; y0 = y1; y1 = t; }
     const int dmaj = low ? adx : ady, dmin = low ? ady : adx;
     const int step = low ? ((y1 < y0) ? -1 : 1) : ((x1 < x0) ? -1 : 1);
-    if (pixels) *pixels += dmaj + 1;
     int D = 2 * dmin - dmaj; // search.py:66 / :85
     int aa = low ? x0 : y0, bb = low ? y0 : x0;
     const int aend = aa + dmaj;
@@ -44,19 +49,27 @@ __device__ __forceinline__ int circle_x32(int c) {
 
 #define TRRT_LANE_RMAX 46000 /* r*r must fit 31 bits */
 
+// Outcome of arc_blocked_lane, returned by value (in registers): through pointer parameters the caller's counters lived on
+// its stack.
+struct ArcLane {
+    bool blocked;
+    int cand_px, angle_tests; // counters: candidate pixels inside the box, blocked pixels given the angular test
+};
+
 // rrt.py:173-174 for a curved edge, one lane: is any pixel of getArc(begin, land, u) not free?
-__device__ __noinline__ bool arc_blocked_lane(const Grid m, double bx, double by, double lx, double ly, double usteer, double iccx,
-                                              double iccy, double rad, int *cand_px, int *angle_tests) {
+__device__ __noinline__ ArcLane arc_blocked_lane(const Grid m, double bx, double by, double lx, double ly, double usteer, double iccx,
+                                                 double iccy, double rad) {
+    ArcLane o = {false, 0, 0};
     const long long xc_ = trunc_ll(iccx), yc_ = trunc_ll(iccy), r_ = trunc_ll(rad);
     if (!(r_ < TRRT_LANE_RMAX)) { // enormous radius (cond() allows up to ~1e6): generic 64-bit raster
         const Group<1> solo;
         unsigned long long a = 0, b = 0;
-        bool hit = arc_blocked_impl<1, long long>(solo, m, bx, by, lx, ly, usteer, iccx, iccy, xc_, yc_, r_, &a, &b);
-        *cand_px += (int)a; *angle_tests += (int)b;
-        return hit;
+        o.blocked = arc_blocked_impl<1, long long>(solo, m, bx, by, lx, ly, usteer, iccx, iccy, xc_, yc_, r_, &a, &b);
+        o.cand_px = (int)a; o.angle_tests = (int)b;
+        return o;
     }
     ArcTest A;
-    A.iccx = iccx; A.iccy = iccy; A.usteer = usteer; A.literal_ready = false;
+    A.iccx = iccx; A.iccy = iccy; A.usteer = usteer;
     A.u1x = bx - iccx; A.u1y = by - iccy;
     A.u2x = lx - iccx; A.u2y = ly - iccy;
     A.n1 = A.u1x * A.u1x + A.u1y * A.u1y;
@@ -96,7 +109,7 @@ __device__ __noinline__ bool arc_blocked_lane(const Grid m, double bx, double by
     // clip to the image: valid() is x < shape[0], y < shape[1] (square maps)
     const double fxlo = fmax(0.0, floor(iccx + xlo)), fxhi = fmin((double)(m.H - 1), ceil(iccx + xhi));
     const double fylo = fmax(0.0, floor(iccy + ylo)), fyhi = fmin((double)(m.W - 1), ceil(iccy + yhi));
-    if (!(fxlo <= fxhi) || !(fylo <= fyhi)) return false; // nothing of the arc can be inside the image
+    if (!(fxlo <= fxhi) || !(fylo <= fyhi)) return o; // nothing of the arc can be inside the image
     const int xc = (int)xc_, yc = (int)yc_, r = (int)r_; // box non-empty => the centre is within rout of the image
     const int oxlo = (int)fxlo - xc, oxhi = (int)fxhi - xc, oylo = (int)fylo - yc, oyhi = (int)fyhi - yc;
     const int tmax = (int)circle_tmax(r_);
@@ -114,7 +127,7 @@ __device__ __noinline__ bool arc_blocked_lane(const Grid m, double bx, double by
         // x_t lies in (t, r]: can +x_t or -x_t fall into [mlo, mhi] at all?
         const bool plus_ok = (mhi > ta) && (mlo <= r), minus_ok = (-mlo > ta) && (-mhi <= r);
         if (!plus_ok && !minus_ok) continue;
-        *cand_px += (tb - ta + 1) * ((plus_ok ? 1 : 0) + (minus_ok ? 1 : 0));
+        o.cand_px += (tb - ta + 1) * ((plus_ok ? 1 : 0) + (minus_ok ? 1 : 0));
         int xt = (ta == 0) ? r : circle_x32(rr - ta * ta); // x_0 = r
         for (int t = ta; t <= tb; t++) {
             const int c = rr - t * t;
@@ -127,8 +140,8 @@ __device__ __noinline__ bool arc_blocked_lane(const Grid m, double bx, double by
                 const int px = (k < 2) ? xc + sx : (k == 2 ? xc + t : xc - t);
                 const int py = (k < 2) ? (k == 0 ? yc + t : yc - t) : yc + sx;
                 if (!m.free_nb(px, py)) { // inside the image by construction of the box
-                    *angle_tests += 1;
-                    if (arc_keeps_pixel(A, bx, by, lx, ly, (long long)px, (long long)py)) return true;
+                    o.angle_tests++;
+                    if (arc_keeps_pixel(A, bx, by, lx, ly, (long long)px, (long long)py)) { o.blocked = true; return o; }
                 }
             }
         }
@@ -153,10 +166,10 @@ __device__ __noinline__ bool arc_blocked_lane(const Grid m, double bx, double by
             }
         }
         if (!drawmore) break;
-        *angle_tests += 1;
-        if (arc_keeps_pixel(A, bx, by, lx, ly, (long long)px, (long long)py)) return true;
+        o.angle_tests++;
+        if (arc_keeps_pixel(A, bx, by, lx, ly, (long long)px, (long long)py)) { o.blocked = true; return o; }
     }
-    return false;
+    return o;
 }
 
 } // namespace trrt

@@ -89,8 +89,9 @@ __device__ __noinline__ void tree_insert(int32_t *tab, int tmask, double x, doub
 // tree_find that also reports where its probe sequence ended: for a miss that is the first empty slot on the key's
 // probe path.  Nothing is ever deleted, so an insert of the same key may resume there instead of hashing again
 // (the commit loop is a serial chain: every instruction and every dependent load taken out of it counts --
-// 69.6 -> 66.2 ms per cfg-3 step).
-__device__ __noinline__ int tree_find_slot(const int32_t *tab, int tmask, const double *nx, const double *ny, const double *nth, double x,
+// 69.6 -> 66.2 ms per cfg-3 step).  Inlined (one call site): as a call, its probe counter and slot were on the caller's stack
+// (cfg 3: 28.94 ms inlined, 29.78 ms as a call; profiles/r6/NOTES.md).
+__device__ __forceinline__ int tree_find_slot(const int32_t *tab, int tmask, const double *nx, const double *ny, const double *nth, double x,
                                               double y, double t, unsigned long long &probes, int &slot) {
     unsigned s = hash3(x, y, t) & (unsigned)tmask;
     for (;;) {
@@ -131,7 +132,7 @@ struct Expand {
 // alone (speculative schedule) and takes the single-lane code of trrt_lane.cuh.
 template <int GA>
 __device__ __forceinline__ bool ray_clear(const Group<GA> &ga, const Grid &m, long long ax, long long ay, long long bx, long long by, int *px) {
-    if (GA == 1) return los_lane(m, ax, ay, bx, by, px);
+    if (GA == 1) { *px += los_lane_pixels(m, ax, ay, bx, by); return los_lane(m, ax, ay, bx, by); }
     unsigned long long p = 0;
     bool ok = los_group<GA>(ga, m, ax, ay, bx, by, &p);
     *px += (int)p;
@@ -142,8 +143,8 @@ __device__ __forceinline__ bool ray_clear(const Group<GA> &ga, const Grid &m, lo
 template <int GA>
 __device__ __forceinline__ void expand_from(const Group<GA> &ga, const Grid &m, const BikeParams &P, double ox, double oy, double oth,
                                            double qx, double qy, double qth, double gx, double gy, double gth, Expand &e_out) {
-    // results are built in locals (only the three pixel counters have their address taken by the callees), so that
-    // after inlining the caller's Expand stays in registers
+    // results are built in locals (only the inlined ray_clear takes the address of a pixel counter; no call receives a
+    // reference or a pointer), so that after inlining the caller's Expand stays in registers
     Expand e;
     int lospx = 0, arcpx = 0, arcang = 0;
     Steer s;
@@ -175,7 +176,8 @@ __device__ __forceinline__ void expand_from(const Group<GA> &ga, const Grid &m, 
     if (!ok) {
         if (s.straight) { e.flags |= 2; e.code = TRRT_IT_NOT_RUN; e.lospx = lospx; e_out = e; return; } // rrt.py:170-171 -> TypeError in the reference
         e.udist = s.dist / 3;
-        drive_bf(P, ox, oy, s.bfx, s.bfy, s.steer, s.iccx, s.iccy, s.rad, e.udist, e.wx, e.wy, e.wth);
+        const Pose d = drive_bf(P, ox, oy, s.bfx, s.bfy, s.steer, s.iccx, s.iccy, s.rad, e.udist);
+        e.wx = d.x; e.wy = d.y; e.wth = d.theta;
         e.drive = 1;
     }
     // goal test input (rrt.py:191-198) depends only on qnew
@@ -188,7 +190,8 @@ __device__ __forceinline__ void expand_from(const Group<GA> &ga, const Grid &m, 
     if (s.straight) {
         blocked = !ray_clear<GA>(ga, m, trunc_ll(ox), trunc_ll(oy), trunc_ll(e.wx), trunc_ll(e.wy), &arcpx);
     } else if (GA == 1) {
-        blocked = arc_blocked_lane(m, ox, oy, e.wx, e.wy, s.steer, s.iccx, s.iccy, s.rad, &arcpx, &arcang);
+        const ArcLane r = arc_blocked_lane(m, ox, oy, e.wx, e.wy, s.steer, s.iccx, s.iccy, s.rad);
+        blocked = r.blocked; arcpx = r.cand_px; arcang = r.angle_tests;
     } else {
         unsigned long long apx = 0, aang = 0;
         blocked = arc_blocked<GA>(ga, m, ox, oy, e.wx, e.wy, s.steer, s.iccx, s.iccy, s.rad, &apx, &aang);
@@ -365,9 +368,11 @@ __device__ __forceinline__ bool nearest_tie_audit(const Group<G> &g, const doubl
     return amb;
 }
 
+// c: the group's counter sums, written to the query's row when a.counters is set; nullptr when the kernel has already summed
+// into that row (rrt_kernel_spec)
 template <int G>
 __device__ __forceinline__ void rrt_finish(const RrtDev &a, int64_t q, const Group<G> &g, const RrtQuery &Q, int K, int iters, int n, int sol,
-                                           int status, int nlos, const RrtCounters &c) {
+                                           int status, int nlos, const RrtCounters *c) {
     if (g.gl == 0) {
         if (Q.it_near || Q.it_new || Q.it_code) {
 #pragma unroll 1
@@ -382,10 +387,10 @@ __device__ __forceinline__ void rrt_finish(const RrtDev &a, int64_t q, const Gro
         a.status[q] = status;
         a.iters[q] = iters;
         if (a.n_los) a.n_los[q] = nlos;
-        if (a.counters) {
+        if (a.counters && c) {
             unsigned long long *o = a.counters + q * 9;
-            o[0] = c.scan; o[1] = c.los; o[2] = c.lospx; o[3] = c.arcpx; o[4] = c.arcang; o[5] = c.steer; o[6] = c.drive; o[7] = c.probe;
-            o[8] = c.ties;
+            o[0] = c->scan; o[1] = c->los; o[2] = c->lospx; o[3] = c->arcpx; o[4] = c->arcang; o[5] = c->steer; o[6] = c->drive;
+            o[7] = c->probe; o[8] = c->ties;
         }
     }
     if (a.row_start) { // packed copy of the rows that exist: one row reservation per query, coalesced copies by the group
@@ -468,7 +473,7 @@ __global__ void __launch_bounds__(128) rrt_kernel_coop(const RrtDev a) {
             break;
         }
     }
-    rrt_finish<G>(a, q, g, Q, K, k - 1, n, sol, status, nlos, c);
+    rrt_finish<G>(a, q, g, Q, K, k - 1, n, sol, status, nlos, &c);
 }
 
 // ---------------------------------------------------------------------------
@@ -730,6 +735,15 @@ __device__ __forceinline__ void nearest_staged(double2 *tile /* [2][2][TILE_PAIR
     bd_out = bd; bi_out = bi;
 }
 
+// Counters launches of rrt_kernel_spec: every lane adds its share straight to the query's row, so no counter is carried
+// through the window loop.  Nine per-lane sums would hold 18 registers across the expansion, and a per-warp copy (14 x 72 B)
+// does not fit the kernel's 48 KB of static shared memory: with sQ the kernel uses 48 968 of 49 152 bytes.  The group zeroes
+// the row when it takes the query: the C ABI has always had the kernel write the whole row, so callers other than
+// Planner.rrt need not clear d_counters.
+__device__ __forceinline__ void count_add(const RrtDev &a, int64_t q, int k, unsigned long long v) {
+    if (v) atomicAdd(a.counters + q * 9 + k, v);
+}
+
 // CTA shape of rrt_kernel_spec, also read by its launch: 2 CTAs of 14 warps = 28 warps per SM at 72 registers, so the
 // 4 096 queries of cfg 3 are resident at once (4 144 warps), no second wave.  Measured on B200 (cfg 3): 448 x 2 39.4 ms,
 // 384 x 2 43.9 ms, 512 x 2 (64 registers) 42.4 ms, 768 x 1 43.0 ms; see profiles/r2/NOTES.md.
@@ -752,7 +766,6 @@ __global__ void __launch_bounds__(SPEC_THREADS, SPEC_BLOCKS_PER_SM) rrt_kernel_s
     constexpr int NW = SPEC_THREADS / 32;
     static_assert(NW <= 32, "one lane per warp of the CTA in the scan partition");
     __shared__ double2 pool_q[(G == 32) ? NW : 1][32];            // sample of lane l of warp w
-    __shared__ const double *pool_x[(G == 32) ? NW : 1], *pool_y[(G == 32) ? NW : 1];
     __shared__ int pool_n[(G == 32) ? NW : 1];                    // nodes to scan (0: warp w has nothing to scan)
     __shared__ double pool_d[(G == 32) ? 2 * NW : 1][32];         // partial minima: one slot per (warp, tree) overlap
     __shared__ int pool_i[(G == 32) ? 2 * NW : 1][32];
@@ -761,14 +774,22 @@ __global__ void __launch_bounds__(SPEC_THREADS, SPEC_BLOCKS_PER_SM) rrt_kernel_s
     // space would be copied to every thread's local stack (192 bytes); one copy per CTA in shared memory serves all of them
     // (1712 -> 1312 bytes of stack).
     __shared__ BikeParams sP;
+    // The query's map, row pointers and goal are the same in every lane of a group.  As per-lane copies they held ~35
+    // registers for the whole window and pushed the expansion's live set onto the stack; one copy per warp in shared memory
+    // is read where it is needed (the pooled scan reads the other warps' tree pointers from it too).  G < 32 puts several
+    // groups in a warp; those instantiations keep a copy per lane.
+    // Invariant: warp v writes sQ[v] only in rrt_setup, at the top of a loop trip, i.e. after the previous window's
+    // __syncthreads_or; other warps read sQ[v].nx / .ny only in the pooled scan, between the window's two CTA barriers,
+    // and only when pool_n[v] > 0.  A write to sQ inside a window would race with those reads.
+    __shared__ RrtQuery sQ[(G == 32) ? NW : 1];
+    RrtQuery Qlane;
+    RrtQuery &Q = (G == 32) ? sQ[threadIdx.x >> 5] : Qlane;
     for (int i = threadIdx.x; i < (int)(sizeof(BikeParams) / 4); i += blockDim.x) reinterpret_cast<int *>(&sP)[i] = reinterpret_cast<const int *>(&a.P)[i];
     __syncthreads();
     // persistent groups: queries differ a lot in length (27% of the cfg-3 queries end early), so each group
     // pulls the next query from a counter instead of owning a fixed one.  One loop trip = one window.
     bool have = false, drained = false;
     int64_t q = 0;
-    RrtQuery Q;
-    RrtCounters c = {0, 0, 0, 0, 0, 0, 0, 0, 0}; // lane-private sums, folded at the end
     int n = 1, nlos = 0, sol = -1, status = TRRT_OK_NOT_FOUND, iters = 0, k0 = 0;
     TRRT_PROF(unsigned long long pf[24]; for (int i_ = 0; i_ < 24; i_++) pf[i_] = 0; long long t0_, t1_ = 0, t2_, t3_, t4_ = 0, t5_ = 0;)
     for (;;) {
@@ -779,8 +800,8 @@ __global__ void __launch_bounds__(SPEC_THREADS, SPEC_BLOCKS_PER_SM) rrt_kernel_s
             if (qq >= (unsigned long long)a.nq) drained = true;
             else {
                 q = (int64_t)qq;
+                if (a.counters && g.gl == 0) for (int j = 0; j < 9; j++) a.counters[q * 9 + j] = 0; // summed into by count_add
                 rrt_setup<G>(a, q, g, Q);
-                c = RrtCounters{0, 0, 0, 0, 0, 0, 0, 0, 0};
                 n = 1; nlos = 0; sol = -1; status = TRRT_OK_NOT_FOUND; iters = 0; k0 = 0;
                 have = true;
             }
@@ -819,7 +840,7 @@ __global__ void __launch_bounds__(SPEC_THREADS, SPEC_BLOCKS_PER_SM) rrt_kernel_s
             const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
             const bool scan_me = have && g.any(live);
             pool_q[wid][lane] = make_double2(qx, qy);
-            if (lane == 0) { pool_n[wid] = scan_me ? n : 0; pool_x[wid] = Q.nx; pool_y[wid] = Q.ny; }
+            if (lane == 0) pool_n[wid] = scan_me ? n : 0;
             TRRT_PROF(t1_ = clock64();)
             __syncthreads();
             TRRT_PROF(t4_ = clock64();)
@@ -857,7 +878,7 @@ __global__ void __launch_bounds__(SPEC_THREADS, SPEC_BLOCKS_PER_SM) rrt_kernel_s
                     double pd = INFINITY;
                     int pi = 0x7fffffff;
                     ScanStats st = {0, 0, 0, 0, 0, 0}; // counted in the phase-profile build only
-                    if (lo < hi) nearest_staged(scan_tile, pool_x[v], pool_y[v], lo, hi, sq.x, sq.y,
+                    if (lo < hi) nearest_staged(scan_tile, sQ[v].nx, sQ[v].ny, lo, hi, sq.x, sq.y,
                                                 (double)(a.W / 2), (double)(a.H / 2), pd, pi, st); // origin: the map centre
                     TRRT_PROF(if (lo < hi) { pf[11] += st.rechecked; pf[12] += st.settled; pf[13] += st.fp64; pf[14]++; pf[15] += st.blocks; pf[5] += st.cyc_wait; pf[6] += st.cyc_settle; })
                     const int slot = b0 + (wid - k0v);
@@ -885,7 +906,7 @@ __global__ void __launch_bounds__(SPEC_THREADS, SPEC_BLOCKS_PER_SM) rrt_kernel_s
             expand_from<1>(solo, Q.m, sP, Q.nx[near], Q.ny[near], Q.nth[near], qx, qy, qth, Q.gx, Q.gy, Q.gth, e);
             if (e.code == EX_ACCEPT) exist = tree_find_slot(Q.tab, Q.tmask, Q.nx, Q.ny, Q.nth, e.wx, e.wy, e.wth, probes, islot);
         }
-        c.probe += probes;
+        if (a.counters) count_add(a, q, 7, probes);
         g.sync();
         TRRT_PROF(t3_ = clock64(); { const unsigned long long s_ = t3_ - t2_; pf[3] += s_; pf[4] += s_ * s_ >> 10; })
         // ---------------- pass: fold the new nodes forward, find the first lane that has to start over
@@ -943,8 +964,8 @@ __global__ void __launch_bounds__(SPEC_THREADS, SPEC_BLOCKS_PER_SM) rrt_kernel_s
                     near_j = near;
                     const int before = __popc(done & lane_lt); // nodes inserted by the earlier lanes of the window
                     if (a.counters) {
-                        c.scan += (unsigned long long)(n + before); c.steer++;
-                        if (nearest_tie_audit<1>(solo, Q.nx, Q.ny, near, bd, qx, qy, false)) c.ties++; // window nodes have higher indices
+                        count_add(a, q, 0, (unsigned long long)(n + before)); count_add(a, q, 5, 1);
+                        if (nearest_tie_audit<1>(solo, Q.nx, Q.ny, near, bd, qx, qy, false)) count_add(a, q, 8, 1); // window nodes have higher indices
                     }
                     if (e.code == TRRT_IT_STEER_CONSTRAINT) code = TRRT_IT_STEER_CONSTRAINT; // rrt.py:166
                     else {
@@ -954,7 +975,10 @@ __global__ void __launch_bounds__(SPEC_THREADS, SPEC_BLOCKS_PER_SM) rrt_kernel_s
                             if (nl >= 1) Q.los_log[pos] = (e.flags >> 6) & 1;
                             if (nl >= 2) Q.los_log[pos + 1] = (e.flags >> 7) & 1;
                         }
-                        if (a.counters) { c.los += nl; c.lospx += e.lospx; c.arcpx += e.arcpx; c.arcang += e.arcang; c.drive += e.drive; }
+                        if (a.counters) {
+                            count_add(a, q, 1, nl); count_add(a, q, 2, e.lospx); count_add(a, q, 3, e.arcpx); count_add(a, q, 4, e.arcang);
+                            count_add(a, q, 6, e.drive);
+                        }
                         if (e.flags & 2) code = TRRT_IT_NOT_RUN;                              // rrt.py:170-171 raises
                         else if (e.code == TRRT_IT_ARC_BLOCKED) code = TRRT_IT_ARC_BLOCKED;   // rrt.py:174
                         else if (exist >= 0) { code = TRRT_IT_EXISTING_NODE; newi = exist; edge = newi != near; } // rrt.py:179 false
@@ -1002,11 +1026,7 @@ __global__ void __launch_bounds__(SPEC_THREADS, SPEC_BLOCKS_PER_SM) rrt_kernel_s
         TRRT_PROF({ const unsigned long long s_ = clock64() - t3_; pf[7] += s_; pf[8] += s_ * s_ >> 10; const unsigned long long w_ = clock64() - t2_; pf[9] += w_ * w_ >> 10; })
         k0 += end;
         if (finished || k0 >= K - 1) { // query finished
-            if (a.counters) { // fold the lane-private counters
-                c.scan = g.sum(c.scan); c.los = g.sum(c.los); c.lospx = g.sum(c.lospx); c.arcpx = g.sum(c.arcpx); c.arcang = g.sum(c.arcang);
-                c.steer = g.sum(c.steer); c.drive = g.sum(c.drive); c.probe = g.sum(c.probe); c.ties = g.sum(c.ties);
-            }
-            rrt_finish<G>(a, q, g, Q, K, iters, n, sol, status, nlos, c);
+            rrt_finish<G>(a, q, g, Q, K, iters, n, sol, status, nlos, nullptr);
             g.sync();
             have = false;
         }
