@@ -66,7 +66,9 @@ typedef enum trrt_status {
     TRRT_ERR_REF_RAISES_DRIVE_NONE = 4,   /* [TypeError: drive() after straight steer, rrt.py:170-171,275] */
     TRRT_ERR_REF_RAISES_ARGMIN_EMPTY = 5, /* [ValueError: np.argmin([]), search.py:262]        */
     TRRT_ERR_CAPACITY = 6,                /* heap / path / node capacity of the call exceeded  */
-    TRRT_ERR_REF_RAISES_NO_NEAREST = 7    /* [TypeError: findnearest of a childless tree, main.py:79-81] */
+    TRRT_ERR_REF_RAISES_NO_NEAREST = 7,   /* [TypeError: findnearest of a childless tree, main.py:79-81] */
+    TRRT_PAUSED = 8                       /* trrt_rrt_batch: stopped at its d_stop_at iteration with iterations left;
+                                             a call with resume = 1 continues it */
 } trrt_status;
 
 /* outcome of one RRT loop iteration (rrt.py:141-201) */
@@ -185,7 +187,8 @@ typedef struct trrt_rrt_args {
     uint64_t *d_counters; /* [n_queries][9]: nodes scanned, los calls, los pixels, arc candidate pixels, arc angle tests, steer calls,
                              drive calls, hash probes, nearest decisions where a lower-indexed node has a larger squared distance with the
                              SAME rounded sqrt (the only way argmin(d2) can differ from the reference's argmin(sqrt); expected 0);
-                             may be NULL */
+                             may be NULL.  A resumed query adds to its row; counter 7 then counts the probes of the rebuilt
+                             index (see d_stop_at / resume), so it is the one counter that depends on where a run paused */
     /* scratch */
     void *d_work;
     size_t work_bytes; /* >= trrt_rrt_workspace_bytes(n_queries, K) */
@@ -204,6 +207,21 @@ typedef struct trrt_rrt_args {
     double *d_pack_th;
     int32_t *d_pack_parent;
     double *d_pack_u;       /* [rows][5]; NULL unless d_u is given too */
+    /* Pause and resume.  d_stop_at[q] (clamped to [0, K-1]; NULL = K-1 for every query): query q runs no loop iteration
+       whose 0-based index it = k-1 is >= d_stop_at[q].  A query that reaches its stop with iterations left and has not
+       ended gets status TRRT_PAUSED and iters = d_stop_at[q]; it then holds exactly what rrt.rrt plans with
+       K = d_stop_at[q] + 1 over the first d_stop_at[q] samples.  A query that ends earlier (found, raises, capacity) keeps
+       its usual status; d_stop_at[q] = K-1 is the behaviour of a call without stops.
+       resume = 1: the call continues every query whose d_status is TRRT_PAUSED from the tree, logs, LOS-log position and
+       counters in the output arrays, at iteration d_iters[q], up to d_stop_at[q] (or K-1).  The query's `in G` index is
+       rebuilt from its n_nodes nodes (it lives in d_work and does not survive a call).  A query that is not paused, or
+       whose stop is <= d_iters[q], is not written at all.  K, starts, goals, samples, map ids and params must be those of
+       the pausing call, and the optional outputs (logs, d_u, d_counters) the same set of arrays.  Any sequence of pauses
+       and resumes, under any lanes and schedule, gives the outputs of one uninterrupted call bit for bit, except counter
+       7 (hash probes).  Not combined with the packed copy: d_row_start with d_stop_at or resume is
+       TRRT_ERR_INVALID_ARGUMENT. */
+    const int32_t *d_stop_at; /* [n_queries] or NULL */
+    int32_t resume;           /* 0 / 1 */
 } trrt_rrt_args;
 
 size_t trrt_rrt_workspace_bytes(int64_t n_queries, int32_t K);

@@ -46,6 +46,7 @@ class CRrtArgs(C.Structure):
         ("d_work", C.c_void_p), ("work_bytes", C.c_size_t),
         ("d_pack_rows", C.c_void_p), ("d_row_start", C.c_void_p), ("d_pack_x", C.c_void_p), ("d_pack_y", C.c_void_p),
         ("d_pack_th", C.c_void_p), ("d_pack_parent", C.c_void_p), ("d_pack_u", C.c_void_p),
+        ("d_stop_at", C.c_void_p), ("resume", C.c_int32),
     ]
 
 

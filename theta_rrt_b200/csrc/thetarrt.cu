@@ -1002,6 +1002,8 @@ int trrt_rrt_batch(const trrt_rrt_args *args, void *stream) {
     if (A.d_los_log && !A.d_n_los) return TRRT_ERR_INVALID_ARGUMENT;
     if (A.d_row_start && (!A.d_pack_rows || !A.d_pack_x || !A.d_pack_y || !A.d_pack_th || !A.d_pack_parent || (A.d_pack_u && !A.d_u)))
         return TRRT_ERR_INVALID_ARGUMENT;
+    if (A.resume != 0 && A.resume != 1) return TRRT_ERR_INVALID_ARGUMENT;
+    if (A.d_row_start && (A.d_stop_at || A.resume)) return TRRT_ERR_INVALID_ARGUMENT; // packing is for whole runs
     if (A.work_bytes < trrt_rrt_workspace_bytes(A.n_queries, A.K)) return TRRT_ERR_WORKSPACE_TOO_SMALL;
     if ((uintptr_t)A.d_work & 7) return TRRT_ERR_INVALID_ARGUMENT;
     if ((uintptr_t)A.d_sample_xy & (A.sample_xy_i16 ? 3 : 7)) return TRRT_ERR_INVALID_ARGUMENT; // read as short2 / int2
@@ -1017,6 +1019,7 @@ int trrt_rrt_batch(const trrt_rrt_args *args, void *stream) {
     d.pack_rows = (unsigned long long *)A.d_pack_rows; d.row_start = (long long *)A.d_row_start;
     d.px = A.d_pack_x; d.py = A.d_pack_y; d.pth = A.d_pack_th; d.pparent = A.d_pack_parent; d.pu = A.d_pack_u;
     d.tab = (int32_t *)((char *)A.d_work + 256); d.tsize = rrt_tsize(A.K);
+    d.stop_at = A.d_stop_at; d.resume = A.resume;
     cudaStream_t st = (cudaStream_t)stream;
     int threads = 128;
     int64_t blocks = (A.n_queries * G + threads - 1) / threads;

@@ -51,6 +51,9 @@ struct RrtDev {
     long long *row_start;
     double *px, *py, *pth, *pu;
     int32_t *pparent;
+    // pause and resume (see trrt_rrt_args in thetarrt.h): per-query stop iteration or nullptr (K-1); resume paused queries
+    const int32_t *stop_at;
+    int resume;
 };
 
 __device__ __forceinline__ unsigned hash3(double x, double y, double t) {
@@ -238,8 +241,23 @@ struct RrtQuery {
     uint8_t *it_code, *los_log;
     int32_t *tab;
     int tmask;
+    int limit; // iterations it < limit run (d_stop_at clamped to [0, K-1]); fits the padding after tmask
     double gx, gy, gth;
 };
+// one copy per warp of rrt_kernel_spec<32> sits in its static shared memory, which has 184 bytes to spare
+static_assert(sizeof(RrtQuery) == 152, "RrtQuery grew: rrt_kernel_spec's shared memory budget");
+
+// the query's stop: iterations it < limit run
+__device__ __forceinline__ int query_limit(const RrtDev &a, int64_t q) {
+    if (!a.stop_at) return a.K - 1;
+    const int s = a.stop_at[q];
+    return s < 0 ? 0 : (s > a.K - 1 ? a.K - 1 : s);
+}
+
+// a resume call continues query q: it is paused and its stop lies beyond the iterations it has run
+__device__ __forceinline__ bool query_resumes(const RrtDev &a, int64_t q) {
+    return a.status[q] == TRRT_PAUSED && a.iters[q] < query_limit(a, q);
+}
 
 // pointers of query q (no memory is touched)
 __device__ __forceinline__ void rrt_ptrs(const RrtDev &a, int64_t q, RrtQuery &Q) {
@@ -257,6 +275,7 @@ __device__ __forceinline__ void rrt_ptrs(const RrtDev &a, int64_t q, RrtQuery &Q
     Q.los_log = a.los_log ? a.los_log + q * (int64_t)(K - 1) * 2 : nullptr;
     Q.tab = a.tab + q * (int64_t)a.tsize;
     Q.tmask = a.tsize - 1;
+    Q.limit = query_limit(a, q);
     Q.gx = a.goal[3 * q]; Q.gy = a.goal[3 * q + 1]; Q.gth = standardangle(a.goal[3 * q + 2]);
 }
 
@@ -284,6 +303,27 @@ __device__ __forceinline__ void rrt_setup(const RrtDev &a, int64_t q, const Grou
     }
     g.sync();
     if (g.gl == 0) tree_insert(Q.tab, Q.tmask, Q.nx[0], Q.ny[0], Q.nth[0], 0);
+    g.sync();
+}
+
+// A paused query (resume calls): pointers, the loop state left in the output arrays, and its index rebuilt over nodes
+// [0, n) by the group.  The nodes are distinct keys, so every insertion order gives a table with the same lookups (only
+// the probe counts differ).  Node 0 and the counter row are not touched.
+template <int G>
+__device__ __forceinline__ void rrt_setup_resume(const RrtDev &a, int64_t q, const Group<G> &g, RrtQuery &Q, int &n, int &iters,
+                                                 int &nlos) {
+    rrt_ptrs(a, q, Q);
+    n = a.n_nodes[q];
+    iters = a.iters[q];
+    nlos = a.n_los ? a.n_los[q] : 0;
+    TRRT_CHECK(n >= 1 && n <= a.K && iters >= 0 && iters < Q.limit);
+#pragma unroll 4
+    for (int i = g.gl; i < a.tsize; i += G) Q.tab[i] = 0;
+    g.sync();
+    for (int i = g.gl; i < n; i += G) {
+        const double x = Q.nx[i], y = Q.ny[i], t = Q.nth[i];
+        tree_insert_cas(Q.tab, Q.tmask, (int)(hash3(x, y, t) & (unsigned)Q.tmask), i);
+    }
     g.sync();
 }
 
@@ -373,6 +413,7 @@ __device__ __forceinline__ bool nearest_tie_audit(const Group<G> &g, const doubl
 template <int G>
 __device__ __forceinline__ void rrt_finish(const RrtDev &a, int64_t q, const Group<G> &g, const RrtQuery &Q, int K, int iters, int n, int sol,
                                            int status, int nlos, const RrtCounters *c) {
+    if (status == TRRT_OK_NOT_FOUND && iters < K - 1) status = TRRT_PAUSED; // the query's stop cut the loop
     if (g.gl == 0) {
         if (Q.it_near || Q.it_new || Q.it_code) {
 #pragma unroll 1
@@ -389,8 +430,8 @@ __device__ __forceinline__ void rrt_finish(const RrtDev &a, int64_t q, const Gro
         if (a.n_los) a.n_los[q] = nlos;
         if (a.counters && c) {
             unsigned long long *o = a.counters + q * 9;
-            o[0] = c->scan; o[1] = c->los; o[2] = c->lospx; o[3] = c->arcpx; o[4] = c->arcang; o[5] = c->steer; o[6] = c->drive;
-            o[7] = c->probe; o[8] = c->ties;
+            const unsigned long long v[9] = {c->scan, c->los, c->lospx, c->arcpx, c->arcang, c->steer, c->drive, c->probe, c->ties};
+            for (int j = 0; j < 9; j++) o[j] = (a.resume ? o[j] : 0ull) + v[j]; // a resumed query adds to its row
         }
     }
     if (a.row_start) { // packed copy of the rows that exist: one row reservation per query, coalesced copies by the group
@@ -435,13 +476,15 @@ __global__ void __launch_bounds__(128) rrt_kernel_coop(const RrtDev a) {
     const Group<G> g;
     const int64_t q = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) / G;
     if (q >= a.nq) return; // whole groups leave together
+    if (a.resume && !query_resumes(a, q)) return; // not written at all
     const int K = a.K;
     RrtQuery Q;
-    rrt_setup<G>(a, q, g, Q);
     RrtCounters c = {0, 0, 0, 0, 0, 0, 0, 0, 0};
-    int n = 1, nlos = 0, sol = -1, status = TRRT_OK_NOT_FOUND;
+    int n = 1, nlos = 0, sol = -1, status = TRRT_OK_NOT_FOUND, it0 = 0;
+    if (a.resume) rrt_setup_resume<G>(a, q, g, Q, n, it0, nlos);
+    else rrt_setup<G>(a, q, g, Q);
     int k;
-    for (k = 1; k < K; k++) {
+    for (k = it0 + 1; k <= Q.limit; k++) {
         const int it = k - 1;
         int sx, sy;
         sample_xy(a, Q, it, sx, sy);
@@ -793,16 +836,23 @@ __global__ void __launch_bounds__(SPEC_THREADS, SPEC_BLOCKS_PER_SM) rrt_kernel_s
     int n = 1, nlos = 0, sol = -1, status = TRRT_OK_NOT_FOUND, iters = 0, k0 = 0;
     TRRT_PROF(unsigned long long pf[24]; for (int i_ = 0; i_ < 24; i_++) pf[i_] = 0; long long t0_, t1_ = 0, t2_, t3_, t4_ = 0, t5_ = 0;)
     for (;;) {
-        if (!have && !drained) {
+        while (!have && !drained) { // a resume call skips the queries it does not continue
             unsigned long long qq = 0;
             if (g.gl == 0) qq = atomicAdd(a.next_query, 1ull);
             qq = g.bcast(qq, 0);
             if (qq >= (unsigned long long)a.nq) drained = true;
             else {
                 q = (int64_t)qq;
-                if (a.counters && g.gl == 0) for (int j = 0; j < 9; j++) a.counters[q * 9 + j] = 0; // summed into by count_add
-                rrt_setup<G>(a, q, g, Q);
-                n = 1; nlos = 0; sol = -1; status = TRRT_OK_NOT_FOUND; iters = 0; k0 = 0;
+                sol = -1; status = TRRT_OK_NOT_FOUND;
+                if (a.resume) {
+                    if (!query_resumes(a, q)) continue;
+                    rrt_setup_resume<G>(a, q, g, Q, n, iters, nlos);
+                    k0 = iters;
+                } else {
+                    if (a.counters && g.gl == 0) for (int j = 0; j < 9; j++) a.counters[q * 9 + j] = 0; // summed into by count_add
+                    rrt_setup<G>(a, q, g, Q);
+                    n = 1; nlos = 0; iters = 0; k0 = 0;
+                }
                 have = true;
             }
         }
@@ -819,7 +869,7 @@ __global__ void __launch_bounds__(SPEC_THREADS, SPEC_BLOCKS_PER_SM) rrt_kernel_s
         e.wx = e.wy = e.wth = NAN; // never equal to a node
         if (have) {
             const int my_it = k0 + g.gl;
-            if (my_it < K - 1) {
+            if (my_it < Q.limit) { // beyond the query's stop: TRRT_IT_NOT_RUN cuts the window there
                 int sx, sy;
                 sample_xy(a, Q, my_it, sx, sy);
                 qx = (double)sx; qy = (double)sy;
@@ -1025,7 +1075,7 @@ __global__ void __launch_bounds__(SPEC_THREADS, SPEC_BLOCKS_PER_SM) rrt_kernel_s
         g.sync(); // tree and index writes of this window are visible to every lane's next phase A
         TRRT_PROF({ const unsigned long long s_ = clock64() - t3_; pf[7] += s_; pf[8] += s_ * s_ >> 10; const unsigned long long w_ = clock64() - t2_; pf[9] += w_ * w_ >> 10; })
         k0 += end;
-        if (finished || k0 >= K - 1) { // query finished
+        if (finished || k0 >= Q.limit) { // query finished or paused
             rrt_finish<G>(a, q, g, Q, K, iters, n, sol, status, nlos, nullptr);
             g.sync();
             have = false;

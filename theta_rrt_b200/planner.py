@@ -21,10 +21,13 @@ from .params import Params
 
 STATUS_NAMES = {0: "OK_FOUND", 1: "OK_NOT_FOUND", 2: "ERR_ENDPOINT_INVALID", 3: "ERR_ENDPOINT_BLOCKED",
                 4: "ERR_REF_RAISES_DRIVE_NONE", 5: "ERR_REF_RAISES_ARGMIN_EMPTY", 6: "ERR_CAPACITY",
-                7: "ERR_REF_RAISES_NO_NEAREST"}
+                7: "ERR_REF_RAISES_NO_NEAREST", 8: "PAUSED"}
+PAUSED = 8  # Planner.rrt(..., stop_at=...): stopped with iterations left; Planner.rrt_resume continues it
 SEG_NOT_RUN = 255
 IT_NEW_NODE, IT_EXISTING_NODE, IT_QRAND_BLOCKED, IT_QRAND_IN_TREE, IT_STEER_CONSTRAINT, IT_ARC_BLOCKED = range(6)
 IT_NOT_RUN = 255
+# RrtResult.counters columns.  A resumed query (rrt_resume) adds to its row; hash_probes then counts probes in the index the
+# resume rebuilt, so it is the one column that depends on where a run paused.
 COUNTER_NAMES = ("nodes_scanned", "los_calls", "los_pixels", "arc_candidate_pixels", "arc_angle_tests",
                  "steer_calls", "drive_calls", "hash_probes", "nearest_sqrt_ties")
 
@@ -244,13 +247,18 @@ class Planner:
 
     # ------------------------------------------------------------------ K2
     def rrt(self, starts, goals, sample_xy, sample_th, K=None, params=None, map_id=None, logs=False, want_u=True,
-            counters=False, lanes=0, schedule=0, work_key="rrt", reuse=None, pack=False, packed=None):
+            counters=False, lanes=0, schedule=0, work_key="rrt", reuse=None, pack=False, packed=None, stop_at=None):
         """rrt.rrt for a batch.  starts/goals float64 [q,3] (x, y, theta_deg); sample_xy int32 [q,K-1,2];
         sample_th float64 [q,K-1].  K = builtins.K (node capacity; K-1 iterations).
         pack=True: the kernel also leaves a packed copy of the tree rows that exist (pack_x, pack_y, pack_theta,
         pack_parent, pack_u; query q owns rows row_start[q] ... + n_nodes[q] - 1, pack_total rows in all); `packed` may
-        pass a dict of such arrays to use; its pack_total must then hold the first row to use (0 for arrays of this call's own)."""
+        pass a dict of such arrays to use; its pack_total must then hold the first row to use (0 for arrays of this call's own).
+        stop_at: an int or [q] ints in [0, K-1] (a CUDA int32 tensor is clamped to that range on the device): query q runs
+        no iteration it >= stop_at[q].  A query stopped with iterations left has status PAUSED and iters = stop_at[q], and
+        holds exactly what rrt.rrt plans with K = stop_at[q] + 1; rrt_resume continues it."""
         P = params or self.params
+        if pack and stop_at is not None:
+            raise ValueError("pack=True plans whole runs: it cannot be combined with stop_at")
         with torch.cuda.device(self.device):
             starts = self._dev(starts, torch.float64).reshape(-1, 3)
             goals = self._dev(goals, torch.float64).reshape(-1, 3)
@@ -266,6 +274,7 @@ class Planner:
             xy16 = isinstance(sample_xy, torch.Tensor) and sample_xy.dtype == torch.int16
             sample_xy = self._dev(sample_xy, torch.int16 if xy16 else torch.int32).reshape(nq, K - 1, 2)
             mid = self._map_ids(map_id, nq)
+            stop = self._stop_at(stop_at, nq, K)
             dev = self.device
             f64 = dict(dtype=torch.float64, device=dev)
             i32 = dict(dtype=torch.int32, device=dev)
@@ -300,31 +309,76 @@ class Planner:
                     packed["pack_total"].zero_()
                 for k, v in packed.items():  # a reused set: the caller has set pack_total to the first row to use
                     setattr(res, k, v)
-            wb = self.lib.trrt_rrt_workspace_bytes(nq, K)
-            work = self._scratch(work_key, wb)  # concurrent launches (rrt_host) must not share a workspace
-            g = self.grid
-            ptr = lambda t: t.data_ptr() if t is not None else None  # noqa: E731
-            a = _lib.CRrtArgs(d_bits=g.bits.data_ptr(), n_maps=g.n_maps, H=g.H, W=g.W, d_map_id=ptr(mid),
-                              params=P.to_c(), n_queries=nq, K=K, lanes_per_query=int(lanes), schedule=int(schedule),
-                              sample_xy_i16=int(xy16),
-                              d_start=starts.data_ptr(), d_goal=goals.data_ptr(), d_sample_xy=sample_xy.data_ptr(),
-                              d_sample_th=sample_th.data_ptr(), d_node_x=res.node_x.data_ptr(),
-                              d_node_y=res.node_y.data_ptr(), d_node_th=res.node_theta.data_ptr(),
-                              d_parent=res.parent.data_ptr(), d_u=ptr(res.u), d_n_nodes=res.n_nodes.data_ptr(),
-                              d_sol=res.sol.data_ptr(), d_status=res.status.data_ptr(), d_iters=res.iters.data_ptr(),
-                              d_it_near=ptr(res.it_near), d_it_new=ptr(res.it_new), d_it_code=ptr(res.it_code),
-                              d_los_log=ptr(res.los_log), d_n_los=ptr(res.n_los), d_counters=ptr(res.counters),
-                              d_work=work.data_ptr(), work_bytes=work.numel(),
-                              d_pack_rows=ptr(res.pack_total) if pack else None, d_row_start=ptr(res.row_start) if pack else None,
-                              d_pack_x=ptr(res.pack_x) if pack else None, d_pack_y=ptr(res.pack_y) if pack else None,
-                              d_pack_th=ptr(res.pack_theta) if pack else None,
-                              d_pack_parent=ptr(res.pack_parent) if pack else None,
-                              d_pack_u=ptr(res.pack_u) if (pack and want_u) else None)
-            _lib.check(self.lib.trrt_rrt_batch(C.byref(a), self._stream()), "trrt_rrt_batch")
-            res.lanes = int(lanes)
-            # keep inputs alive until the stream has consumed them
-            res._keep = (starts, goals, sample_xy, sample_th, mid)
+            # the inputs stay alive until the stream has consumed them, and rrt_resume plans with them again
+            res._keep = (starts, goals, sample_xy, sample_th, mid, P, self.grid)
+            res._packed = bool(pack)
+            self._rrt_launch(res, stop, lanes, schedule, resume=False, work_key=work_key)
         return res
+
+    def rrt_resume(self, res: RrtResult, stop_at=None, lanes=0, schedule=0) -> RrtResult:
+        """Continue the PAUSED queries of `res` (a result of rrt(..., stop_at=...)) in place, with the inputs, params and
+        map ids it was planned with: each runs from iteration iters[q] up to stop_at[q] (default K-1), and may pause
+        again.  Other queries, and paused ones whose stop is <= iters[q], are not written.  lanes and schedule may differ
+        from the pausing call.  Any sequence of pauses and resumes returns what one uninterrupted call returns, bit for
+        bit, except counter 7 (hash probes, which count probes in the query's rebuilt index).  Returns res."""
+        keep = getattr(res, "_keep", None)
+        if keep is None or len(keep) != 7 or keep[6] is not self.grid:
+            raise ValueError("rrt_resume continues a result that Planner.rrt planned on this planner's grid")
+        if res._packed:
+            raise ValueError("a result planned with pack=True cannot be resumed")
+        with torch.cuda.device(self.device):
+            stop = self._stop_at(stop_at, res.node_x.shape[0], res.K)
+            self._rrt_launch(res, stop, lanes, schedule, resume=True)
+        return res
+
+    def _stop_at(self, stop_at, nq, K):
+        """stop_at of rrt / rrt_resume -> int32 [nq] device tensor, or None.  Host values outside [0, K-1] raise."""
+        if stop_at is None:
+            return None
+        if isinstance(stop_at, torch.Tensor) and stop_at.is_cuda:
+            t = self._dev(stop_at, torch.int32).reshape(-1)  # left on the device: the kernel clamps it to [0, K-1]
+        else:
+            a = np.asarray(stop_at.cpu() if isinstance(stop_at, torch.Tensor) else stop_at)
+            if a.dtype.kind not in "iu":
+                raise ValueError(f"stop_at must be integers, got {a.dtype}")
+            if a.ndim == 0:
+                a = np.full(nq, int(a), np.int64)
+            a = a.reshape(-1)
+            if a.size and (int(a.min()) < 0 or int(a.max()) > K - 1):
+                raise ValueError(f"stop_at must lie in [0, K-1 = {K - 1}]")
+            t = self._dev(a, torch.int32)
+        if t.numel() != nq:
+            raise ValueError(f"stop_at has {t.numel()} values for {nq} queries")
+        return t
+
+    def _rrt_launch(self, res, stop, lanes, schedule, resume, work_key="rrt"):
+        """One trrt_rrt_batch call over the inputs kept in res._keep, writing res's arrays."""
+        starts, goals, sample_xy, sample_th, mid, P, g = res._keep
+        nq, K = res.node_x.shape[0], res.K
+        pack = res._packed
+        wb = self.lib.trrt_rrt_workspace_bytes(nq, K)
+        work = self._scratch(work_key, wb)  # concurrent launches (rrt_host) must not share a workspace
+        ptr = lambda t: t.data_ptr() if t is not None else None  # noqa: E731
+        a = _lib.CRrtArgs(d_bits=g.bits.data_ptr(), n_maps=g.n_maps, H=g.H, W=g.W, d_map_id=ptr(mid),
+                          params=P.to_c(), n_queries=nq, K=K, lanes_per_query=int(lanes), schedule=int(schedule),
+                          sample_xy_i16=int(sample_xy.dtype == torch.int16),
+                          d_start=starts.data_ptr(), d_goal=goals.data_ptr(), d_sample_xy=sample_xy.data_ptr(),
+                          d_sample_th=sample_th.data_ptr(), d_node_x=res.node_x.data_ptr(),
+                          d_node_y=res.node_y.data_ptr(), d_node_th=res.node_theta.data_ptr(),
+                          d_parent=res.parent.data_ptr(), d_u=ptr(res.u), d_n_nodes=res.n_nodes.data_ptr(),
+                          d_sol=res.sol.data_ptr(), d_status=res.status.data_ptr(), d_iters=res.iters.data_ptr(),
+                          d_it_near=ptr(res.it_near), d_it_new=ptr(res.it_new), d_it_code=ptr(res.it_code),
+                          d_los_log=ptr(res.los_log), d_n_los=ptr(res.n_los), d_counters=ptr(res.counters),
+                          d_work=work.data_ptr(), work_bytes=work.numel(),
+                          d_pack_rows=ptr(res.pack_total) if pack else None, d_row_start=ptr(res.row_start) if pack else None,
+                          d_pack_x=ptr(res.pack_x) if pack else None, d_pack_y=ptr(res.pack_y) if pack else None,
+                          d_pack_th=ptr(res.pack_theta) if pack else None,
+                          d_pack_parent=ptr(res.pack_parent) if pack else None,
+                          d_pack_u=ptr(res.pack_u) if (pack and res.u is not None) else None,
+                          d_stop_at=ptr(stop), resume=int(resume))
+        _lib.check(self.lib.trrt_rrt_batch(C.byref(a), self._stream()), "trrt_rrt_batch")
+        res.lanes = int(lanes)
+        res._stop = stop  # alive until the stream has consumed it
 
     _TREE = ("node_x", "node_y", "node_theta", "parent", "u")
     _PACKED = {"node_x": "pack_x", "node_y": "pack_y", "node_theta": "pack_theta", "parent": "pack_parent", "u": "pack_u"}

@@ -154,10 +154,12 @@ def rrt(start, goal, debug=False):
 
 
 def rrt_batch(starts, goals, seeds=None, sample_xy=None, sample_th=None, K=None, logs=False, lanes=0,
-              seed_stream="host") -> RrtResult:
+              seed_stream="host", stop_at=None) -> RrtResult:
     """Many independent rrt() calls in one launch.  Either pass per-query `seeds` (the stream of query q equals
     `np.random.seed(seeds[q])` followed by K-1 rand_conf calls, drawn by numpy on the host with seed_stream="host" or
-    on the device with seed_stream="device", Planner.rand_conf: the same bits) or explicit sample arrays."""
+    on the device with seed_stream="device", Planner.rand_conf: the same bits) or explicit sample arrays.
+    stop_at: per-query iteration stops (Planner.rrt); Planner.rrt_resume continues the paused queries with the samples
+    the result keeps."""
     if seed_stream not in SEED_STREAMS:
         raise ValueError(f"seed_stream must be one of {SEED_STREAMS}")
     p = _context.current_planner()
@@ -173,14 +175,14 @@ def rrt_batch(starts, goals, seeds=None, sample_xy=None, sample_th=None, K=None,
         nq = len(starts)
         if seed_stream == "device":
             sample_xy, sample_th = p.rand_conf(goals, seeds, K)
-            return p.rrt(starts, goals, sample_xy, sample_th, K=K, logs=logs, lanes=lanes)
+            return p.rrt(starts, goals, sample_xy, sample_th, K=K, logs=logs, lanes=lanes, stop_at=stop_at)
         sample_xy = np.empty((nq, K - 1, 2), np.int32)
         sample_th = np.empty((nq, K - 1), np.float64)
         for q in range(nq):
             g = ((goals[q, 0], goals[q, 1]), goals[q, 2])
             sample_xy[q], sample_th[q] = samples.make_stream(g, K - 1, int(seeds[q]), p.grid.shape, P.xystdv,
                                                              P.anglestdv)
-    return p.rrt(starts, goals, sample_xy, sample_th, K=K, logs=logs, lanes=lanes)
+    return p.rrt(starts, goals, sample_xy, sample_th, K=K, logs=logs, lanes=lanes, stop_at=stop_at)
 
 
 def findnearest(tree, goal):
