@@ -228,6 +228,43 @@ size_t trrt_rrt_workspace_bytes(int64_t n_queries, int32_t K);
 int trrt_rrt_batch(const trrt_rrt_args *args, void *stream);
 
 /* ---------------------------------------------------------------------------
+ * Seed races (OR-parallel RRT).  The same rrt.rrt loop (rrt.py:141-201) for
+ * queries that race each other in groups: usually one (start, goal) problem
+ * with many sample streams, of which the first to reach the goal is wanted.
+ * trrt_rrt_batch(args, s) is trrt_rrt_race_batch(args, NULL, s).
+ *
+ * best[g] is the smallest d_iters of a member of group g whose status is
+ * TRRT_OK_FOUND (d_iters counts the solving iteration).  Rule: a member of g
+ * runs no loop iteration it (0-based) once a member of g is known to have
+ * found the goal with iters <= it.  Hence:
+ *   - the members that solve at best[g] are never cut, and d_key[g] ends as
+ *     (best[g] << 32) | q with q the LOWEST query index among them: the argmin
+ *     of a run of every member to its end, whatever the lanes, schedule,
+ *     timing or number of SMs;
+ *   - a member that is cut has status TRRT_PAUSED and holds exactly what
+ *     rrt.rrt plans with K = d_iters[q] + 1 (see d_stop_at / resume); where it
+ *     is cut depends on timing, within best[g] <= d_iters[q] <= K-1;
+ *   - members that end otherwise (found later but before they learnt of the
+ *     winner, reference raises, capacity) and groups without a winner give the
+ *     outputs of trrt_rrt_batch bit for bit.
+ * On a call with resume = 0 the library fills d_key with 0xff bytes (UINT64_MAX
+ * = no member has found the goal) on the call's stream.  On a resume call the
+ * caller passes back the same d_key, untouched: paused members continue up to
+ * min(d_stop_at[q], best[g]) and may be cut again; a member whose d_iters[q]
+ * is >= best[g] is not written.  A resume through trrt_rrt_batch continues
+ * paused members as plain queries.  Rejected (TRRT_ERR_INVALID_ARGUMENT,
+ * before any device work): d_row_start with a race, n_groups < 1, NULL d_group
+ * or d_key, n_queries >= 2^32.
+ * ------------------------------------------------------------------------- */
+typedef struct trrt_rrt_race {
+    const int32_t *d_group; /* [n_queries] race group of query q; ids outside [0, n_groups) race nobody */
+    int64_t n_groups;
+    uint64_t *d_key;        /* [n_groups] (iters << 32) | q of the winner, UINT64_MAX = none */
+} trrt_rrt_race;
+
+int trrt_rrt_race_batch(const trrt_rrt_args *args, const trrt_rrt_race *race, void *stream);
+
+/* ---------------------------------------------------------------------------
  * Single-step entry points (batches of independent inputs, one result each);
  * they run the same device functions as the fused kernel.
  *   trrt_steer_batch  replaces rrt.steer (rrt.py:306-541).

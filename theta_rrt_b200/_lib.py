@@ -50,6 +50,11 @@ class CRrtArgs(C.Structure):
     ]
 
 
+class CRrtRace(C.Structure):
+    """struct trrt_rrt_race."""
+    _fields_ = [("d_group", C.c_void_p), ("n_groups", C.c_int64), ("d_key", C.c_void_p)]
+
+
 class CThetaArgs(C.Structure):
     """struct trrt_theta_args."""
     _fields_ = [
@@ -110,6 +115,7 @@ SIGNATURES = {
                                      C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "trrt_rrt_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int32]),
     "trrt_rrt_batch": (C.c_int, [C.POINTER(CRrtArgs), C.c_void_p]),
+    "trrt_rrt_race_batch": (C.c_int, [C.POINTER(CRrtArgs), C.POINTER(CRrtRace), C.c_void_p]),
     "trrt_steer_batch": (C.c_int, [C.POINTER(CParams), C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "trrt_drive_batch": (C.c_int, [C.POINTER(CParams), C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
     "trrt_arc_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int64, C.c_void_p,

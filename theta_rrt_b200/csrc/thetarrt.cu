@@ -989,13 +989,24 @@ static BikeParams to_dev(const trrt_params &p) {
     return b;
 }
 
-int trrt_rrt_batch(const trrt_rrt_args *args, void *stream) {
+int trrt_rrt_batch(const trrt_rrt_args *args, void *stream) { return trrt_rrt_race_batch(args, nullptr, stream); }
+
+int trrt_rrt_race_batch(const trrt_rrt_args *args, const trrt_rrt_race *race, void *stream) {
     if (!args) return TRRT_ERR_INVALID_ARGUMENT;
     const trrt_rrt_args &A = *args;
+    // packed rows plan whole runs; the key packs the query index into 32 bits
+    if (race && (A.d_row_start || race->n_groups < 1 || !race->d_group || !race->d_key || A.n_queries > (int64_t)0xffffffffll))
+        return TRRT_ERR_INVALID_ARGUMENT;
     int e = check_map(A.n_maps, A.H, A.W);
     if (e) return e;
     if (A.n_queries < 0 || A.K < 1) return TRRT_ERR_INVALID_ARGUMENT;
-    if (A.n_queries == 0) return TRRT_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    // a fresh race starts with no member that has found the goal; a resume keeps the caller's keys
+    const bool fill_key = race && A.resume == 0;
+    if (A.n_queries == 0) {
+        if (fill_key) CUDA_TRY(cudaMemsetAsync(race->d_key, 0xff, (size_t)race->n_groups * sizeof(uint64_t), st));
+        return TRRT_OK;
+    }
     if (!A.d_bits || !A.d_start || !A.d_goal || (A.K > 1 && (!A.d_sample_xy || !A.d_sample_th)) || !A.d_node_x || !A.d_node_y || !A.d_node_th ||
         !A.d_parent || !A.d_n_nodes || !A.d_sol || !A.d_status || !A.d_iters || !A.d_work)
         return TRRT_ERR_INVALID_ARGUMENT;
@@ -1020,7 +1031,11 @@ int trrt_rrt_batch(const trrt_rrt_args *args, void *stream) {
     d.px = A.d_pack_x; d.py = A.d_pack_y; d.pth = A.d_pack_th; d.pparent = A.d_pack_parent; d.pu = A.d_pack_u;
     d.tab = (int32_t *)((char *)A.d_work + 256); d.tsize = rrt_tsize(A.K);
     d.stop_at = A.d_stop_at; d.resume = A.resume;
-    cudaStream_t st = (cudaStream_t)stream;
+    d.race_group = race ? race->d_group : nullptr; d.n_race_groups = race ? race->n_groups : 0;
+    d.race_key = race ? (unsigned long long *)race->d_key : nullptr;
+    if (G != 1 && G != 2 && G != 4 && G != 8 && G != 16 && G != 32) return TRRT_ERR_INVALID_ARGUMENT;
+    if (A.schedule != 0 && A.schedule != 1) return TRRT_ERR_INVALID_ARGUMENT;
+    if (fill_key) CUDA_TRY(cudaMemsetAsync(race->d_key, 0xff, (size_t)race->n_groups * sizeof(uint64_t), st));
     int threads = 128;
     int64_t blocks = (A.n_queries * G + threads - 1) / threads;
     if (A.schedule == 1) { // cooperative: G lanes on one iteration at a time

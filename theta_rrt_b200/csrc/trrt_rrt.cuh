@@ -54,6 +54,11 @@ struct RrtDev {
     // pause and resume (see trrt_rrt_args in thetarrt.h): per-query stop iteration or nullptr (K-1); resume paused queries
     const int32_t *stop_at;
     int resume;
+    // seed races (see trrt_rrt_race in thetarrt.h): race group of each query or nullptr (no race), and per group the
+    // key (iters << 32) | q of the best FOUND member published so far, ~0 = none
+    const int32_t *race_group;
+    int64_t n_race_groups;
+    unsigned long long *race_key;
 };
 
 __device__ __forceinline__ unsigned hash3(double x, double y, double t) {
@@ -254,9 +259,40 @@ __device__ __forceinline__ int query_limit(const RrtDev &a, int64_t q) {
     return s < 0 ? 0 : (s > a.K - 1 ? a.K - 1 : s);
 }
 
-// a resume call continues query q: it is paused and its stop lies beyond the iterations it has run
-__device__ __forceinline__ bool query_resumes(const RrtDev &a, int64_t q) {
-    return a.status[q] == TRRT_PAUSED && a.iters[q] < query_limit(a, q);
+// Seed races.  A member of race group g runs no iteration it >= best[g], the smallest iters of a member of g that ended
+// with TRRT_OK_FOUND.  Members publish with atomicMin on race_key[g] = (iters << 32) | q, so the key keeps the lowest
+// query index among equal iteration counts.  A member reads the key while it runs: a stale value is >= the final best[g]
+// and only delays a cut, so the members that solve at best[g] are never cut and the winner does not depend on timing.
+// Group ids outside [0, n_race_groups) race nobody.
+__device__ __forceinline__ int race_group_of(const RrtDev &a, int64_t q) {
+    const int gi = a.race_group[q];
+    return (gi >= 0 && gi < a.n_race_groups) ? gi : -1;
+}
+__device__ __forceinline__ unsigned long long race_key_load(const unsigned long long *p) {
+    unsigned long long v; // bypasses L1: other SMs publish into L2
+    asm volatile("ld.relaxed.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p));
+    return v;
+}
+// lim lowered to the best[g] the group's key shows now (a.race_group set; one lane reads, the caller broadcasts)
+__device__ __forceinline__ int race_limit(const RrtDev &a, int64_t q, int lim) {
+    const int gi = race_group_of(a, q);
+    if (gi < 0) return lim;
+    TRRT_CHECK(gi < a.n_race_groups);
+    const unsigned long long best = race_key_load(a.race_key + gi) >> 32; // 0xffffffff: no member has found the goal
+    return best < (unsigned long long)lim ? (int)best : lim;
+}
+// the same bound, read by the group's leader and the same in every lane
+template <int G>
+__device__ __forceinline__ int race_limit_group(const RrtDev &a, int64_t q, const Group<G> &g, int lim) {
+    if (!a.race_group) return lim;
+    return g.bcast(g.gl == 0 ? race_limit(a, q, lim) : lim, 0);
+}
+
+// a resume call continues query q: it is paused and its stop (and its race group's best) lies beyond the iterations it
+// has run
+template <int G>
+__device__ __forceinline__ bool query_resumes(const RrtDev &a, int64_t q, const Group<G> &g) {
+    return a.status[q] == TRRT_PAUSED && a.iters[q] < race_limit_group<G>(a, q, g, query_limit(a, q));
 }
 
 // pointers of query q (no memory is touched)
@@ -427,6 +463,10 @@ __device__ __forceinline__ void rrt_finish(const RrtDev &a, int64_t q, const Gro
         a.sol[q] = sol;
         a.status[q] = status;
         a.iters[q] = iters;
+        if (a.race_group && status == TRRT_OK_FOUND) { // publish to the race group (launcher: q < 2^32)
+            const int gi = race_group_of(a, q);
+            if (gi >= 0) atomicMin(a.race_key + gi, ((unsigned long long)iters << 32) | (unsigned long long)q);
+        }
         if (a.n_los) a.n_los[q] = nlos;
         if (a.counters && c) {
             unsigned long long *o = a.counters + q * 9;
@@ -476,7 +516,7 @@ __global__ void __launch_bounds__(128) rrt_kernel_coop(const RrtDev a) {
     const Group<G> g;
     const int64_t q = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) / G;
     if (q >= a.nq) return; // whole groups leave together
-    if (a.resume && !query_resumes(a, q)) return; // not written at all
+    if (a.resume && !query_resumes<G>(a, q, g)) return; // not written at all
     const int K = a.K;
     RrtQuery Q;
     RrtCounters c = {0, 0, 0, 0, 0, 0, 0, 0, 0};
@@ -486,6 +526,7 @@ __global__ void __launch_bounds__(128) rrt_kernel_coop(const RrtDev a) {
     int k;
     for (k = it0 + 1; k <= Q.limit; k++) {
         const int it = k - 1;
+        if (a.race_group && it >= race_limit_group<G>(a, q, g, Q.limit)) break; // a member of the race group found the goal by it
         int sx, sy;
         sample_xy(a, Q, it, sx, sy);
         const double qx = (double)sx, qy = (double)sy;
@@ -845,7 +886,7 @@ __global__ void __launch_bounds__(SPEC_THREADS, SPEC_BLOCKS_PER_SM) rrt_kernel_s
                 q = (int64_t)qq;
                 sol = -1; status = TRRT_OK_NOT_FOUND;
                 if (a.resume) {
-                    if (!query_resumes(a, q)) continue;
+                    if (!query_resumes<G>(a, q, g)) continue;
                     rrt_setup_resume<G>(a, q, g, Q, n, iters, nlos);
                     k0 = iters;
                 } else {
@@ -867,9 +908,11 @@ __global__ void __launch_bounds__(SPEC_THREADS, SPEC_BLOCKS_PER_SM) rrt_kernel_s
         Expand e;
         e.code = TRRT_IT_NOT_RUN; e.flags = 0; e.lospx = e.arcpx = e.arcang = e.drive = 0;
         e.wx = e.wy = e.wth = NAN; // never equal to a node
+        // iterations it < lim run: the query's stop, lowered to its race group's best (sQ is not written in a window)
+        const int lim = have ? race_limit_group<G>(a, q, g, Q.limit) : 0;
         if (have) {
             const int my_it = k0 + g.gl;
-            if (my_it < Q.limit) { // beyond the query's stop: TRRT_IT_NOT_RUN cuts the window there
+            if (my_it < lim) { // beyond the query's stop: TRRT_IT_NOT_RUN cuts the window there
                 int sx, sy;
                 sample_xy(a, Q, my_it, sx, sy);
                 qx = (double)sx; qy = (double)sy;
@@ -1075,7 +1118,7 @@ __global__ void __launch_bounds__(SPEC_THREADS, SPEC_BLOCKS_PER_SM) rrt_kernel_s
         g.sync(); // tree and index writes of this window are visible to every lane's next phase A
         TRRT_PROF({ const unsigned long long s_ = clock64() - t3_; pf[7] += s_; pf[8] += s_ * s_ >> 10; const unsigned long long w_ = clock64() - t2_; pf[9] += w_ * w_ >> 10; })
         k0 += end;
-        if (finished || k0 >= Q.limit) { // query finished or paused
+        if (finished || k0 >= lim) { // query finished or paused
             rrt_finish<G>(a, q, g, Q, K, iters, n, sol, status, nlos, nullptr);
             g.sync();
             have = false;

@@ -15,7 +15,7 @@ from dataclasses import dataclass, field
 import numpy as np
 import torch
 
-from . import _lib
+from . import _lib, samples
 from .grid import OccupancyGrid
 from .params import Params
 
@@ -66,9 +66,41 @@ class RrtResult:
     pack_theta: torch.Tensor | None = None
     pack_parent: torch.Tensor | None = None
     pack_u: torch.Tensor | None = None
+    # seed races (rrt(..., race=...)): per race group, the key (iters << 32) | q of the winner (int64 bit pattern of the
+    # C ABI's uint64, -1 = none), and decoded: the winning query (-1 = none) and its iters (-1 = none)
+    race_key: torch.Tensor | None = None
+    race_winner: torch.Tensor | None = None
+    race_iters: torch.Tensor | None = None
 
     def host(self):
         return _host_dict(self)
+
+
+@dataclass
+class RaceResult:
+    """Planner.rrt_race output, per problem: winner (query index into result, -1 = no seed reached the goal),
+    winner_seed (int64, -1 = none) and iters (the winner's iterations, -1 = none); result holds every member."""
+    result: RrtResult
+    winner: torch.Tensor
+    winner_seed: torch.Tensor
+    iters: torch.Tensor
+
+    def host(self):
+        return {"winner": self.winner.cpu().numpy(), "winner_seed": self.winner_seed.cpu().numpy(),
+                "iters": self.iters.cpu().numpy()}
+
+
+def race_key(iters, q):
+    """The race key of a member that found the goal: (iters << 32) | q, as trrt_rrt_race_batch packs it."""
+    return (int(iters) << 32) | int(q)
+
+
+def race_decode(key: torch.Tensor):
+    """int64 race keys -> (winner int32, iters int32), -1 where the key is UINT64_MAX (no member found the goal)."""
+    none = key == -1
+    winner = torch.where(none, torch.full_like(key, -1), key & 0xffffffff).to(torch.int32)
+    iters = torch.where(none, torch.full_like(key, -1), key >> 32).to(torch.int32)
+    return winner, iters
 
 
 @dataclass
@@ -247,7 +279,8 @@ class Planner:
 
     # ------------------------------------------------------------------ K2
     def rrt(self, starts, goals, sample_xy, sample_th, K=None, params=None, map_id=None, logs=False, want_u=True,
-            counters=False, lanes=0, schedule=0, work_key="rrt", reuse=None, pack=False, packed=None, stop_at=None):
+            counters=False, lanes=0, schedule=0, work_key="rrt", reuse=None, pack=False, packed=None, stop_at=None,
+            race=None, race_groups=None):
         """rrt.rrt for a batch.  starts/goals float64 [q,3] (x, y, theta_deg); sample_xy int32 [q,K-1,2];
         sample_th float64 [q,K-1].  K = builtins.K (node capacity; K-1 iterations).
         pack=True: the kernel also leaves a packed copy of the tree rows that exist (pack_x, pack_y, pack_theta,
@@ -255,10 +288,17 @@ class Planner:
         pass a dict of such arrays to use; its pack_total must then hold the first row to use (0 for arrays of this call's own).
         stop_at: an int or [q] ints in [0, K-1] (a CUDA int32 tensor is clamped to that range on the device): query q runs
         no iteration it >= stop_at[q].  A query stopped with iterations left has status PAUSED and iters = stop_at[q], and
-        holds exactly what rrt.rrt plans with K = stop_at[q] + 1; rrt_resume continues it."""
+        holds exactly what rrt.rrt plans with K = stop_at[q] + 1; rrt_resume continues it.
+        race: [q] race group ids (seed races, trrt_rrt_race_batch): a query runs no iteration it once a member of its
+        group has found the goal with iters <= it, and is then PAUSED.  Host ids must be >= 0 and give race_groups =
+        max + 1 groups; a CUDA int32 tensor is used in place and needs race_groups (ids outside [0, race_groups) race
+        nobody).  The result's race_key / race_winner / race_iters hold each group's winner: the lowest query index
+        among the members with the fewest iterations to the goal."""
         P = params or self.params
         if pack and stop_at is not None:
             raise ValueError("pack=True plans whole runs: it cannot be combined with stop_at")
+        if pack and race is not None:
+            raise ValueError("pack=True plans whole runs: it cannot be combined with a race")
         with torch.cuda.device(self.device):
             starts = self._dev(starts, torch.float64).reshape(-1, 3)
             goals = self._dev(goals, torch.float64).reshape(-1, 3)
@@ -275,6 +315,7 @@ class Planner:
             sample_xy = self._dev(sample_xy, torch.int16 if xy16 else torch.int32).reshape(nq, K - 1, 2)
             mid = self._map_ids(map_id, nq)
             stop = self._stop_at(stop_at, nq, K)
+            groups = self._race_groups(race, race_groups, nq)
             dev = self.device
             f64 = dict(dtype=torch.float64, device=dev)
             i32 = dict(dtype=torch.int32, device=dev)
@@ -312,15 +353,21 @@ class Planner:
             # the inputs stay alive until the stream has consumed them, and rrt_resume plans with them again
             res._keep = (starts, goals, sample_xy, sample_th, mid, P, self.grid)
             res._packed = bool(pack)
+            res._race = None
+            if groups is not None:
+                res._race = groups
+                res.race_key = torch.empty(groups[1], dtype=torch.int64, device=dev)
             self._rrt_launch(res, stop, lanes, schedule, resume=False, work_key=work_key)
         return res
 
-    def rrt_resume(self, res: RrtResult, stop_at=None, lanes=0, schedule=0) -> RrtResult:
+    def rrt_resume(self, res: RrtResult, stop_at=None, lanes=0, schedule=0, race=True) -> RrtResult:
         """Continue the PAUSED queries of `res` (a result of rrt(..., stop_at=...)) in place, with the inputs, params and
         map ids it was planned with: each runs from iteration iters[q] up to stop_at[q] (default K-1), and may pause
         again.  Other queries, and paused ones whose stop is <= iters[q], are not written.  lanes and schedule may differ
         from the pausing call.  Any sequence of pauses and resumes returns what one uninterrupted call returns, bit for
-        bit, except counter 7 (hash probes, which count probes in the query's rebuilt index).  Returns res."""
+        bit, except counter 7 (hash probes, which count probes in the query's rebuilt index).  A result planned with a race
+        keeps racing (paused members continue up to their group's best iters, and may be cut again) unless race=False,
+        which continues them as plain queries and leaves race_key as it is.  Returns res."""
         keep = getattr(res, "_keep", None)
         if keep is None or len(keep) != 7 or keep[6] is not self.grid:
             raise ValueError("rrt_resume continues a result that Planner.rrt planned on this planner's grid")
@@ -328,8 +375,35 @@ class Planner:
             raise ValueError("a result planned with pack=True cannot be resumed")
         with torch.cuda.device(self.device):
             stop = self._stop_at(stop_at, res.node_x.shape[0], res.K)
-            self._rrt_launch(res, stop, lanes, schedule, resume=True)
+            self._rrt_launch(res, stop, lanes, schedule, resume=True, race=bool(race))
         return res
+
+    def _race_groups(self, race, race_groups, nq):
+        """race / race_groups of rrt -> (int32 [nq] device tensor, n_groups), or None."""
+        if race is None:
+            if race_groups is not None:
+                raise ValueError("race_groups is given without race group ids")
+            return None
+        if isinstance(race, torch.Tensor) and race.is_cuda:
+            if race_groups is None:
+                raise ValueError("a CUDA tensor of race group ids needs race_groups (the ids are not read on the host)")
+            t = self._dev(race, torch.int32).reshape(-1)
+            n = int(race_groups)
+        else:
+            a = np.asarray(race.cpu() if isinstance(race, torch.Tensor) else race).reshape(-1)
+            if a.dtype.kind not in "iu":
+                raise ValueError(f"race group ids must be integers, got {a.dtype}")
+            if a.size and int(a.min()) < 0:
+                raise ValueError("race group ids must be >= 0")
+            n = int(race_groups) if race_groups is not None else (int(a.max()) + 1 if a.size else 1)
+            if a.size and int(a.max()) >= 2 ** 31:
+                raise ValueError("race group ids must fit int32")
+            t = self._dev(a, torch.int32)
+        if n < 1:
+            raise ValueError("race_groups must be >= 1")
+        if t.numel() != nq:
+            raise ValueError(f"race has {t.numel()} group ids for {nq} queries")
+        return t, n
 
     def _stop_at(self, stop_at, nq, K):
         """stop_at of rrt / rrt_resume -> int32 [nq] device tensor, or None.  Host values outside [0, K-1] raise."""
@@ -351,8 +425,9 @@ class Planner:
             raise ValueError(f"stop_at has {t.numel()} values for {nq} queries")
         return t
 
-    def _rrt_launch(self, res, stop, lanes, schedule, resume, work_key="rrt"):
-        """One trrt_rrt_batch call over the inputs kept in res._keep, writing res's arrays."""
+    def _rrt_launch(self, res, stop, lanes, schedule, resume, work_key="rrt", race=True):
+        """One trrt_rrt_race_batch call over the inputs kept in res._keep, writing res's arrays; the race of res, if any,
+        takes part unless race=False."""
         starts, goals, sample_xy, sample_th, mid, P, g = res._keep
         nq, K = res.node_x.shape[0], res.K
         pack = res._packed
@@ -376,7 +451,14 @@ class Planner:
                           d_pack_parent=ptr(res.pack_parent) if pack else None,
                           d_pack_u=ptr(res.pack_u) if (pack and res.u is not None) else None,
                           d_stop_at=ptr(stop), resume=int(resume))
-        _lib.check(self.lib.trrt_rrt_batch(C.byref(a), self._stream()), "trrt_rrt_batch")
+        groups = getattr(res, "_race", None) if race else None
+        rc = None
+        if groups is not None:
+            rc = _lib.CRrtRace(d_group=groups[0].data_ptr(), n_groups=groups[1], d_key=res.race_key.data_ptr())
+        _lib.check(self.lib.trrt_rrt_race_batch(C.byref(a), C.byref(rc) if rc is not None else None, self._stream()),
+                   "trrt_rrt_race_batch")
+        if groups is not None:
+            res.race_winner, res.race_iters = race_decode(res.race_key)
         res.lanes = int(lanes)
         res._stop = stop  # alive until the stream has consumed it
 
@@ -403,6 +485,8 @@ class Planner:
         row_start (int64 [q]).  The size of a piece's copy is known once its row count has reached the host, so the
         copies of a batch are issued one call later (or in host_sync()), on copy streams of their own, while the next
         batch is already being planned; the packed rows are double-buffered per piece."""
+        if kw.get("race") is not None:
+            raise ValueError("rrt_host plans independent queries: use rrt(..., race=...) for seed races")
         ins = [t if isinstance(t, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(t))
                for t in (starts, goals, sample_xy, sample_th)]
         nq = ins[0].shape[0]
@@ -783,6 +867,42 @@ class Planner:
                                                      nz.data_ptr(), sxy.data_ptr(), int(xy_dtype == torch.int16),
                                                      sth.data_ptr(), self._stream()), "trrt_rand_conf_batch")
         return sxy, sth
+
+    def rrt_race(self, starts, goals, seeds, K=None, seed_stream="device", lanes=0, schedule=0, stop_at=None,
+                 logs=False, params=None) -> RaceResult:
+        """Seed races for P problems: problem p = (starts[p], goals[p]) float64 [P, 3] is planned once per seed of
+        seeds[p] (integers [P, S], the stream of np.random.seed(seed) followed by rand_conf calls, drawn on the device or,
+        with seed_stream="host", by numpy), and its S members race each other (rrt(..., race=...)): member s of problem p
+        is query p * S + s of the result.  One call; returns per problem the winning query, its seed and its iters."""
+        if seed_stream not in SEED_STREAMS:
+            raise ValueError(f"seed_stream must be one of {SEED_STREAMS}")
+        P = params or self.params
+        K = int(K if K is not None else P.K)
+        starts = np.asarray(starts.cpu() if isinstance(starts, torch.Tensor) else starts, np.float64).reshape(-1, 3)
+        goals = np.asarray(goals.cpu() if isinstance(goals, torch.Tensor) else goals, np.float64).reshape(-1, 3)
+        seeds = np.asarray(seeds.cpu() if isinstance(seeds, torch.Tensor) else seeds)
+        n_prob = starts.shape[0]
+        if goals.shape[0] != n_prob or seeds.ndim != 2 or seeds.shape[0] != n_prob or seeds.shape[1] < 1:
+            raise ValueError(f"rrt_race wants starts and goals [P, 3] and seeds [P, S], got {starts.shape}, {goals.shape}, "
+                             f"{seeds.shape}")
+        S = seeds.shape[1]
+        flat = legacy_seeds(seeds)
+        m_starts, m_goals = np.repeat(starts, S, axis=0), np.repeat(goals, S, axis=0)
+        if seed_stream == "device":
+            sxy, sth = self.rand_conf(m_goals, flat, K, params=P)
+        else:
+            sxy = np.empty((len(flat), K - 1, 2), np.int32)
+            sth = np.empty((len(flat), K - 1), np.float64)
+            for q, g in enumerate(m_goals):
+                sxy[q], sth[q] = samples.make_stream(((g[0], g[1]), g[2]), K - 1, int(flat[q]), self.grid.shape,
+                                                     P.xystdv, P.anglestdv)
+        res = self.rrt(m_starts, m_goals, sxy, sth, K=K, params=P, logs=logs, lanes=lanes, schedule=schedule,
+                       stop_at=stop_at, race=np.repeat(np.arange(n_prob), S), race_groups=n_prob)
+        seed_dev = torch.from_numpy(flat.astype(np.int64)).to(self.device)
+        w = res.race_winner
+        found = w >= 0
+        winner_seed = torch.where(found, seed_dev[w.clamp(min=0).long()], torch.full_like(w, -1, dtype=torch.int64))
+        return RaceResult(result=res, winner=w, winner_seed=winner_seed, iters=res.race_iters)
 
     # ------------------------------------------------------------------ main.py missions
     def missions(self, start_goal=None, waypoints=None, seeds=None, normals=None, normal_range=None, map_id=None, K=None,

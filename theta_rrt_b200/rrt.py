@@ -185,6 +185,27 @@ def rrt_batch(starts, goals, seeds=None, sample_xy=None, sample_th=None, K=None,
     return p.rrt(starts, goals, sample_xy, sample_th, K=K, logs=logs, lanes=lanes, stop_at=stop_at)
 
 
+def rrt_race(start, goal, seeds, K=None):
+    """Seed race for one problem: rrt(start, goal) under np.random.seed(seed) for every seed of `seeds`, planned in one
+    launch whose members stop once one of them has reached the goal (Planner.rrt_race, device-drawn streams).  Returns
+    (seed, (sol, G, cameFrom)) for the winner -- the seed that reaches the goal in the fewest iterations, the first of
+    them in `seeds` on a tie -- where the tuple is what `np.random.seed(seed); rrt(start, goal)` returns; (None, None)
+    when no seed reaches the goal.  numpy's global generator is not touched."""
+    p = _context.current_planner()
+    K = int(K or p.params.K)
+    start = (start[0], standardangle(start[1]))
+    goal = (goal[0], standardangle(goal[1]))
+    seeds = np.asarray(seeds).reshape(1, -1)
+    r = p.rrt_race([[start[0][0], start[0][1], start[1]]], [[goal[0][0], goal[0][1], goal[1]]], seeds, K=K, logs=True)
+    w = int(r.winner.cpu()[0])
+    if w < 0:
+        return None, None
+    res = r.result
+    h = {k: getattr(res, k)[w:w + 1].cpu().numpy() for k in ("n_nodes", "node_x", "node_y", "node_theta", "parent", "u",
+                                                               "sol", "it_near", "it_new")}
+    return int(seeds[0, w]), result_to_dicts(h, 0, start)
+
+
 def findnearest(tree, goal):
     """rrt.py:117-128 for a G dict as returned by rrt()."""
     p = _context.current_planner()
