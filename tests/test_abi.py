@@ -3,13 +3,12 @@ import ctypes as C
 import os
 import re
 
+from tests import util
 from theta_rrt_b200 import _lib
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def header_symbols():
-    src = open(os.path.join(ROOT, "include", "thetarrt.h")).read()
+    src = open(os.path.join(util.ROOT, "include", "thetarrt.h")).read()
     src = re.sub(r"/\*.*?\*/", "", src, flags=re.S)
     return sorted(set(re.findall(r"\b(trrt_[a-z0-9_]+)\s*\(", src)))
 
@@ -42,6 +41,15 @@ def test_trivial_host_calls():
 
 
 def test_struct_layouts_match_header():
+    # every ctypes mirror has the header's members in the header's order
+    for name, mirror in (("trrt_params", _lib.CParams), ("trrt_rrt_args", _lib.CRrtArgs), ("trrt_rrt_race", _lib.CRrtRace),
+                         ("trrt_theta_args", _lib.CThetaArgs), ("trrt_mission_args", _lib.CMissionArgs),
+                         ("trrt_legacy_normals_args", _lib.CLegacyNormalsArgs)):
+        assert [f[0] for f in mirror._fields_] == util.struct_members(name), name
+    # members added after d_pack_u keep the offsets of the earlier ones
+    assert _lib.CRrtArgs._fields_[-2:] == [("d_stop_at", C.c_void_p), ("resume", C.c_int32)]
+    assert "trrt_rrt_race_batch" in _lib.SIGNATURES
     # sizes the CUDA side was compiled with (offsets are exercised by the GPU tests)
     assert C.sizeof(_lib.CParams) == 8 + 8 * 8
     assert C.sizeof(_lib.CRrtArgs) % 8 == 0 and C.sizeof(_lib.CThetaArgs) % 8 == 0
+    assert C.sizeof(_lib.CRrtRace) == 24

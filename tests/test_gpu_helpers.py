@@ -9,16 +9,9 @@ import numpy as np
 import pytest
 
 from tests import util
-from tests.test_gpu_parity import planner_for
+from tests.util import O, planner_for  # noqa: F401  (O is a fixture)
 
 pytestmark = pytest.mark.gpu
-
-
-@pytest.fixture(scope="module")
-def O():
-    from oracle import c_oracle
-    c_oracle.lib()
-    return c_oracle
 
 
 def as_tuples(a):

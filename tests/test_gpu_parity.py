@@ -11,26 +11,9 @@ import numpy as np
 import pytest
 
 from tests import util
+from tests.util import O, bits_equal, planner_for  # noqa: F401  (O is a fixture)
 
 pytestmark = pytest.mark.gpu
-
-
-@pytest.fixture(scope="module")
-def O():
-    from oracle import c_oracle
-    c_oracle.lib()
-    return c_oracle
-
-
-def planner_for(free, **params):
-    from theta_rrt_b200 import OccupancyGrid, Params, Planner
-    return Planner(OccupancyGrid(free), Params(**params))
-
-
-def bits_equal(a, b):
-    a = np.ascontiguousarray(a, np.float64)
-    b = np.ascontiguousarray(b, np.float64)
-    return a.shape == b.shape and np.array_equal(a.view(np.int64), b.view(np.int64))
 
 
 # ------------------------------------------------------------------ grid + LOS

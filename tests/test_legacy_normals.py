@@ -12,6 +12,7 @@ import numpy as np
 import pytest
 
 from oracle import legacy_normals as L
+from tests.util import planner_for
 
 TL_LOG_EPS = 2.0 ** -66
 TL_LOG_MARGIN = 2.0 ** -5
@@ -166,13 +167,6 @@ def test_glibc_log_error_below_margin():
 
 
 # ------------------------------------------------------------------------------------------- GPU
-def planner_for(free=None):
-    from theta_rrt_b200 import OccupancyGrid, Params, Planner
-    if free is None:
-        free = np.ones((64, 64), bool)
-    return Planner(OccupancyGrid(free, device="cuda:0"), Params())
-
-
 def abi_draw(p, seeds, ranges, total, fix_cap):
     """trrt_legacy_normals_draw + host log + fixup through the C ABI with caller-given ranges.
     Returns (normals, undecided count)."""
@@ -207,7 +201,7 @@ def abi_draw(p, seeds, ranges, total, fix_cap):
 @pytest.mark.gpu
 def test_device_cfg3_streams_bitwise():
     """4 096 seeds x 15 000 normals (the cfg-3 rand_conf streams, 5 000 samples each)."""
-    p = planner_for()
+    p = planner_for(device="cuda:0")
     n, L_ = 4096, 15000
     seeds = np.arange(n, dtype=np.int64) * 7919 + 3
     ranges = np.stack([np.arange(n) * L_, np.arange(n) * L_ + L_], 1)
@@ -222,7 +216,7 @@ def test_device_cfg3_streams_bitwise():
 
 @pytest.mark.gpu
 def test_device_edge_seeds_odd_lengths_any_order_and_retry():
-    p = planner_for()
+    p = planner_for(device="cuda:0")
     seeds = EDGE_SEEDS * 2
     lengths = [0, 1, 2, 3, 245, 246, 491, 624, 1249, 15001, 7, 0, 999, 2, 246, 5000, 1, 313, 3, 10001]
     # ranges in a shuffled order with gaps between them: only [begin, end) of each seed is written
@@ -259,7 +253,7 @@ def test_rand_conf_matches_make_stream(maps, xy):
     import torch
     from theta_rrt_b200 import samples
     free = maps["map2"]
-    p = planner_for(free)
+    p = planner_for(free, device="cuda:0")
     rng = np.random.default_rng(8)
     nq, K = 64, 301
     goals = np.stack([rng.uniform(0, 300, nq), rng.uniform(0, 300, nq), rng.uniform(-900, 900, nq)], 1)
@@ -278,7 +272,7 @@ def test_missions_device_seed_stream_equals_host(maps):
     free = maps["map2"]
     sg = map2_queries(free, 256, 2024)
     seeds = np.arange(256) + 9000
-    p = planner_for(free)
+    p = planner_for(free, device="cuda:0")
     hh = p.missions(start_goal=sg, seeds=seeds, K=300).host()
     hd = p.missions(start_goal=sg, seeds=seeds, K=300, seed_stream="device").host()
     assert (hh["n_seg"] > 0).sum() > 200

@@ -10,18 +10,12 @@ import pytest
 
 from tests import util
 from tests.mission_oracle import mission_chain
+from tests.util import bits_equal_nan, planner_for
 from tests.test_main_chain import check_segments, golden
 
 
 def seed_normals(seed, K, n_seg):
     return np.random.RandomState(seed).standard_normal(3 * (K - 1) * n_seg)
-
-
-def bits_equal(a, b):
-    a, b = np.asarray(a, np.float64), np.asarray(b, np.float64)
-    if a.shape != b.shape or not np.array_equal(np.isnan(a), np.isnan(b)):
-        return False
-    return np.array_equal(np.where(np.isnan(a), 0.0, a).view(np.int64), np.where(np.isnan(b), 0.0, b).view(np.int64))
 
 
 def node_row(n):
@@ -33,15 +27,15 @@ def compare_with_oracle(h, m, o):
     assert int(h["status"][m]) == o["status"] and int(h["stop_seg"][m]) == o["stop_seg"], m
     for s, rec in enumerate(o["segments"]):
         for key in ("begin", "end", "solution", "nearest"):
-            assert bits_equal(h[key][m, s], node_row(rec[key])), (m, s, key)
-        assert bits_equal(h["mindist"][m, s], np.nan if rec["mindist"] is None else rec["mindist"]), (m, s)
+            assert bits_equal_nan(h[key][m, s], node_row(rec[key])), (m, s, key)
+        assert bits_equal_nan(h["mindist"][m, s], np.nan if rec["mindist"] is None else rec["mindist"]), (m, s)
         got = tuple(int(h[k][m, s]) for k in ("n_nodes", "n_edges", "iters", "seg_status"))
         assert got == (rec["n_nodes"], rec["n_edges"], rec["iters"], rec["status"]), (m, s)
     for s in range(len(o["segments"]), h["seg_status"].shape[1]):
         assert int(h["seg_status"][m, s]) == 255
     n = len(o["path"])
     assert int(h["path_len"][m]) == n, m
-    assert bits_equal(h["path"][m, :n], o["path"]), m
+    assert bits_equal_nan(h["path"][m, :n], o["path"]), m
     assert np.array_equal(h["path_seg"][m, :n], o["path_seg"]), m
 
 
@@ -102,11 +96,6 @@ def test_mission_records_conversion():
 
 
 # ---------------------------------------------------------------------------------------------------- GPU
-def planner_for(free, **kw):
-    from theta_rrt_b200 import OccupancyGrid, Params, Planner
-    return Planner(OccupancyGrid(free, device="cuda:0"), Params(**kw))
-
-
 def oracle_batch(free, h, seeds, K, maps_by_id=None, params=None):
     out = []
     for m, seed in enumerate(seeds):
@@ -147,7 +136,7 @@ def test_missions_reproduce_main_kat(maps, case):
     from theta_rrt_b200.main import mission_records
     free = maps[case["map"]]
     wp = [tuple(w) for w in case["waypoints"]]
-    h = planner_for(free).missions(waypoints=[wp], seeds=[case["seed"]], K=case["K"]).host()
+    h = planner_for(free, device="cuda:0").missions(waypoints=[wp], seeds=[case["seed"]], K=case["K"]).host()
     recs = mission_records(h, 0)
     check_segments(recs, case)
     compare_with_oracle(h, 0, mission_chain(free, wp, seed_normals(case["seed"], case["K"], len(wp) - 1), case["K"]))
@@ -169,7 +158,7 @@ def map2_batch(maps):
     free = maps["map2"]
     sg = map2_queries(free, 256, 2024)
     seeds = np.arange(256) + 9000
-    res = planner_for(free).missions(start_goal=sg, seeds=seeds, K=300)
+    res = planner_for(free, device="cuda:0").missions(start_goal=sg, seeds=seeds, K=300)
     h = res.host()
     return free, sg, seeds, h
 
@@ -194,7 +183,7 @@ def test_missions_map1_astar_small_k(maps):
     from oracle import c_oracle as O
     sg = map2_queries(free, 32, 77)
     seeds = np.arange(32) + 100
-    h = planner_for(free, THETASTAR=False).missions(start_goal=sg, seeds=seeds, K=100).host()
+    h = planner_for(free, device="cuda:0", THETASTAR=False).missions(start_goal=sg, seeds=seeds, K=100).host()
     assert h["n_seg"].max() > 50
     check_batch(h, oracle_batch(free, h, seeds, 100, params=O.Params(thetastar=0)), h["route"]["status"])
 
@@ -223,7 +212,7 @@ def test_missions_childless_tree_stop(maps, monkeypatch):
     free = maps["map2"]
     wp = [tuple(w) for w in M.REFERENCE_WAYPOINTS]
     seeds = np.arange(16)
-    h = planner_for(free).missions(waypoints=[wp] * 16, seeds=seeds, K=3).host()
+    h = planner_for(free, device="cuda:0").missions(waypoints=[wp] * 16, seeds=seeds, K=3).host()
     stops = 0
     M.set_map(free)
     monkeypatch.setattr(builtins, "K", 3)
@@ -248,27 +237,27 @@ def test_missions_childless_tree_stop(maps, monkeypatch):
 def test_missions_batch_invariance(map2_batch):
     free, sg, seeds, h = map2_batch
     perm = np.random.default_rng(3).permutation(len(sg))[:97]
-    h2 = planner_for(free).missions(start_goal=sg[perm], seeds=seeds[perm], K=300).host()
+    h2 = planner_for(free, device="cuda:0").missions(start_goal=sg[perm], seeds=seeds[perm], K=300).host()
     S2 = h2["seg_status"].shape[1]
     for i, m in enumerate(perm):
         for k in ("status", "stop_seg", "n_seg", "path_len"):
             assert h2[k][i] == h[k][m], (k, m)
         for k in ("begin", "end", "solution", "nearest", "mindist", "n_nodes", "n_edges", "iters", "seg_status"):
-            assert bits_equal(h2[k][i], h[k][m][:S2]), (k, m)
+            assert bits_equal_nan(h2[k][i], h[k][m][:S2]), (k, m)
             assert (h[k][m][S2:] == 255).all() if k == "seg_status" else True
         n = int(h["path_len"][m])
-        assert bits_equal(h2["path"][i, :n], h["path"][m, :n]) and np.array_equal(h2["path_seg"][i, :n], h["path_seg"][m, :n])
+        assert bits_equal_nan(h2["path"][i, :n], h["path"][m, :n]) and np.array_equal(h2["path_seg"][i, :n], h["path_seg"][m, :n])
 
 
 @pytest.mark.gpu
 def test_missions_path_cap_and_caller_normals(map2_batch):
     import torch
     free, sg, seeds, h = map2_batch
-    p = planner_for(free)
+    p = planner_for(free, device="cuda:0")
     sub = np.nonzero(h["path_len"] > 8)[0][:16]
     hc = p.missions(start_goal=sg[sub], seeds=seeds[sub], K=300, path_cap=5).host()
     assert np.array_equal(hc["path_len"], h["path_len"][sub])
-    assert bits_equal(hc["path"], h["path"][sub, :5])
+    assert bits_equal_nan(hc["path"], h["path"][sub, :5])
     with pytest.raises(ValueError):
         p.missions(start_goal=sg[sub], normals=torch.zeros((len(sub), 10), dtype=torch.float64, device="cuda:0"), K=300)
     n_seg = h["n_seg"][sub]
@@ -281,7 +270,7 @@ def test_missions_path_cap_and_caller_normals(map2_batch):
     hf = p.missions(start_goal=sg[sub], normals=z.reshape(-1), normal_range=rng, K=300).host()
     assert np.array_equal(hf["path_len"], hr["path_len"]) and np.array_equal(hf["status"], hr["status"])
     for i, n in enumerate(np.minimum(hr["path_len"], hr["path"].shape[1])):
-        assert bits_equal(hf["path"][i, :n], hr["path"][i, :n])
+        assert bits_equal_nan(hf["path"][i, :n], hr["path"][i, :n])
 
 
 @pytest.mark.gpu

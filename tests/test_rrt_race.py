@@ -4,18 +4,17 @@ A member of a race group runs no iteration it once a member of its group has fou
 winner of a group is the lowest query index among the members with the fewest iterations to the goal: the argmin of
 full oracle runs of every member, whatever the lanes and schedule.  A member that is cut is PAUSED and holds what the
 oracle plans with K = iters + 1; every other member, and every group without a winner, equals the plain call.  The CPU
-tests check the ABI mirror of the header, the host-side rejections and the key helpers."""
+tests check the host-side rejections and the key helpers (the ABI mirror of the header is checked in test_abi.py)."""
 import ctypes as C
 import os
-import re
 from concurrent.futures import ThreadPoolExecutor
 
 import numpy as np
 import pytest
 
 from tests import util
+from tests.util import O, bits_equal, planner_for  # noqa: F401  (O is a fixture)
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 OK_FOUND, OK_NOT_FOUND, PAUSED, NOT_RUN = 0, 1, 8, 255
 COUNTERS_KEPT = [0, 1, 2, 3, 4, 5, 6, 8]  # every counter but 7 (hash probes of a rebuilt index)
 RESUME_CASES = [(32, 0), (16, 0), (8, 0), (1, 0), (8, 1), (32, 1)]
@@ -36,27 +35,6 @@ def expected_winners(status, iters, groups, n_groups):
 
 
 # ------------------------------------------------------------------ CPU
-def struct_members(name):
-    src = open(os.path.join(ROOT, "include", "thetarrt.h")).read()
-    src = re.sub(r"/\*.*?\*/", "", src, flags=re.S)
-    body = re.search(r"typedef struct %s \{(.*?)\} %s;" % (name, name), src, flags=re.S).group(1)
-    names = []
-    for decl in body.split(";"):
-        decl = decl.strip()
-        if decl:
-            head, *rest = decl.split(",")
-            names.append(re.findall(r"\w+", head)[-1])
-            names += [r.strip().lstrip("*").strip() for r in rest]
-    return names
-
-
-def test_crrtrace_mirrors_header():
-    from theta_rrt_b200 import _lib
-    assert [f[0] for f in _lib.CRrtRace._fields_] == struct_members("trrt_rrt_race")
-    assert C.sizeof(_lib.CRrtRace) == 24
-    assert "trrt_rrt_race_batch" in _lib.SIGNATURES
-
-
 def test_host_rejections():
     """Rejected before any device work (these calls need no device)."""
     from theta_rrt_b200 import _lib
@@ -101,34 +79,13 @@ def test_expected_winners_table():
 
 
 # ------------------------------------------------------------------ GPU
-@pytest.fixture(scope="module")
-def O():
-    from oracle import c_oracle
-    c_oracle.lib()
-    return c_oracle
-
-
-def planner_for(free, **params):
-    from theta_rrt_b200 import OccupancyGrid, Params, Planner
-    return Planner(OccupancyGrid(free), Params(**params))
-
-
-def bits_equal(a, b):
-    a = np.ascontiguousarray(a, np.float64)
-    b = np.ascontiguousarray(b, np.float64)
-    return a.shape == b.shape and np.array_equal(a.view(np.int64), b.view(np.int64))
-
-
 def race_inputs(free, n_prob, S, K, seed):
     """n_prob problems x S seeds: member q = p * S + s plans problem p with the stream of seed seeds[p, s]."""
     from theta_rrt_b200 import samples
     starts, goals = util.random_queries(free, n_prob, seed)
     seeds = (np.arange(n_prob * S).reshape(n_prob, S) * 7 + seed).astype(np.int64)
     ms, mg = np.repeat(starts, S, axis=0), np.repeat(goals, S, axis=0)
-    nq = n_prob * S
-    sxy = np.empty((nq, K - 1, 2), np.int32); sth = np.empty((nq, K - 1))
-    for q in range(nq):
-        sxy[q], sth[q] = samples.make_stream(((mg[q, 0], mg[q, 1]), mg[q, 2]), K - 1, int(seeds.flat[q]), free.shape)
+    sxy, sth = samples.make_streams(mg, K - 1, seeds.reshape(-1), free.shape)
     return dict(problems=(starts, goals), seeds=seeds, inp=(ms, mg, sxy, sth), groups=np.repeat(np.arange(n_prob), S),
                 K=K, free=free)
 

@@ -2,8 +2,8 @@
 
 A pause is a window boundary the caller chooses, so every sequence of pauses and resumes, under any lanes and schedule,
 must return what one uninterrupted call returns, bit for bit; a query paused at stop_at[q] = k must hold what the
-oracle plans with K = k + 1.  The CPU tests check the ABI mirror of the header."""
-import ctypes as C
+oracle plans with K = k + 1.  The CPU test checks the PAUSED status of the header; the ABI mirror is checked in
+test_abi.py."""
 import os
 import re
 
@@ -11,68 +11,41 @@ import numpy as np
 import pytest
 
 from tests import util
+from tests.util import O, bits_equal, planner_for  # noqa: F401  (O is a fixture)
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PAUSED, OK_FOUND, OK_NOT_FOUND, NOT_RUN = 8, 0, 1, 255
 # counter 7 (hash probes) counts probes in the index a resume rebuilds: the one counter that depends on the pauses
 COUNTERS_KEPT = [0, 1, 2, 3, 4, 5, 6, 8]
 
 
-# ------------------------------------------------------------------ CPU: the ABI mirror
-def rrt_args_members():
-    src = open(os.path.join(ROOT, "include", "thetarrt.h")).read()
-    src = re.sub(r"/\*.*?\*/", "", src, flags=re.S)
-    body = re.search(r"typedef struct trrt_rrt_args \{(.*?)\} trrt_rrt_args;", src, flags=re.S).group(1)
-    names = []
-    for decl in body.split(";"):
-        decl = decl.strip()
-        if not decl:
-            continue
-        head, *rest = decl.split(",")
-        names.append(re.findall(r"\w+", head)[-1])
-        names += [r.strip().lstrip("*").strip() for r in rest]
-    return names
-
-
-def test_crrtargs_mirrors_header():
-    from theta_rrt_b200 import _lib
-    assert [f[0] for f in _lib.CRrtArgs._fields_] == rrt_args_members()
-    assert C.sizeof(_lib.CRrtArgs) % 8 == 0
-    assert _lib.CRrtArgs._fields_[-2:] == [("d_stop_at", C.c_void_p), ("resume", C.c_int32)]
-
-
+# ------------------------------------------------------------------ CPU
 def test_paused_status_in_header_and_names():
     from theta_rrt_b200 import planner
-    src = open(os.path.join(ROOT, "include", "thetarrt.h")).read()
+    src = open(os.path.join(util.ROOT, "include", "thetarrt.h")).read()
     assert re.search(r"\bTRRT_PAUSED\s*=\s*8\b", src)
     assert planner.PAUSED == PAUSED and planner.STATUS_NAMES[PAUSED] == "PAUSED"
 
 
+def test_result_buffers_and_launch_state():
+    """host() returns the outputs, not the launch state that rrt_resume plans with; fits() decides which buffers rrt_host
+    may reuse."""
+    import dataclasses
+    from theta_rrt_b200.planner import RrtResult
+    res = RrtResult.empty(3, 5, "cpu", want_u=True, logs=True, counters=False)
+    assert res.u.shape == (3, 5, 5) and res.it_near.shape == (3, 4) and res.counters is None
+    res.launch = object()
+    assert set(res.host()) == {f.name for f in dataclasses.fields(RrtResult)} - {"launch"}
+    assert res.fits(3, 5, True, True, False)
+    for args in ((4, 5, True, True, False), (3, 6, True, True, False), (3, 5, False, True, False),
+                 (3, 5, True, False, False), (3, 5, True, True, True)):
+        assert not res.fits(*args), args
+
+
 # ------------------------------------------------------------------ GPU
-@pytest.fixture(scope="module")
-def O():
-    from oracle import c_oracle
-    c_oracle.lib()
-    return c_oracle
-
-
-def planner_for(free, **params):
-    from theta_rrt_b200 import OccupancyGrid, Params, Planner
-    return Planner(OccupancyGrid(free), Params(**params))
-
-
-def bits_equal(a, b):
-    a = np.ascontiguousarray(a, np.float64)
-    b = np.ascontiguousarray(b, np.float64)
-    return a.shape == b.shape and np.array_equal(a.view(np.int64), b.view(np.int64))
-
-
 def streams(free, nq, K, query_seed, stream_seed):
     from theta_rrt_b200 import samples
     starts, goals = util.random_queries(free, nq, query_seed)
-    sxy = np.empty((nq, K - 1, 2), np.int32); sth = np.empty((nq, K - 1))
-    for q in range(nq):
-        sxy[q], sth[q] = samples.make_stream(((goals[q, 0], goals[q, 1]), goals[q, 2]), K - 1, stream_seed + q, free.shape)
+    sxy, sth = samples.make_streams(goals, K - 1, np.arange(nq) + stream_seed, free.shape)
     return starts, goals, sxy, sth
 
 

@@ -12,6 +12,7 @@ import numpy as np
 import pytest
 
 from tests import util
+from tests.util import O, bits_equal  # noqa: F401  (O is a fixture)
 
 SRC = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "theta_rrt_b200", "csrc", "trrt_rrt.cuh")
 
@@ -249,26 +250,10 @@ def test_procedure_ties_duplicates_and_overflow():
 
 
 # ------------------------------------------------------------------ GPU, bit for bit against the C oracle
-@pytest.fixture(scope="module")
-def O():
-    from oracle import c_oracle
-    c_oracle.lib()
-    return c_oracle
-
-
-def bits_equal(a, b):
-    a = np.ascontiguousarray(a, np.float64)
-    b = np.ascontiguousarray(b, np.float64)
-    return a.shape == b.shape and np.array_equal(a.view(np.int64), b.view(np.int64))
-
-
 def streams(free, nq, K, seed):
     from theta_rrt_b200 import samples
     starts, goals = util.random_queries(free, nq, seed)
-    sxy = np.empty((nq, K - 1, 2), np.int32)
-    sth = np.empty((nq, K - 1))
-    for q in range(nq):
-        sxy[q], sth[q] = samples.make_stream(((goals[q, 0], goals[q, 1]), goals[q, 2]), K - 1, q, free.shape)
+    sxy, sth = samples.make_streams(goals, K - 1, np.arange(nq), free.shape)
     return starts, goals, sxy, sth
 
 

@@ -1,10 +1,61 @@
 """Shared helpers for the parity tests."""
 import json
 import os
+import re
 
 import numpy as np
+import pytest
 
-GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+GOLDEN = os.path.join(ROOT, "tests", "golden")
+
+
+@pytest.fixture(scope="module")
+def O():
+    """The C oracle, built and loaded (a module imports this fixture by name)."""
+    from oracle import c_oracle
+    c_oracle.lib()
+    return c_oracle
+
+
+def planner_for(free=None, device=None, **params):
+    """A Planner over `free` (default: an open 64 x 64 map) on `device` (default: OccupancyGrid's, cuda:0) with
+    Params(**params)."""
+    from theta_rrt_b200 import OccupancyGrid, Params, Planner
+    if free is None:
+        free = np.ones((64, 64), bool)
+    grid = OccupancyGrid(free) if device is None else OccupancyGrid(free, device=device)
+    return Planner(grid, Params(**params))
+
+
+def bits_equal(a, b):
+    """float64 arrays equal bit for bit (NaN payloads included)."""
+    a = np.ascontiguousarray(a, np.float64)
+    b = np.ascontiguousarray(b, np.float64)
+    return a.shape == b.shape and np.array_equal(a.view(np.int64), b.view(np.int64))
+
+
+def bits_equal_nan(a, b):
+    """float64 arrays equal bit for bit, where any NaN equals any NaN."""
+    a, b = np.asarray(a, np.float64), np.asarray(b, np.float64)
+    if a.shape != b.shape or not np.array_equal(np.isnan(a), np.isnan(b)):
+        return False
+    return np.array_equal(np.where(np.isnan(a), 0.0, a).view(np.int64), np.where(np.isnan(b), 0.0, b).view(np.int64))
+
+
+def struct_members(name):
+    """Member names of `typedef struct name {...} name;` in include/thetarrt.h, in declaration order."""
+    src = open(os.path.join(ROOT, "include", "thetarrt.h")).read()
+    src = re.sub(r"/\*.*?\*/", "", src, flags=re.S)
+    body = re.search(r"typedef struct %s \{(.*?)\} %s;" % (name, name), src, flags=re.S).group(1)
+    names = []
+    for decl in body.split(";"):
+        decl = decl.strip()
+        if decl:
+            head, *rest = decl.split(",")
+            names.append(re.findall(r"\w+", head)[-1])
+            names += [r.strip().lstrip("*").strip() for r in rest]
+    return names
 
 
 def synthetic_map(n, p, block, seed):

@@ -9,6 +9,7 @@ There is no CPU fallback.
 from __future__ import annotations
 
 import ctypes as C
+import dataclasses
 import operator
 from dataclasses import dataclass, field
 
@@ -32,11 +33,44 @@ COUNTER_NAMES = ("nodes_scanned", "los_calls", "los_pixels", "arc_candidate_pixe
                  "steer_calls", "drive_calls", "hash_probes", "nearest_sqrt_ties")
 
 
+# metadata of the result fields that host() leaves out: device state kept for the stream or for a later call, not outputs
+_PRIVATE = {"private": True}
+# tree field of RrtResult -> its packed copy (rrt(..., pack=True))
+_PACKED = {"node_x": "pack_x", "node_y": "pack_y", "node_theta": "pack_theta", "parent": "pack_parent", "u": "pack_u"}
+
+
 def _host_dict(obj):
     out = {}
-    for k, v in obj.__dict__.items():
-        out[k] = v.detach().cpu().numpy() if isinstance(v, torch.Tensor) else v
+    for f in dataclasses.fields(obj):
+        if not f.metadata.get("private"):
+            v = getattr(obj, f.name)
+            out[f.name] = v.detach().cpu().numpy() if isinstance(v, torch.Tensor) else v
     return out
+
+
+def _ptr(t):
+    return t.data_ptr() if t is not None else None
+
+
+def _host_array(x, dtype=None):
+    """numpy copy of a tensor (on any device), or np.asarray of a sequence."""
+    return np.asarray(x.cpu() if isinstance(x, torch.Tensor) else x, dtype)
+
+
+@dataclass
+class _RrtLaunch:
+    """What an RRT launch reads besides its result's arrays: the inputs stay alive until the stream has consumed them,
+    and rrt_resume plans with them again."""
+    starts: torch.Tensor
+    goals: torch.Tensor
+    sample_xy: torch.Tensor
+    sample_th: torch.Tensor
+    map_id: torch.Tensor | None
+    params: Params
+    grid: OccupancyGrid
+    packed: bool  # the kernel writes the result's pack_* arrays
+    race: tuple[torch.Tensor, int] | None  # (group ids int32 [nq] on the device, n_groups)
+    stop: torch.Tensor | None = None  # stop_at of the latest launch
 
 
 @dataclass
@@ -71,6 +105,32 @@ class RrtResult:
     race_key: torch.Tensor | None = None
     race_winner: torch.Tensor | None = None
     race_iters: torch.Tensor | None = None
+    launch: _RrtLaunch | None = field(default=None, repr=False, metadata=_PRIVATE)
+
+    @classmethod
+    def empty(cls, nq, K, device, want_u, logs, counters):
+        """Output buffers of an rrt call over nq queries of capacity K, with the optional outputs it asks for."""
+        f64 = dict(dtype=torch.float64, device=device)
+        i32 = dict(dtype=torch.int32, device=device)
+        res = cls(K=K, node_x=torch.empty((nq, K), **f64), node_y=torch.empty((nq, K), **f64),
+                  node_theta=torch.empty((nq, K), **f64), parent=torch.empty((nq, K), **i32), n_nodes=torch.empty(nq, **i32),
+                  sol=torch.empty(nq, **i32), status=torch.empty(nq, **i32), iters=torch.empty(nq, **i32))
+        if want_u:
+            res.u = torch.empty((nq, K, 5), **f64)
+        if logs:
+            res.it_near = torch.empty((nq, K - 1), **i32)
+            res.it_new = torch.empty((nq, K - 1), **i32)
+            res.it_code = torch.empty((nq, K - 1), dtype=torch.uint8, device=device)
+            res.los_log = torch.zeros((nq, 2 * (K - 1)), dtype=torch.uint8, device=device)
+            res.n_los = torch.empty(nq, **i32)
+        if counters:
+            res.counters = torch.zeros((nq, 9), dtype=torch.int64, device=device)
+        return res
+
+    def fits(self, nq, K, want_u, logs, counters):
+        """True when empty(nq, K, ..., want_u, logs, counters) would have the shapes and optional outputs of this result."""
+        return self.K == K and self.node_x.shape[0] == nq and (self.u is not None) == bool(want_u) \
+            and (self.it_near is not None) == bool(logs) and (self.counters is not None) == bool(counters)
 
     def host(self):
         return _host_dict(self)
@@ -114,6 +174,7 @@ class ThetaResult:
     n_los: torch.Tensor | None = None
     pushes: torch.Tensor | None = None
     extra: dict = field(default_factory=dict)
+    keep: tuple = field(default=(), repr=False, metadata=_PRIVATE)  # inputs alive until the stream has consumed them
 
     def host(self):
         return _host_dict(self)
@@ -127,7 +188,8 @@ class MissionResult:
     status (0 = the chain ran to its end; 4 / 7 = it stopped where the reference raises; otherwise the route search's
     status), stop_seg (-1 when the chain ran to its end), n_seg, waypoints (int32 [B, wp_cap, 2], n_waypoints of them
     valid), path (float64 [B, path_cap, 8] = x, y, theta, u[5] of main.path_nodes, segment after segment), path_seg
-    (segment of each row) and path_len (full length, also when it exceeds path_cap; rows past it are not written)."""
+    (segment of each row) and path_len (full length, also when it exceeds path_cap; rows past it are not written).
+    schedule: the dispatch order (mission_schedule) as (order, n_active) host arrays."""
     K: int
     begin: torch.Tensor
     end: torch.Tensor
@@ -147,6 +209,8 @@ class MissionResult:
     path_seg: torch.Tensor
     path_len: torch.Tensor
     route: ThetaResult | None = None
+    schedule: tuple | None = None
+    keep: tuple = field(default=(), repr=False, metadata=_PRIVATE)  # inputs alive until the stream has consumed them
 
     def host(self):
         out = _host_dict(self)
@@ -156,6 +220,20 @@ class MissionResult:
 
 
 SEED_STREAMS = ("host", "device")
+
+
+def _check_seed_stream(seed_stream):
+    """Raises ValueError unless seed_stream names one of SEED_STREAMS."""
+    if seed_stream not in SEED_STREAMS:
+        raise ValueError(f"seed_stream must be one of {SEED_STREAMS}")
+
+
+def _ranges(counts):
+    """[begin, end) int64 [n, 2] of consecutive pieces of the given lengths."""
+    rng = np.zeros((len(counts), 2), np.int64)
+    rng[:, 1] = np.cumsum(counts)
+    rng[1:, 0] = rng[:-1, 1]
+    return rng
 
 
 def legacy_seeds(seeds):
@@ -196,6 +274,15 @@ class Planner:
         self.device = grid.device
         self.params = params or Params()
         self._work = {}
+        self._pin = {}
+        # rrt_host's pipeline: per piece a planning stream and a copy stream, and device buffers by piece shape; the
+        # events host_sync waits for; the valid_rows_only pieces whose row copies are still to be issued; the last call's
+        # tensors, referenced until the next call
+        self._streams, self._copy_streams = [], []
+        self._host_cache = {}
+        self._pending = []
+        self._deferred = []
+        self._inflight = []
 
     # ------------------------------------------------------------------ helpers
     def _stream(self):
@@ -251,12 +338,10 @@ class Planner:
                 out = torch.empty(n, dtype=torch.uint8, device=self.device)
             g = self.grid
             if layout == "tiles":
-                _lib.check(self.lib.trrt_los_batch_tiled(g.tiles.data_ptr(), g.n_maps, g.H, g.W,
-                                                         mid.data_ptr() if mid is not None else None, seg.data_ptr(),
+                _lib.check(self.lib.trrt_los_batch_tiled(g.tiles.data_ptr(), g.n_maps, g.H, g.W, _ptr(mid), seg.data_ptr(),
                                                          n, out.data_ptr(), self._stream()), "trrt_los_batch_tiled")
             else:
-                _lib.check(self.lib.trrt_los_batch(g.bits.data_ptr(), g.n_maps, g.H, g.W,
-                                                   mid.data_ptr() if mid is not None else None, seg.data_ptr(), n,
+                _lib.check(self.lib.trrt_los_batch(g.bits.data_ptr(), g.n_maps, g.H, g.W, _ptr(mid), seg.data_ptr(), n,
                                                    out.data_ptr(), self._stream()), "trrt_los_batch")
         return out
 
@@ -273,14 +358,13 @@ class Planner:
             wb = self.lib.trrt_nearest_workspace_bytes(n, nq)
             work = self._scratch("nearest", wb)
             _lib.check(self.lib.trrt_nearest_batch(x.data_ptr(), y.data_ptr(), n, qxy.data_ptr(), nq, idx.data_ptr(),
-                                                   d2.data_ptr() if want_d2 else None, work.data_ptr(), work.numel(),
+                                                   _ptr(d2), work.data_ptr(), work.numel(),
                                                    self._stream()), "trrt_nearest_batch")
         return (idx, d2) if want_d2 else idx
 
     # ------------------------------------------------------------------ K2
     def rrt(self, starts, goals, sample_xy, sample_th, K=None, params=None, map_id=None, logs=False, want_u=True,
-            counters=False, lanes=0, schedule=0, work_key="rrt", reuse=None, pack=False, packed=None, stop_at=None,
-            race=None, race_groups=None):
+            counters=False, lanes=0, schedule=0, pack=False, packed=None, stop_at=None, race=None, race_groups=None):
         """rrt.rrt for a batch.  starts/goals float64 [q,3] (x, y, theta_deg); sample_xy int32 [q,K-1,2];
         sample_th float64 [q,K-1].  K = builtins.K (node capacity; K-1 iterations).
         pack=True: the kernel also leaves a packed copy of the tree rows that exist (pack_x, pack_y, pack_theta,
@@ -294,6 +378,15 @@ class Planner:
         max + 1 groups; a CUDA int32 tensor is used in place and needs race_groups (ids outside [0, race_groups) race
         nobody).  The result's race_key / race_winner / race_iters hold each group's winner: the lowest query index
         among the members with the fewest iterations to the goal."""
+        return self._rrt(starts, goals, sample_xy, sample_th, K=K, params=params, map_id=map_id, logs=logs, want_u=want_u,
+                         counters=counters, lanes=lanes, schedule=schedule, pack=pack, packed=packed, stop_at=stop_at,
+                         race=race, race_groups=race_groups)
+
+    def _rrt(self, starts, goals, sample_xy, sample_th, K=None, params=None, map_id=None, logs=False, want_u=True,
+             counters=False, lanes=0, schedule=0, pack=False, packed=None, stop_at=None, race=None, race_groups=None,
+             work_key="rrt", reuse=None):
+        """rrt, with the workspace of `work_key` and the output buffers of `reuse` when they fit (rrt_host keeps one
+        workspace and one result per piece: concurrent launches must not share a workspace)."""
         P = params or self.params
         if pack and stop_at is not None:
             raise ValueError("pack=True plans whole runs: it cannot be combined with stop_at")
@@ -316,49 +409,34 @@ class Planner:
             mid = self._map_ids(map_id, nq)
             stop = self._stop_at(stop_at, nq, K)
             groups = self._race_groups(race, race_groups, nq)
-            dev = self.device
-            f64 = dict(dtype=torch.float64, device=dev)
-            i32 = dict(dtype=torch.int32, device=dev)
-            if reuse is not None and reuse.K == K and reuse.node_x.shape[0] == nq and (reuse.u is not None) == bool(want_u) \
-                    and (reuse.it_near is not None) == bool(logs) and (reuse.counters is not None) == bool(counters):
-                res = reuse  # caller-provided result buffers of the right shape (rrt_host keeps one set per stream)
+            if reuse is not None and reuse.fits(nq, K, want_u, logs, counters):
+                res = reuse
                 if counters:
                     res.counters.zero_()
             else:
-                res = RrtResult(K=K, node_x=torch.empty((nq, K), **f64), node_y=torch.empty((nq, K), **f64),
-                                node_theta=torch.empty((nq, K), **f64), parent=torch.empty((nq, K), **i32),
-                                n_nodes=torch.empty(nq, **i32), sol=torch.empty(nq, **i32), status=torch.empty(nq, **i32),
-                                iters=torch.empty(nq, **i32))
-                if want_u:
-                    res.u = torch.empty((nq, K, 5), **f64)
-                if logs:
-                    res.it_near = torch.empty((nq, K - 1), **i32)
-                    res.it_new = torch.empty((nq, K - 1), **i32)
-                    res.it_code = torch.empty((nq, K - 1), dtype=torch.uint8, device=dev)
-                    res.los_log = torch.zeros((nq, 2 * (K - 1)), dtype=torch.uint8, device=dev)
-                    res.n_los = torch.empty(nq, **i32)
-                if counters:
-                    res.counters = torch.zeros((nq, 9), dtype=torch.int64, device=dev)
+                res = RrtResult.empty(nq, K, self.device, want_u, logs, counters)
             if pack:
                 if packed is None:
-                    packed = {"pack_x": torch.empty(nq * K, **f64), "pack_y": torch.empty(nq * K, **f64),
-                              "pack_theta": torch.empty(nq * K, **f64), "pack_parent": torch.empty(nq * K, **i32),
-                              "row_start": torch.empty(nq, dtype=torch.int64, device=dev),
-                              "pack_total": torch.empty(1, dtype=torch.int64, device=dev)}
-                    if want_u:
-                        packed["pack_u"] = torch.empty((nq * K, 5), **f64)
+                    packed = self._packed_rows(nq, K, want_u)
                     packed["pack_total"].zero_()
                 for k, v in packed.items():  # a reused set: the caller has set pack_total to the first row to use
                     setattr(res, k, v)
-            # the inputs stay alive until the stream has consumed them, and rrt_resume plans with them again
-            res._keep = (starts, goals, sample_xy, sample_th, mid, P, self.grid)
-            res._packed = bool(pack)
-            res._race = None
+            res.launch = _RrtLaunch(starts, goals, sample_xy, sample_th, mid, P, self.grid, packed=bool(pack), race=groups)
             if groups is not None:
-                res._race = groups
-                res.race_key = torch.empty(groups[1], dtype=torch.int64, device=dev)
+                res.race_key = torch.empty(groups[1], dtype=torch.int64, device=self.device)
             self._rrt_launch(res, stop, lanes, schedule, resume=False, work_key=work_key)
         return res
+
+    def _packed_rows(self, nq, K, want_u, pieces=1):
+        """Device arrays for the packed tree rows of nq queries of capacity K (trrt_rrt_args d_pack_*): the pack_* arrays
+        of _PACKED (pack_u when want_u), row_start int64 [nq] and pack_total, one int64 row counter per piece."""
+        dev = self.device
+        d = {p: torch.empty((nq * K, 5) if t == "u" else nq * K, dtype=torch.int32 if t == "parent" else torch.float64,
+                            device=dev)
+             for t, p in _PACKED.items() if t != "u" or want_u}
+        d["row_start"] = torch.empty(nq, dtype=torch.int64, device=dev)
+        d["pack_total"] = torch.empty(pieces, dtype=torch.int64, device=dev)
+        return d
 
     def rrt_resume(self, res: RrtResult, stop_at=None, lanes=0, schedule=0, race=True) -> RrtResult:
         """Continue the PAUSED queries of `res` (a result of rrt(..., stop_at=...)) in place, with the inputs, params and
@@ -368,10 +446,9 @@ class Planner:
         bit, except counter 7 (hash probes, which count probes in the query's rebuilt index).  A result planned with a race
         keeps racing (paused members continue up to their group's best iters, and may be cut again) unless race=False,
         which continues them as plain queries and leaves race_key as it is.  Returns res."""
-        keep = getattr(res, "_keep", None)
-        if keep is None or len(keep) != 7 or keep[6] is not self.grid:
+        if res.launch is None or res.launch.grid is not self.grid:
             raise ValueError("rrt_resume continues a result that Planner.rrt planned on this planner's grid")
-        if res._packed:
+        if res.launch.packed:
             raise ValueError("a result planned with pack=True cannot be resumed")
         with torch.cuda.device(self.device):
             stop = self._stop_at(stop_at, res.node_x.shape[0], res.K)
@@ -390,7 +467,7 @@ class Planner:
             t = self._dev(race, torch.int32).reshape(-1)
             n = int(race_groups)
         else:
-            a = np.asarray(race.cpu() if isinstance(race, torch.Tensor) else race).reshape(-1)
+            a = _host_array(race).reshape(-1)
             if a.dtype.kind not in "iu":
                 raise ValueError(f"race group ids must be integers, got {a.dtype}")
             if a.size and int(a.min()) < 0:
@@ -412,7 +489,7 @@ class Planner:
         if isinstance(stop_at, torch.Tensor) and stop_at.is_cuda:
             t = self._dev(stop_at, torch.int32).reshape(-1)  # left on the device: the kernel clamps it to [0, K-1]
         else:
-            a = np.asarray(stop_at.cpu() if isinstance(stop_at, torch.Tensor) else stop_at)
+            a = _host_array(stop_at)
             if a.dtype.kind not in "iu":
                 raise ValueError(f"stop_at must be integers, got {a.dtype}")
             if a.ndim == 0:
@@ -426,32 +503,31 @@ class Planner:
         return t
 
     def _rrt_launch(self, res, stop, lanes, schedule, resume, work_key="rrt", race=True):
-        """One trrt_rrt_race_batch call over the inputs kept in res._keep, writing res's arrays; the race of res, if any,
+        """One trrt_rrt_race_batch call over the inputs kept in res.launch, writing res's arrays; the race of res, if any,
         takes part unless race=False."""
-        starts, goals, sample_xy, sample_th, mid, P, g = res._keep
+        L, g = res.launch, res.launch.grid
         nq, K = res.node_x.shape[0], res.K
-        pack = res._packed
         wb = self.lib.trrt_rrt_workspace_bytes(nq, K)
-        work = self._scratch(work_key, wb)  # concurrent launches (rrt_host) must not share a workspace
-        ptr = lambda t: t.data_ptr() if t is not None else None  # noqa: E731
-        a = _lib.CRrtArgs(d_bits=g.bits.data_ptr(), n_maps=g.n_maps, H=g.H, W=g.W, d_map_id=ptr(mid),
-                          params=P.to_c(), n_queries=nq, K=K, lanes_per_query=int(lanes), schedule=int(schedule),
-                          sample_xy_i16=int(sample_xy.dtype == torch.int16),
-                          d_start=starts.data_ptr(), d_goal=goals.data_ptr(), d_sample_xy=sample_xy.data_ptr(),
-                          d_sample_th=sample_th.data_ptr(), d_node_x=res.node_x.data_ptr(),
+        work = self._scratch(work_key, wb)
+        # a result reused by a call without packing must not hand its earlier pack arrays to the kernel
+        pk = {n: _ptr(getattr(res, n)) if L.packed else None for n in ("pack_total", "row_start", *_PACKED.values())}
+        if res.u is None:
+            pk["pack_u"] = None
+        a = _lib.CRrtArgs(d_bits=g.bits.data_ptr(), n_maps=g.n_maps, H=g.H, W=g.W, d_map_id=_ptr(L.map_id),
+                          params=L.params.to_c(), n_queries=nq, K=K, lanes_per_query=int(lanes), schedule=int(schedule),
+                          sample_xy_i16=int(L.sample_xy.dtype == torch.int16),
+                          d_start=L.starts.data_ptr(), d_goal=L.goals.data_ptr(), d_sample_xy=L.sample_xy.data_ptr(),
+                          d_sample_th=L.sample_th.data_ptr(), d_node_x=res.node_x.data_ptr(),
                           d_node_y=res.node_y.data_ptr(), d_node_th=res.node_theta.data_ptr(),
-                          d_parent=res.parent.data_ptr(), d_u=ptr(res.u), d_n_nodes=res.n_nodes.data_ptr(),
+                          d_parent=res.parent.data_ptr(), d_u=_ptr(res.u), d_n_nodes=res.n_nodes.data_ptr(),
                           d_sol=res.sol.data_ptr(), d_status=res.status.data_ptr(), d_iters=res.iters.data_ptr(),
-                          d_it_near=ptr(res.it_near), d_it_new=ptr(res.it_new), d_it_code=ptr(res.it_code),
-                          d_los_log=ptr(res.los_log), d_n_los=ptr(res.n_los), d_counters=ptr(res.counters),
+                          d_it_near=_ptr(res.it_near), d_it_new=_ptr(res.it_new), d_it_code=_ptr(res.it_code),
+                          d_los_log=_ptr(res.los_log), d_n_los=_ptr(res.n_los), d_counters=_ptr(res.counters),
                           d_work=work.data_ptr(), work_bytes=work.numel(),
-                          d_pack_rows=ptr(res.pack_total) if pack else None, d_row_start=ptr(res.row_start) if pack else None,
-                          d_pack_x=ptr(res.pack_x) if pack else None, d_pack_y=ptr(res.pack_y) if pack else None,
-                          d_pack_th=ptr(res.pack_theta) if pack else None,
-                          d_pack_parent=ptr(res.pack_parent) if pack else None,
-                          d_pack_u=ptr(res.pack_u) if (pack and res.u is not None) else None,
-                          d_stop_at=ptr(stop), resume=int(resume))
-        groups = getattr(res, "_race", None) if race else None
+                          d_pack_rows=pk["pack_total"], d_row_start=pk["row_start"], d_pack_x=pk["pack_x"],
+                          d_pack_y=pk["pack_y"], d_pack_th=pk["pack_theta"], d_pack_parent=pk["pack_parent"],
+                          d_pack_u=pk["pack_u"], d_stop_at=_ptr(stop), resume=int(resume))
+        groups = L.race if race else None
         rc = None
         if groups is not None:
             rc = _lib.CRrtRace(d_group=groups[0].data_ptr(), n_groups=groups[1], d_key=res.race_key.data_ptr())
@@ -460,10 +536,7 @@ class Planner:
         if groups is not None:
             res.race_winner, res.race_iters = race_decode(res.race_key)
         res.lanes = int(lanes)
-        res._stop = stop  # alive until the stream has consumed it
-
-    _TREE = ("node_x", "node_y", "node_theta", "parent", "u")
-    _PACKED = {"node_x": "pack_x", "node_y": "pack_y", "node_theta": "pack_theta", "parent": "pack_parent", "u": "pack_u"}
+        L.stop = stop
 
     def rrt_host(self, starts, goals, sample_xy, sample_th, out, K=None, chunks=4, wait=True, valid_rows_only=False, **kw):
         """rrt.rrt for a batch whose inputs and outputs live in (pinned) HOST memory: the queries are cut into
@@ -496,17 +569,15 @@ class Planner:
         if defer:
             if "n_nodes" not in out or "row_start" not in out:
                 raise ValueError("valid_rows_only needs 'n_nodes' and 'row_start' among the outputs")
-            for k in self._TREE:
+            for k in _PACKED:
                 if k in out and not (out[k].is_pinned() and out[k].is_contiguous()):
                     raise ValueError(f"valid_rows_only needs a contiguous pinned host tensor for '{k}'")
         with torch.cuda.device(self.device):
             main = torch.cuda.current_stream(self.device)
-            if not hasattr(self, "_streams") or len(self._streams) < chunks:
+            if len(self._streams) < chunks:
                 self.host_sync()  # nothing may be in flight on streams that are about to be replaced
                 self._streams = [torch.cuda.Stream(self.device) for _ in range(chunks)]
                 self._copy_streams = [torch.cuda.Stream(self.device) for _ in range(chunks)]
-            if not hasattr(self, "_host_cache"):
-                self._host_cache = {}
             Kc = int(K) if K is not None else ins[3].numel() // nq + 1
             pk = None
             if defer:
@@ -518,19 +589,12 @@ class Planner:
                 pkey = ("packed", nq, Kc, chunks, want_u)
                 pc = self._host_cache.get(pkey)
                 if pc is None:
-                    def new_set():
-                        d = {"pack_x": torch.empty(nq * Kc, dtype=torch.float64, device=self.device),
-                             "pack_y": torch.empty(nq * Kc, dtype=torch.float64, device=self.device),
-                             "pack_theta": torch.empty(nq * Kc, dtype=torch.float64, device=self.device),
-                             "pack_parent": torch.empty(nq * Kc, dtype=torch.int32, device=self.device),
-                             "row_start": torch.empty(nq, dtype=torch.int64, device=self.device),
-                             "pack_total": torch.empty(chunks, dtype=torch.int64, device=self.device),
-                             "total_host": torch.zeros(chunks, dtype=torch.int64).pin_memory(), "free": [None] * chunks}
-                        if want_u:
-                            d["pack_u"] = torch.empty((nq * Kc, 5), dtype=torch.float64, device=self.device)
-                        return d
+                    sets = [self._packed_rows(nq, Kc, want_u, pieces=chunks) for _ in range(2)]
+                    for s in sets:
+                        s["total_host"] = torch.zeros(chunks, dtype=torch.int64).pin_memory()
+                        s["free"] = [None] * chunks
                     first = torch.tensor([nq * c // chunks * Kc for c in range(chunks)], dtype=torch.int64).pin_memory()
-                    pc = {"sets": [new_set(), new_set()], "turn": 0, "first": first}
+                    pc = {"sets": sets, "turn": 0, "first": first}
                     self._host_cache[pkey] = pc
                 pk = pc["sets"][pc["turn"]]
                 pc["turn"] = 1 - pc["turn"]
@@ -556,14 +620,15 @@ class Planner:
                         if pk["free"][c] is not None:
                             st.wait_event(pk["free"][c])  # the copies that still read this set's rows of the piece
                             pk["free"][c] = None
-                        packed = {k: pk[k] for k in ("pack_x", "pack_y", "pack_theta", "pack_parent", "pack_u") if k in pk}
+                        packed = {p: pk[p] for p in _PACKED.values() if p in pk}
                         packed["row_start"] = pk["row_start"][lo:hi]
                         packed["pack_total"] = pk["pack_total"][c:c + 1]
                         packed["pack_total"].copy_(pc["first"][c:c + 1], non_blocking=True)
-                    res = self.rrt(*din, K=K, work_key=("rrt", c), reuse=cached["res"], want_u=want_u, pack=defer, packed=packed, **kw)
+                    res = self._rrt(*din, K=K, want_u=want_u, pack=defer, packed=packed, work_key=("rrt", c),
+                                    reuse=cached["res"], **kw)
                     cached["res"] = res
                     for name, t in out.items():
-                        if defer and name in self._TREE:
+                        if defer and name in _PACKED:
                             continue
                         t[lo:hi].copy_(getattr(res, name), non_blocking=True)
                     if defer:
@@ -576,11 +641,11 @@ class Planner:
                 elif wait:
                     main.wait_event(done)
                 else:
-                    self._pending = [e for e in getattr(self, "_pending", []) if not e.query()] + [done]
-            self._inflight = keep  # tensors stay referenced until the next call
+                    self._track(done)
+            self._inflight = keep
             if defer:
                 # the previous batch first (its row counts are on the host by now), this one only if the caller waits
-                previous, self._deferred = getattr(self, "_deferred", []), deferred
+                previous, self._deferred = self._deferred, deferred
                 self._issue_tree_copies(previous)
                 if wait:
                     self._issue_tree_copies(self._deferred)
@@ -597,7 +662,7 @@ class Planner:
             cs = self._copy_streams[c]
             cs.wait_event(done)
             with torch.cuda.stream(cs):
-                for name, pname in self._PACKED.items():
+                for name, pname in _PACKED.items():
                     if name not in out or pname not in pk:
                         continue
                     m = 5 if name == "u" else 1
@@ -606,16 +671,20 @@ class Planner:
             copied = torch.cuda.Event()
             copied.record(cs)
             pk["free"][c] = copied
-            self._pending = [e for e in getattr(self, "_pending", []) if not e.query()] + [copied]
+            self._track(copied)
+
+    def _track(self, event):
+        """Keep `event` for host_sync, dropping the kept events that have completed."""
+        self._pending = [e for e in self._pending if not e.query()] + [event]
 
     def host_sync(self):
         """Make the planner's current stream wait for every piece enqueued by rrt_host(..., wait=False)."""
         with torch.cuda.device(self.device):
-            if getattr(self, "_deferred", None):
+            if self._deferred:
                 self._issue_tree_copies(self._deferred)
                 self._deferred = []
             main = torch.cuda.current_stream(self.device)
-            for e in getattr(self, "_pending", []):
+            for e in self._pending:
                 main.wait_event(e)
             self._pending = []
 
@@ -671,8 +740,7 @@ class Planner:
             mid = self._map_ids(map_id, n)
             out = torch.empty(n, dtype=torch.uint8, device=self.device)
             g = self.grid
-            _lib.check(self.lib.trrt_arc_batch(g.bits.data_ptr(), g.n_maps, g.H, g.W,
-                                               mid.data_ptr() if mid is not None else None, n, inp.data_ptr(),
+            _lib.check(self.lib.trrt_arc_batch(g.bits.data_ptr(), g.n_maps, g.H, g.W, _ptr(mid), n, inp.data_ptr(),
                                                out.data_ptr(), int(lanes), self._stream()), "trrt_arc_batch")
         return out
 
@@ -707,7 +775,7 @@ class Planner:
             out = torch.empty((n, 2), dtype=torch.uint8, device=self.device)
             g = self.grid
             cp = P.to_c()
-            _lib.check(self.lib.trrt_clearance_batch(g.bits.data_ptr(), g.n_maps, g.H, g.W, mid.data_ptr() if mid is not None else None,
+            _lib.check(self.lib.trrt_clearance_batch(g.bits.data_ptr(), g.n_maps, g.H, g.W, _ptr(mid),
                                                      C.byref(cp), n, inp.data_ptr(), out.data_ptr(), self._stream()),
                        "trrt_clearance_batch")
         return out
@@ -747,13 +815,12 @@ class Planner:
             if log_los:
                 los_cap = g.H * g.W
                 res.los_log = torch.zeros((nq, los_cap), dtype=torch.uint8, device=dev)
-            ptr = lambda t: t.data_ptr() if t is not None else None  # noqa: E731
-            a = _lib.CThetaArgs(d_bits=g.bits.data_ptr(), n_maps=g.n_maps, H=g.H, W=g.W, d_map_id=ptr(mid),
+            a = _lib.CThetaArgs(d_bits=g.bits.data_ptr(), n_maps=g.n_maps, H=g.H, W=g.W, d_map_id=_ptr(mid),
                                 thetastar=int(bool(thetastar)), lanes_per_query=int(lanes), n_queries=nq,
                                 d_start_goal=sg.data_ptr(), d_path=res.path.data_ptr(), path_cap=int(path_cap),
                                 d_path_len=res.path_len.data_ptr(), d_cost=res.cost.data_ptr(),
                                 d_expanded=res.expanded.data_ptr(), d_status=res.status.data_ptr(),
-                                d_los_log=ptr(res.los_log), los_cap=int(los_cap), d_n_los=res.n_los.data_ptr(),
+                                d_los_log=_ptr(res.los_log), los_cap=int(los_cap), d_n_los=res.n_los.data_ptr(),
                                 d_pushes=res.pushes.data_ptr(), n_slots=int(n_slots), heap_cap=int(heap_cap),
                                 d_work=None, work_bytes=0, d_order=None)
             order = None
@@ -778,7 +845,7 @@ class Planner:
             a.work_bytes = work.numel()
             _lib.check(self.lib.trrt_theta_batch(C.byref(a), self._stream()), "trrt_theta_batch")
             res.extra = dict(n_slots=int(a.n_slots), heap_cap=int(a.heap_cap), workspace_bytes=int(wb))
-            res._keep = (sg, mid, order)
+            res.keep = (sg, mid, order)
         return res
 
     # ------------------------------------------------------------------ seeded streams
@@ -797,9 +864,7 @@ class Planner:
             raise ValueError(f"{len(counts)} counts for {n} seeds")
         if n and counts.min() < 0:
             raise ValueError("counts must be >= 0")
-        rng = np.zeros((n, 2), np.int64)
-        rng[:, 1] = np.cumsum(counts)
-        rng[1:, 0] = rng[:-1, 1]
+        rng = _ranges(counts)
         total = int(rng[-1, 1]) if n else 0
         dev = self.device
         with torch.cuda.device(dev):
@@ -836,10 +901,10 @@ class Planner:
         """Two grow-only pinned float64 host buffers of at least n values per key and stream.  A call that reuses them has
         synchronised the stream first, so the copies of the previous call that read them have completed."""
         key = (key, torch.cuda.current_stream(self.device).cuda_stream)
-        cur = getattr(self, "_pin", {}).get(key)
+        cur = self._pin.get(key)
         if cur is None or cur[0].numel() < n:
             cur = tuple(torch.empty(max(int(n), 1024), dtype=torch.float64).pin_memory() for _ in range(2))
-            self.__dict__.setdefault("_pin", {})[key] = cur
+            self._pin[key] = cur
         return cur[0][:n], cur[1][:n]
 
     def rand_conf(self, goals, seeds, K=None, xy_dtype=torch.int32, params=None):
@@ -868,19 +933,26 @@ class Planner:
                                                      sth.data_ptr(), self._stream()), "trrt_rand_conf_batch")
         return sxy, sth
 
+    def _seeded_samples(self, goals, seeds, K, seed_stream, params):
+        """The K-1 rand_conf samples of np.random.seed(seeds[q]) around goals[q] float64 [q, 3], as rrt() takes them:
+        drawn on the device (rand_conf) for seed_stream="device", else by numpy (samples.make_streams, host arrays that
+        rrt() copies).  Each caller has checked seed_stream and seeds as its own contract says."""
+        if seed_stream == "device":
+            return self.rand_conf(goals, seeds, K, params=params)
+        return samples.make_streams(goals, K - 1, seeds, self.grid.shape, params.xystdv, params.anglestdv)
+
     def rrt_race(self, starts, goals, seeds, K=None, seed_stream="device", lanes=0, schedule=0, stop_at=None,
                  logs=False, params=None) -> RaceResult:
         """Seed races for P problems: problem p = (starts[p], goals[p]) float64 [P, 3] is planned once per seed of
         seeds[p] (integers [P, S], the stream of np.random.seed(seed) followed by rand_conf calls, drawn on the device or,
         with seed_stream="host", by numpy), and its S members race each other (rrt(..., race=...)): member s of problem p
         is query p * S + s of the result.  One call; returns per problem the winning query, its seed and its iters."""
-        if seed_stream not in SEED_STREAMS:
-            raise ValueError(f"seed_stream must be one of {SEED_STREAMS}")
+        _check_seed_stream(seed_stream)
         P = params or self.params
         K = int(K if K is not None else P.K)
-        starts = np.asarray(starts.cpu() if isinstance(starts, torch.Tensor) else starts, np.float64).reshape(-1, 3)
-        goals = np.asarray(goals.cpu() if isinstance(goals, torch.Tensor) else goals, np.float64).reshape(-1, 3)
-        seeds = np.asarray(seeds.cpu() if isinstance(seeds, torch.Tensor) else seeds)
+        starts = _host_array(starts, np.float64).reshape(-1, 3)
+        goals = _host_array(goals, np.float64).reshape(-1, 3)
+        seeds = _host_array(seeds)
         n_prob = starts.shape[0]
         if goals.shape[0] != n_prob or seeds.ndim != 2 or seeds.shape[0] != n_prob or seeds.shape[1] < 1:
             raise ValueError(f"rrt_race wants starts and goals [P, 3] and seeds [P, S], got {starts.shape}, {goals.shape}, "
@@ -888,14 +960,7 @@ class Planner:
         S = seeds.shape[1]
         flat = legacy_seeds(seeds)
         m_starts, m_goals = np.repeat(starts, S, axis=0), np.repeat(goals, S, axis=0)
-        if seed_stream == "device":
-            sxy, sth = self.rand_conf(m_goals, flat, K, params=P)
-        else:
-            sxy = np.empty((len(flat), K - 1, 2), np.int32)
-            sth = np.empty((len(flat), K - 1), np.float64)
-            for q, g in enumerate(m_goals):
-                sxy[q], sth[q] = samples.make_stream(((g[0], g[1]), g[2]), K - 1, int(flat[q]), self.grid.shape,
-                                                     P.xystdv, P.anglestdv)
+        sxy, sth = self._seeded_samples(m_goals, flat, K, seed_stream, P)
         res = self.rrt(m_starts, m_goals, sxy, sth, K=K, params=P, logs=logs, lanes=lanes, schedule=schedule,
                        stop_at=stop_at, race=np.repeat(np.arange(n_prob), S), race_groups=n_prob)
         seed_dev = torch.from_numpy(flat.astype(np.int64)).to(self.device)
@@ -928,8 +993,7 @@ class Planner:
             raise ValueError("K must be >= 2")
         if (seeds is None) == (normals is None):
             raise ValueError("pass exactly one of seeds and normals")
-        if seed_stream not in SEED_STREAMS:
-            raise ValueError(f"seed_stream must be one of {SEED_STREAMS}")
+        _check_seed_stream(seed_stream)
         g = self.grid
         with torch.cuda.device(self.device):
             route = None
@@ -956,46 +1020,7 @@ class Planner:
                 n_seg = np.maximum(n_wp_h - 1, 0)
             order, n_active = mission_schedule(n_seg)
             S = len(n_active)
-            need = 3 * (K - 1) * n_seg
-            if seeds is not None:
-                seeds = np.asarray(seeds).reshape(-1)
-                if len(seeds) != B:
-                    raise ValueError(f"{len(seeds)} seeds for {B} missions")
-                if seed_stream == "device":
-                    nz, rng_d = self.legacy_normals(seeds, need)
-                    if nz.numel() == 0:
-                        nz = torch.zeros(1, dtype=torch.float64, device=self.device)
-                else:
-                    rng = np.zeros((B, 2), np.int64)
-                    rng[:, 1] = np.cumsum(need)
-                    rng[1:, 0] = rng[:-1, 1]
-                    flat = np.empty(int(need.sum()), np.float64)
-                    for m in range(B):
-                        if need[m]:
-                            flat[rng[m, 0]:rng[m, 1]] = np.random.RandomState(int(seeds[m])).standard_normal(int(need[m]))
-                    nz = self._dev(flat, torch.float64) if flat.size else torch.zeros(1, dtype=torch.float64, device=self.device)
-            else:
-                nz = self._dev(normals, torch.float64)
-                if normal_range is None:
-                    if nz.dim() != 2 or nz.shape[0] != B:
-                        raise ValueError("normals without normal_range must be a [missions, L] array")
-                    L = nz.shape[1]
-                    rng = np.stack([np.arange(B) * L, np.arange(B) * L + L], axis=1).astype(np.int64)
-                else:
-                    rng = (normal_range.cpu().numpy() if isinstance(normal_range, torch.Tensor) else np.asarray(normal_range))
-                    rng = rng.astype(np.int64).reshape(B, 2)
-                nz = nz.reshape(-1)
-                if B and (rng.min() < 0 or rng[:, 1].max() > nz.numel() or (rng[:, 1] < rng[:, 0]).any()):
-                    raise ValueError("normal_range outside the normals")
-                short = np.nonzero(rng[:, 1] - rng[:, 0] < need)[0]
-                if len(short):
-                    m = int(short[0])
-                    raise ValueError(f"mission {m} has {int(rng[m, 1] - rng[m, 0])} normals, its {int(n_seg[m])} segments "
-                                     f"need {int(need[m])} (3 * (K-1) per segment)")
-                if nz.numel() == 0:
-                    nz = torch.zeros(1, dtype=torch.float64, device=self.device)
-            if not (seeds is not None and seed_stream == "device"):
-                rng_d = self._dev(rng, torch.int64) if B else None
+            nz, rng_d = self._mission_normals(n_seg, K, seeds, normals, normal_range, seed_stream)
             order_d = self._dev(order, torch.int32)
             mid = self._map_ids(map_id, B)
             if path_cap is None:
@@ -1011,17 +1036,17 @@ class Planner:
                                 seg_status=torch.empty((B, Sc), **i32), status=torch.empty(B, **i32),
                                 stop_seg=torch.empty(B, **i32), n_seg=torch.empty(B, **i32), waypoints=wp,
                                 n_waypoints=n_wp, path=torch.empty((B, int(path_cap), 8), **f64),
-                                path_seg=torch.empty((B, int(path_cap)), **i32), path_len=torch.empty(B, **i32), route=route)
+                                path_seg=torch.empty((B, int(path_cap)), **i32), path_len=torch.empty(B, **i32), route=route,
+                                schedule=(order, n_active))
             if B == 0:
                 return res
             wb = self.lib.trrt_mission_workspace_bytes(B, K)
             work = self._scratch("mission", wb)
-            ptr = lambda t: t.data_ptr() if t is not None else None  # noqa: E731
             n_active_h = np.ascontiguousarray(n_active, dtype=np.int32)
-            a = _lib.CMissionArgs(d_bits=g.bits.data_ptr(), n_maps=g.n_maps, H=g.H, W=g.W, d_map_id=ptr(mid),
+            a = _lib.CMissionArgs(d_bits=g.bits.data_ptr(), n_maps=g.n_maps, H=g.H, W=g.W, d_map_id=_ptr(mid),
                                   params=P.to_c(), xystdv=float(P.xystdv), anglestdv=float(P.anglestdv), n_missions=B, K=K,
                                   d_waypoints=wp.data_ptr(), wp_cap=int(wp.shape[1]), d_n_waypoints=n_wp.data_ptr(),
-                                  d_route_status=ptr(route_status), d_normals=nz.data_ptr(), d_normal_range=rng_d.data_ptr(),
+                                  d_route_status=_ptr(route_status), d_normals=nz.data_ptr(), d_normal_range=rng_d.data_ptr(),
                                   d_order=order_d.data_ptr(), n_stages=S, n_active=n_active_h.ctypes.data if S else None,
                                   seg_cap=Sc, d_seg_begin=res.begin.data_ptr(), d_seg_end=res.end.data_ptr(),
                                   d_seg_solution=res.solution.data_ptr(), d_seg_nearest=res.nearest.data_ptr(),
@@ -1032,6 +1057,49 @@ class Planner:
                                   d_path=res.path.data_ptr(), d_path_seg=res.path_seg.data_ptr(), path_cap=int(path_cap),
                                   d_path_len=res.path_len.data_ptr(), d_work=work.data_ptr(), work_bytes=work.numel())
             _lib.check(self.lib.trrt_mission_batch(C.byref(a), self._stream()), "trrt_mission_batch")
-            res._keep = (nz, rng_d, order_d, mid)
-            res.schedule = (order, n_active)
+            res.keep = (nz, rng_d, order_d, mid)
         return res
+
+    def _mission_normals(self, n_seg, K, seeds, normals, normal_range, seed_stream):
+        """The normals of a missions call and their [begin, end) per mission, both on the device: numpy's streams of
+        `seeds` (seed_stream "host"), the same drawn on the device ("device"), or the caller's `normals` and
+        `normal_range`, checked against the 3 * (K-1) values each segment of n_seg[m] needs.  An empty stream is one
+        zero, so that the kernel has a valid pointer."""
+        B = len(n_seg)
+        need = 3 * (K - 1) * n_seg
+        rng_d = None
+        if seeds is not None:
+            seeds = np.asarray(seeds).reshape(-1)
+            if len(seeds) != B:
+                raise ValueError(f"{len(seeds)} seeds for {B} missions")
+            if seed_stream == "device":
+                nz, rng_d = self.legacy_normals(seeds, need)
+            else:
+                rng = _ranges(need)
+                flat = np.empty(int(need.sum()), np.float64)
+                for m in range(B):
+                    if need[m]:
+                        flat[rng[m, 0]:rng[m, 1]] = np.random.RandomState(int(seeds[m])).standard_normal(int(need[m]))
+                nz = self._dev(flat, torch.float64)
+        else:
+            nz = self._dev(normals, torch.float64)
+            if normal_range is None:
+                if nz.dim() != 2 or nz.shape[0] != B:
+                    raise ValueError("normals without normal_range must be a [missions, L] array")
+                L = nz.shape[1]
+                rng = np.stack([np.arange(B) * L, np.arange(B) * L + L], axis=1).astype(np.int64)
+            else:
+                rng = _host_array(normal_range).astype(np.int64).reshape(B, 2)
+            nz = nz.reshape(-1)
+            if B and (rng.min() < 0 or rng[:, 1].max() > nz.numel() or (rng[:, 1] < rng[:, 0]).any()):
+                raise ValueError("normal_range outside the normals")
+            short = np.nonzero(rng[:, 1] - rng[:, 0] < need)[0]
+            if len(short):
+                m = int(short[0])
+                raise ValueError(f"mission {m} has {int(rng[m, 1] - rng[m, 0])} normals, its {int(n_seg[m])} segments "
+                                 f"need {int(need[m])} (3 * (K-1) per segment)")
+        if nz.numel() == 0:
+            nz = torch.zeros(1, dtype=torch.float64, device=self.device)
+        if rng_d is None and B:
+            rng_d = self._dev(rng, torch.int64)
+        return nz, rng_d

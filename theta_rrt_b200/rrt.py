@@ -15,7 +15,7 @@ import builtins
 import numpy as np
 
 from . import _context, samples
-from .planner import (IT_ARC_BLOCKED, IT_NOT_RUN, IT_QRAND_BLOCKED, IT_QRAND_IN_TREE, SEED_STREAMS, Planner, RrtResult)
+from .planner import IT_ARC_BLOCKED, IT_NOT_RUN, IT_QRAND_BLOCKED, IT_QRAND_IN_TREE, Planner, RrtResult, _check_seed_stream
 from .samples import standardangle as _standardangle_np
 
 
@@ -160,8 +160,7 @@ def rrt_batch(starts, goals, seeds=None, sample_xy=None, sample_th=None, K=None,
     on the device with seed_stream="device", Planner.rand_conf: the same bits) or explicit sample arrays.
     stop_at: per-query iteration stops (Planner.rrt); Planner.rrt_resume continues the paused queries with the samples
     the result keeps."""
-    if seed_stream not in SEED_STREAMS:
-        raise ValueError(f"seed_stream must be one of {SEED_STREAMS}")
+    _check_seed_stream(seed_stream)
     p = _context.current_planner()
     P = p.params
     K = int(K or P.K)
@@ -172,16 +171,7 @@ def rrt_batch(starts, goals, seeds=None, sample_xy=None, sample_th=None, K=None,
     if sample_xy is None:
         if seeds is None:
             raise ValueError("pass seeds or sample arrays")
-        nq = len(starts)
-        if seed_stream == "device":
-            sample_xy, sample_th = p.rand_conf(goals, seeds, K)
-            return p.rrt(starts, goals, sample_xy, sample_th, K=K, logs=logs, lanes=lanes, stop_at=stop_at)
-        sample_xy = np.empty((nq, K - 1, 2), np.int32)
-        sample_th = np.empty((nq, K - 1), np.float64)
-        for q in range(nq):
-            g = ((goals[q, 0], goals[q, 1]), goals[q, 2])
-            sample_xy[q], sample_th[q] = samples.make_stream(g, K - 1, int(seeds[q]), p.grid.shape, P.xystdv,
-                                                             P.anglestdv)
+        sample_xy, sample_th = p._seeded_samples(goals, seeds, K, seed_stream, P)
     return p.rrt(starts, goals, sample_xy, sample_th, K=K, logs=logs, lanes=lanes, stop_at=stop_at)
 
 

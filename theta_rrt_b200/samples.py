@@ -51,6 +51,17 @@ def make_stream(goal, n, seed, shape, xystdv=0.4, anglestdv=100):
     return stream_from_normals(z, goal, shape, xystdv, anglestdv)
 
 
+def make_streams(goals, n, seeds, shape, xystdv=0.4, anglestdv=100):
+    """make_stream for many queries: goals [q, 3] = (x, y, theta), seed int(seeds[q]) for query q.
+    Returns (xy int32 [q, n, 2], theta float64 [q, n])."""
+    goals = np.asarray(goals, dtype=np.float64).reshape(-1, 3)
+    xy = np.empty((len(goals), n, 2), np.int32)
+    th = np.empty((len(goals), n), np.float64)
+    for q, g in enumerate(goals):
+        xy[q], th[q] = make_stream(((g[0], g[1]), g[2]), n, int(seeds[q]), shape, xystdv, anglestdv)
+    return xy, th
+
+
 def draw_stream_global(goal, n, shape, xystdv=0.4, anglestdv=100):
     """Same, but consuming numpy's GLOBAL legacy generator like the reference does."""
     z = np.random.standard_normal(3 * n)
