@@ -130,6 +130,104 @@ int trrt_los_batch_tiled(const uint64_t *d_tiles, int n_maps, int H, int W, cons
                          int64_t n, uint8_t *d_out, void *stream);
 
 /* ---------------------------------------------------------------------------
+ * grid_edit.  Replaces the in-place mutation of builtins.imarray (main.py:42;
+ * the reference draws into it itself, search.getCircle(draw=True),
+ * search.py:139-141): imarray[y0:y1, x0:x1] = value for n rectangles, on the
+ * grid of trrt_pack_grid and, when d_tiles is not NULL, on its strip copy of
+ * trrt_tile_grid (only the entries the rectangles touch are rebuilt).
+ * d_rects: int32 [n][5] = x0, y0, x1, y1, map: pixels x0 <= x < x1,
+ * y0 <= y < y1 of map `map`; clipped to the image; empty rectangles and map
+ * ids outside [0, n_maps) do nothing.  d_free: uint8 [n], non-zero = set free,
+ * 0 = set blocked.  Blocked wins: a pixel that a free and a blocked rectangle
+ * of one call both cover ends blocked, whatever their order (the free masks
+ * are ORed in first, then the blocked ones cleared).  Padding bits stay 0.
+ * Bad arguments return TRRT_ERR_INVALID_ARGUMENT before any device work.
+ * Work that reads the grid on other streams is the caller's to order.
+ * ------------------------------------------------------------------------- */
+int trrt_grid_edit(uint32_t *d_bits, uint64_t *d_tiles /* NULL: no strip copy */, int n_maps, int H, int W,
+                   const int32_t *d_rects /* [n][5] x0, y0, x1, y1, map */, const uint8_t *d_free /* [n] */, int64_t n, void *stream);
+
+/* ---------------------------------------------------------------------------
+ * validate_tree.  Re-runs, on the map as it is now, the edge test that
+ * admitted each stored edge of trrt_rrt_batch trees: `False in
+ * [freespace(px) for px in getArc(qnear.xy, qnew.xy, u)]` (rrt.py:173-174),
+ * for node i's edge from parent[i] with u[i] (search.getArc / getCircle,
+ * search.py:96-182; a straight u, NaN icc / rad, is the Bresenham line between
+ * the int-truncated endpoints).  Nothing else is tested: a node whose own
+ * pixel is blocked but whose edge raster is free stays valid, as the
+ * reference would have admitted it.  The tree arrays are those of
+ * trrt_rrt_args (d_u required).
+ *   d_edge_ok [n_queries][K]: 1 for a node without a parent (-1), the verdict
+ *     for every other node < n_nodes (a parent outside [0, n_nodes) fails),
+ *     0 for rows at or past n_nodes;
+ *   d_node_ok [n_queries][K]: 1 when edge_ok holds for every node of the walk
+ *     main.path_nodes does from i: it follows parent for at most n_nodes - 1
+ *     steps and stops at a node without a parent; 0 past n_nodes;
+ *   d_sol_ok [n_queries]: node_ok[sol], -1 when sol < 0.
+ * lanes: lanes per edge, the values trrt_arc_batch accepts (0 = 8).
+ * d_work: 4-byte aligned scratch of trrt_validate_tree_workspace_bytes.
+ * K > 2^30 is TRRT_ERR_INVALID_ARGUMENT (the walk tables pack a node index
+ * and a bit into one int32).
+ * ------------------------------------------------------------------------- */
+typedef struct trrt_validate_tree_args {
+    const uint32_t *d_bits;
+    int32_t n_maps, H, W;
+    const int32_t *d_map_id;  /* [n_queries] map each tree was planned on, or NULL (all map 0) */
+    int64_t n_queries;
+    int32_t K;
+    int32_t lanes;
+    const double *d_node_x;   /* [n_queries][K] */
+    const double *d_node_y;   /* [n_queries][K] */
+    const int32_t *d_parent;  /* [n_queries][K] */
+    const double *d_u;        /* [n_queries][K][5] */
+    const int32_t *d_n_nodes; /* [n_queries] */
+    const int32_t *d_sol;     /* [n_queries] */
+    uint8_t *d_edge_ok;       /* [n_queries][K] */
+    uint8_t *d_node_ok;       /* [n_queries][K] */
+    int8_t *d_sol_ok;         /* [n_queries] */
+    void *d_work;
+    size_t work_bytes;
+} trrt_validate_tree_args;
+
+size_t trrt_validate_tree_workspace_bytes(int64_t n_queries, int32_t K); /* 256 + 12 * n_queries * K */
+int trrt_validate_tree(const trrt_validate_tree_args *args, void *stream);
+
+/* ---------------------------------------------------------------------------
+ * validate_path.  Planned rows re-checked on the map as it is now, read in
+ * place from the padded per-query arrays:
+ *   mode 0, Theta* / A* routes of trrt_theta_batch (d_route int32
+ *     [n][path_cap][2]): step 0 = search.freespace(wp[0]) (search.py:27-33),
+ *     step t = search.lineofsight(wp[t-1], wp[t]) (search.py:35-94);
+ *   mode 1, mission path rows of trrt_mission_batch (d_rows float64
+ *     [n][path_cap][8] = x, y, theta, u[5]; d_row_seg [n][path_cap]): step r =
+ *     the edge test of trrt_validate_tree from row r-1 to row r with row r's u
+ *     when both rows belong to one segment, 1 at a segment's first row.
+ * d_step_ok uint8 [n][path_cap]: rows past min(path_len, path_cap) are 0.
+ * d_ok uint8 [n]: 1 when d_status is 0 and every stored step is ok.  Only
+ * the stored prefix is checked: a path with path_len > path_cap and every
+ * stored step ok gets d_ok = 1 although its unstored steps were never tested
+ * (plan with a larger path_cap to check them).
+ * ------------------------------------------------------------------------- */
+typedef struct trrt_validate_path_args {
+    const uint32_t *d_bits;
+    int32_t n_maps, H, W;
+    const int32_t *d_map_id;  /* [n_paths] or NULL */
+    int32_t mode;             /* 0 routes, 1 mission rows */
+    int32_t lanes;            /* as trrt_validate_tree */
+    int64_t n_paths;
+    int32_t path_cap;
+    const int32_t *d_route;   /* mode 0 */
+    const double *d_rows;     /* mode 1 */
+    const int32_t *d_row_seg; /* mode 1 */
+    const int32_t *d_path_len; /* [n_paths] full length, may exceed path_cap */
+    const int32_t *d_status;  /* [n_paths] */
+    uint8_t *d_step_ok;       /* [n_paths][path_cap] */
+    uint8_t *d_ok;            /* [n_paths] */
+} trrt_validate_path_args;
+
+int trrt_validate_path(const trrt_validate_path_args *args, void *stream);
+
+/* ---------------------------------------------------------------------------
  * K1 nearest_batch.  Replaces the nearest-node scan of rrt.py:156-158
  * (np.argmin over search.L2norm, search.py:13-15): for each integer query
  * point, the index of the tree node with the smallest fp64 squared distance,

@@ -96,6 +96,28 @@ class CLegacyNormalsArgs(C.Structure):
     ]
 
 
+class CValidateTreeArgs(C.Structure):
+    """struct trrt_validate_tree_args."""
+    _fields_ = [
+        ("d_bits", C.c_void_p), ("n_maps", C.c_int32), ("H", C.c_int32), ("W", C.c_int32), ("d_map_id", C.c_void_p),
+        ("n_queries", C.c_int64), ("K", C.c_int32), ("lanes", C.c_int32),
+        ("d_node_x", C.c_void_p), ("d_node_y", C.c_void_p), ("d_parent", C.c_void_p), ("d_u", C.c_void_p),
+        ("d_n_nodes", C.c_void_p), ("d_sol", C.c_void_p),
+        ("d_edge_ok", C.c_void_p), ("d_node_ok", C.c_void_p), ("d_sol_ok", C.c_void_p),
+        ("d_work", C.c_void_p), ("work_bytes", C.c_size_t),
+    ]
+
+
+class CValidatePathArgs(C.Structure):
+    """struct trrt_validate_path_args."""
+    _fields_ = [
+        ("d_bits", C.c_void_p), ("n_maps", C.c_int32), ("H", C.c_int32), ("W", C.c_int32), ("d_map_id", C.c_void_p),
+        ("mode", C.c_int32), ("lanes", C.c_int32), ("n_paths", C.c_int64), ("path_cap", C.c_int32),
+        ("d_route", C.c_void_p), ("d_rows", C.c_void_p), ("d_row_seg", C.c_void_p),
+        ("d_path_len", C.c_void_p), ("d_status", C.c_void_p), ("d_step_ok", C.c_void_p), ("d_ok", C.c_void_p),
+    ]
+
+
 # every symbol include/thetarrt.h declares: name -> (restype, argtypes)
 SIGNATURES = {
     "trrt_version": (C.c_int, []),
@@ -110,6 +132,11 @@ SIGNATURES = {
     "trrt_tile_grid": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "trrt_los_batch_tiled": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int64,
                                        C.c_void_p, C.c_void_p]),
+    "trrt_grid_edit": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int64,
+                                 C.c_void_p]),
+    "trrt_validate_tree_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int32]),
+    "trrt_validate_tree": (C.c_int, [C.POINTER(CValidateTreeArgs), C.c_void_p]),
+    "trrt_validate_path": (C.c_int, [C.POINTER(CValidatePathArgs), C.c_void_p]),
     "trrt_nearest_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int64]),
     "trrt_nearest_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p,
                                      C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),

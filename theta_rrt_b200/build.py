@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "libthetarrt.so")
 SOURCES = ["thetarrt.cu"]
-HEADERS = ["trrt_device.cuh", "trrt_los.cuh", "trrt_bike.cuh", "trrt_lane.cuh", "trrt_rrt.cuh", "trrt_mission.cuh", "trrt_rng.cuh", "trrt_libm.h"]
+HEADERS = ["trrt_device.cuh", "trrt_edit.cuh", "trrt_los.cuh", "trrt_bike.cuh", "trrt_lane.cuh", "trrt_rrt.cuh", "trrt_mission.cuh", "trrt_rng.cuh", "trrt_libm.h"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -14,6 +14,9 @@
 //   findnearest_kernel    rrt.findnearest over the edge log
 //   mission_*_kernel      main.py missions: segment chain around trrt_rrt_batch, findnearest restarts (trrt_mission.cuh)
 //   theta_kernel<G>       K3: A* / lazy Theta*, G lanes per query, G-ary heap
+//   grid_edit_kernel / tile_patch_kernel  map edits in place, rows then the strip entries they touch (trrt_edit.cuh)
+//   validate_edges / validate_chain / validate_path kernels: planned trees, routes and mission paths re-checked
+//                             against the map as it is now (trrt_edit.cuh)
 //   legacy_normals_kernel / legacy_normals_fixup_kernel  numpy RandomState(seed).standard_normal streams (trrt_rng.cuh)
 //   rand_conf_kernel<XY>  rrt.rand_conf samples from such streams
 //
@@ -32,6 +35,7 @@
 #include "../../include/thetarrt.h"
 #include "trrt_bike.cuh"
 #include "trrt_device.cuh"
+#include "trrt_edit.cuh"
 #include "trrt_los.cuh"
 #include "trrt_mission.cuh"
 #include "trrt_rng.cuh"
@@ -892,6 +896,96 @@ int trrt_los_batch_tiled(const uint64_t *d_tiles, int n_maps, int H, int W, cons
     const unsigned blocks = (unsigned)((warps + LOS_WARPS - 1) / LOS_WARPS);
     los_tiled_kernel<<<blocks, LOS_WARPS * 32, 0, (cudaStream_t)stream>>>((const uint4 *)d_tiles, H, (W + 7) / 8, d_map_id, (const int4 *)d_seg,
                                                                           (long long)n, (int)rpw, refill_min, coop_max, d_out);
+    CUDA_TRY(cudaGetLastError());
+    return TRRT_OK;
+}
+
+int trrt_grid_edit(uint32_t *d_bits, uint64_t *d_tiles, int n_maps, int H, int W, const int32_t *d_rects, const uint8_t *d_free, int64_t n,
+                   void *stream) {
+    int e = check_map(n_maps, H, W);
+    if (e) return e;
+    if (n < 0 || !d_bits || (n > 0 && (!d_rects || !d_free)) || ((uintptr_t)d_tiles & 15) != 0) return TRRT_ERR_INVALID_ARGUMENT;
+    if (n == 0) return TRRT_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    const int wpr = (W + 31) / 32, tp = (W + 7) / 8;
+    const unsigned blocks = (unsigned)std::min<int64_t>(n, (int64_t)sm_count() * 64); // a CTA per rectangle, grid-stride beyond
+    grid_edit_kernel<<<blocks, 128, 0, st>>>(d_bits, n_maps, H, wpr, d_rects, d_free, n, 0);
+    CUDA_TRY(cudaGetLastError());
+    grid_edit_kernel<<<blocks, 128, 0, st>>>(d_bits, n_maps, H, wpr, d_rects, d_free, n, 1);
+    CUDA_TRY(cudaGetLastError());
+    if (d_tiles) {
+        tile_patch_kernel<<<blocks, 128, 0, st>>>(d_bits, n_maps, H, wpr, tp, d_rects, n, (uint4 *)d_tiles);
+        CUDA_TRY(cudaGetLastError());
+    }
+    return TRRT_OK;
+}
+
+size_t trrt_validate_tree_workspace_bytes(int64_t n_queries, int32_t K) {
+    if (n_queries < 0 || K < 1) return 0;
+    return 256 + (size_t)n_queries * (size_t)K * 3 * sizeof(int32_t);
+}
+
+// lanes of trrt_arc_batch: 0 = 8; else 1, 2, 4, 8, 16, 32 (0 = not one of them)
+static int edge_lanes(int lanes) {
+    if (lanes == 0) return 8;
+    return (lanes == 1 || lanes == 2 || lanes == 4 || lanes == 8 || lanes == 16 || lanes == 32) ? lanes : 0;
+}
+
+#define TRRT_LANES_SWITCH(G, CALL)                                              \
+    switch (G) {                                                                \
+    case 1: { constexpr int L = 1; CALL; } break;                               \
+    case 2: { constexpr int L = 2; CALL; } break;                               \
+    case 4: { constexpr int L = 4; CALL; } break;                               \
+    case 8: { constexpr int L = 8; CALL; } break;                               \
+    case 16: { constexpr int L = 16; CALL; } break;                             \
+    default: { constexpr int L = 32; CALL; } break;                             \
+    }
+
+int trrt_validate_tree(const trrt_validate_tree_args *args, void *stream) {
+    if (!args) return TRRT_ERR_INVALID_ARGUMENT;
+    const trrt_validate_tree_args &A = *args;
+    int e = check_map(A.n_maps, A.H, A.W);
+    if (e) return e;
+    const int G = edge_lanes(A.lanes);
+    // K <= 2^30: the chain tables pack (node index << 1) | bit into an int32
+    if (A.n_queries < 0 || A.K < 1 || A.K > (1 << 30) || G == 0) return TRRT_ERR_INVALID_ARGUMENT;
+    if (A.n_queries == 0) return TRRT_OK;
+    if (!A.d_bits || !A.d_node_x || !A.d_node_y || !A.d_parent || !A.d_u || !A.d_n_nodes || !A.d_sol || !A.d_edge_ok || !A.d_node_ok ||
+        !A.d_sol_ok || !A.d_work || ((uintptr_t)A.d_work & 3) != 0)
+        return TRRT_ERR_INVALID_ARGUMENT;
+    if (A.work_bytes < trrt_validate_tree_workspace_bytes(A.n_queries, A.K)) return TRRT_ERR_WORKSPACE_TOO_SMALL;
+    TreeDev d;
+    d.bits = A.d_bits; d.n_maps = A.n_maps; d.side = A.H; d.wpr = (A.W + 31) / 32; d.K = A.K; d.map_id = A.d_map_id;
+    d.nq = A.n_queries; d.nx = A.d_node_x; d.ny = A.d_node_y; d.u = A.d_u; d.parent = A.d_parent; d.n_nodes = A.d_n_nodes;
+    d.sol = A.d_sol; d.edge_ok = A.d_edge_ok; d.node_ok = A.d_node_ok; d.sol_ok = A.d_sol_ok; d.work = (int32_t *)A.d_work;
+    cudaStream_t st = (cudaStream_t)stream;
+    const int64_t edges = A.n_queries * (int64_t)A.K;
+    const unsigned eblocks = (unsigned)std::min<int64_t>((edges * G + 127) / 128, (int64_t)sm_count() * 32);
+    TRRT_LANES_SWITCH(G, (validate_edges_kernel<L><<<eblocks, 128, 0, st>>>(d)));
+    CUDA_TRY(cudaGetLastError());
+    const unsigned cblocks = (unsigned)std::min<int64_t>(A.n_queries, (int64_t)sm_count() * 64);
+    validate_chain_kernel<<<cblocks, 256, 0, st>>>(d);
+    CUDA_TRY(cudaGetLastError());
+    return TRRT_OK;
+}
+
+int trrt_validate_path(const trrt_validate_path_args *args, void *stream) {
+    if (!args) return TRRT_ERR_INVALID_ARGUMENT;
+    const trrt_validate_path_args &A = *args;
+    int e = check_map(A.n_maps, A.H, A.W);
+    if (e) return e;
+    const int G = edge_lanes(A.lanes);
+    if (A.n_paths < 0 || A.path_cap < 0 || G == 0 || (A.mode != 0 && A.mode != 1)) return TRRT_ERR_INVALID_ARGUMENT;
+    if (A.n_paths == 0) return TRRT_OK;
+    if (!A.d_bits || !A.d_path_len || !A.d_status || !A.d_ok || (A.path_cap > 0 && !A.d_step_ok)) return TRRT_ERR_INVALID_ARGUMENT;
+    if (A.path_cap > 0 && (A.mode == 0 ? !A.d_route : (!A.d_rows || !A.d_row_seg))) return TRRT_ERR_INVALID_ARGUMENT;
+    PathDev d;
+    d.bits = A.d_bits; d.n_maps = A.n_maps; d.side = A.H; d.wpr = (A.W + 31) / 32; d.mode = A.mode; d.cap = A.path_cap;
+    d.map_id = A.d_map_id; d.n = A.n_paths; d.route = A.d_route; d.rows = A.d_rows; d.row_seg = A.d_row_seg; d.len = A.d_path_len;
+    d.status = A.d_status; d.step_ok = A.d_step_ok; d.ok = A.d_ok;
+    cudaStream_t st = (cudaStream_t)stream;
+    const unsigned blocks = (unsigned)std::min<int64_t>((A.n_paths + 3) / 4, (int64_t)sm_count() * 32); // 4 warps, a warp per path
+    TRRT_LANES_SWITCH(G, (validate_path_kernel<L><<<blocks, 128, 0, st>>>(d)));
     CUDA_TRY(cudaGetLastError());
     return TRRT_OK;
 }

@@ -40,29 +40,34 @@ __device__ __forceinline__ unsigned strip_row_byte(const uint32_t *__restrict__ 
     return (__ldg(bits + (size_t)y * wpr + (xb >> 2)) >> ((xb & 3) * 8)) & 0xffu;
 }
 
+// Strip entry (K, c) of orientation `orient` of one map (src = its packed rows), built from the packed rows.  The one
+// definition of the strip layout on the write side: the full build and the patch after a map edit both call it.
+__device__ __forceinline__ uint4 strip_entry(const uint32_t *__restrict__ src, int side, int wpr, int tp, int orient, int K, int c) {
+    unsigned w[4] = {0u, 0u, 0u, 0u};
+    if (!orient) {
+        // driving axis x: byte j = pixels (8c .. 8c+7, y = 8K-8+j)
+#pragma unroll
+        for (int j = 0; j < 16; j++) w[j >> 2] |= strip_row_byte(src, side, wpr, tp, 8 * K - 8 + j, c) << ((j & 3) * 8);
+    } else {
+        // driving axis y: byte j = pixels (x = 8K-8+j, 8c .. 8c+7): transpose 8 rows of 16 pixels
+#pragma unroll
+        for (int i = 0; i < 8; i++) {
+            const int y = 8 * c + i;
+            const unsigned v = strip_row_byte(src, side, wpr, tp, y, K - 1) | (strip_row_byte(src, side, wpr, tp, y, K) << 8);
+#pragma unroll
+            for (int j = 0; j < 16; j++) w[j >> 2] |= ((v >> j) & 1u) << ((j & 3) * 8 + i);
+        }
+    }
+    return make_uint4(w[0], w[1], w[2], w[3]);
+}
+
 // bit-packed rows -> strip entries of both orientations; one thread per entry
 __global__ void tile_grid_kernel(const uint32_t *__restrict__ bits, int n_maps, int side, int wpr, int tp, uint4 *__restrict__ tiles) {
     const size_t epo = (size_t)(tp + 1) * tp, total = epo * 2 * n_maps;
     for (size_t e = blockIdx.x * (size_t)blockDim.x + threadIdx.x; e < total; e += (size_t)gridDim.x * blockDim.x) {
         const size_t m = e / (2 * epo), r = e - m * 2 * epo;
         const int orient = r >= epo, K = (int)((r - (orient ? epo : 0)) / tp), c = (int)((r - (orient ? epo : 0)) - (size_t)K * tp);
-        const uint32_t *src = bits + m * (size_t)side * wpr;
-        unsigned w[4] = {0u, 0u, 0u, 0u};
-        if (!orient) {
-            // driving axis x: byte j = pixels (8c .. 8c+7, y = 8K-8+j)
-#pragma unroll
-            for (int j = 0; j < 16; j++) w[j >> 2] |= strip_row_byte(src, side, wpr, tp, 8 * K - 8 + j, c) << ((j & 3) * 8);
-        } else {
-            // driving axis y: byte j = pixels (x = 8K-8+j, 8c .. 8c+7): transpose 8 rows of 16 pixels
-#pragma unroll
-            for (int i = 0; i < 8; i++) {
-                const int y = 8 * c + i;
-                const unsigned v = strip_row_byte(src, side, wpr, tp, y, K - 1) | (strip_row_byte(src, side, wpr, tp, y, K) << 8);
-#pragma unroll
-                for (int j = 0; j < 16; j++) w[j >> 2] |= ((v >> j) & 1u) << ((j & 3) * 8 + i);
-            }
-        }
-        tiles[e] = make_uint4(w[0], w[1], w[2], w[3]);
+        tiles[e] = strip_entry(bits + m * (size_t)side * wpr, side, wpr, tp, orient, K, c);
     }
 }
 

@@ -175,6 +175,7 @@ class ThetaResult:
     pushes: torch.Tensor | None = None
     extra: dict = field(default_factory=dict)
     keep: tuple = field(default=(), repr=False, metadata=_PRIVATE)  # inputs alive until the stream has consumed them
+    map_id: torch.Tensor | None = field(default=None, repr=False, metadata=_PRIVATE)  # map of each query (None: map 0)
 
     def host(self):
         return _host_dict(self)
@@ -211,12 +212,37 @@ class MissionResult:
     route: ThetaResult | None = None
     schedule: tuple | None = None
     keep: tuple = field(default=(), repr=False, metadata=_PRIVATE)  # inputs alive until the stream has consumed them
+    map_id: torch.Tensor | None = field(default=None, repr=False, metadata=_PRIVATE)  # map of each mission (None: map 0)
 
     def host(self):
         out = _host_dict(self)
         if self.route is not None:
             out["route"] = self.route.host()
         return out
+
+
+@dataclass
+class TreeValidity:
+    """Planner.validate_tree output: edge_ok uint8 [q, K] (node i's edge from parent[i], tested again; 1 for a node
+    without a parent, 0 at or past n_nodes), node_ok uint8 [q, K] (every edge of the walk from i to the root is ok),
+    sol_ok int8 [q] (node_ok[sol], -1 when there is no solution)."""
+    edge_ok: torch.Tensor
+    node_ok: torch.Tensor
+    sol_ok: torch.Tensor
+
+    def host(self):
+        return _host_dict(self)
+
+
+@dataclass
+class PathValidity:
+    """Planner.validate_path output: step_ok uint8 [q, path_cap] (per stored row; 0 past the path's length) and ok
+    uint8 [q] (status 0 and every stored step ok: steps past path_cap are not checked)."""
+    step_ok: torch.Tensor
+    ok: torch.Tensor
+
+    def host(self):
+        return _host_dict(self)
 
 
 SEED_STREAMS = ("host", "device")
@@ -688,6 +714,76 @@ class Planner:
                 main.wait_event(e)
             self._pending = []
 
+    # ------------------------------------------------------------------ map edits and validation
+    def edit_map(self, rects, free, map_id=None):
+        """Edit this planner's map in place: OccupancyGrid.edit (imarray[y0:y1, x0:x1] = free per rectangle) on the
+        current stream, after every rrt_host piece of this planner that is still in flight, so that no batch enqueued with
+        wait=False plans on a half-edited map.  Work the caller has enqueued on other streams is the caller's to order,
+        as with any in-place write to a tensor.  A paused result resumed after an edit (rrt_resume) plans its remaining
+        iterations on the map as it is at resume time."""
+        with torch.cuda.device(self.device):
+            main = torch.cuda.current_stream(self.device)
+            for e in self._pending + [d[5] for d in self._deferred]:
+                main.wait_event(e)
+            self.grid.edit(rects, free, map_id)
+
+    def validate_tree(self, res: RrtResult, lanes=0) -> TreeValidity:
+        """Test every stored edge of an rrt result again on the map as it is now, with the test that admitted it:
+        getArc(parent.xy, node.xy, u) for node i's edge from parent[i] with u[i] (rrt.py:173-174), the Bresenham line
+        between the int-truncated endpoints for a straight u, on the map the query was planned on.  Nothing more is
+        tested: a node whose own pixel is blocked but whose edge raster is free stays valid, as the reference would have
+        admitted it.  node_ok follows the walk main.path_nodes does (at most n_nodes - 1 parent steps, stopping at a node
+        without a parent).  lanes: lanes per edge (0, 1, 2, 4, 8, 16, 32; the values arc_blocked accepts)."""
+        if res.u is None:
+            raise ValueError("validate_tree needs the edges' u: plan with want_u=True")
+        if res.launch is None or res.launch.grid is not self.grid:
+            raise ValueError("validate_tree checks a result that Planner.rrt planned on this planner's grid")
+        g = self.grid
+        nq, K = res.node_x.shape[0], res.K
+        with torch.cuda.device(self.device):
+            out = TreeValidity(edge_ok=torch.empty((nq, K), dtype=torch.uint8, device=self.device),
+                               node_ok=torch.empty((nq, K), dtype=torch.uint8, device=self.device),
+                               sol_ok=torch.empty(nq, dtype=torch.int8, device=self.device))
+            work = self._scratch("validate_tree", self.lib.trrt_validate_tree_workspace_bytes(nq, K))
+            a = _lib.CValidateTreeArgs(d_bits=g.bits.data_ptr(), n_maps=g.n_maps, H=g.H, W=g.W,
+                                       d_map_id=_ptr(res.launch.map_id), n_queries=nq, K=K, lanes=int(lanes),
+                                       d_node_x=res.node_x.data_ptr(), d_node_y=res.node_y.data_ptr(),
+                                       d_parent=res.parent.data_ptr(), d_u=res.u.data_ptr(), d_n_nodes=res.n_nodes.data_ptr(),
+                                       d_sol=res.sol.data_ptr(), d_edge_ok=out.edge_ok.data_ptr(),
+                                       d_node_ok=out.node_ok.data_ptr(), d_sol_ok=out.sol_ok.data_ptr(),
+                                       d_work=work.data_ptr(), work_bytes=work.numel())
+            _lib.check(self.lib.trrt_validate_tree(C.byref(a), self._stream()), "trrt_validate_tree")
+        return out
+
+    def validate_path(self, res, lanes=0) -> PathValidity:
+        """Check planned rows again on the map as it is now, on the maps they were planned on.  A ThetaResult: step 0 is
+        search.freespace(wp[0]), step t search.lineofsight(wp[t-1], wp[t]); a route passes on the map it was planned on
+        by construction.  A MissionResult: row r is the edge test of validate_tree from row r-1 to row r with row r's u
+        when both rows belong to one segment, and 1 at a segment's first row.  ok: status 0 and every stored row
+        (min(path_len, path_cap)) ok; rows past path_cap were not stored and are not checked, so a path longer than its
+        path_cap can be ok while a step beyond the cap is blocked.  The padded arrays are read in place; nothing waits
+        for the device."""
+        g = self.grid
+        if isinstance(res, ThetaResult):
+            mode, n, cap = 0, res.path.shape[0], res.path.shape[1]
+            ptrs = dict(d_route=res.path.data_ptr(), d_rows=None, d_row_seg=None)
+        elif isinstance(res, MissionResult):
+            mode, n, cap = 1, res.path.shape[0], res.path.shape[1]
+            ptrs = dict(d_route=None, d_rows=res.path.data_ptr(), d_row_seg=res.path_seg.data_ptr())
+        else:
+            raise ValueError("validate_path checks a ThetaResult or a MissionResult")
+        with torch.cuda.device(self.device):
+            out = PathValidity(step_ok=torch.empty((n, cap), dtype=torch.uint8, device=self.device),
+                               ok=torch.empty(n, dtype=torch.uint8, device=self.device))
+            if n == 0:
+                return out
+            a = _lib.CValidatePathArgs(d_bits=g.bits.data_ptr(), n_maps=g.n_maps, H=g.H, W=g.W, d_map_id=_ptr(res.map_id),
+                                       mode=mode, lanes=int(lanes), n_paths=n, path_cap=cap, **ptrs,
+                                       d_path_len=res.path_len.data_ptr(), d_status=res.status.data_ptr(),
+                                       d_step_ok=out.step_ok.data_ptr(), d_ok=out.ok.data_ptr())
+            _lib.check(self.lib.trrt_validate_path(C.byref(a), self._stream()), "trrt_validate_path")
+        return out
+
     def findnearest(self, res: RrtResult, goals, params=None):
         """rrt.findnearest (rrt.py:117-128) for every query of an RrtResult produced with logs=True."""
         if res.it_near is None:
@@ -845,7 +941,8 @@ class Planner:
             a.work_bytes = work.numel()
             _lib.check(self.lib.trrt_theta_batch(C.byref(a), self._stream()), "trrt_theta_batch")
             res.extra = dict(n_slots=int(a.n_slots), heap_cap=int(a.heap_cap), workspace_bytes=int(wb))
-            res.keep = (sg, mid, order)
+            res.keep = (sg, order)
+            res.map_id = mid
         return res
 
     # ------------------------------------------------------------------ seeded streams
@@ -1037,7 +1134,7 @@ class Planner:
                                 stop_seg=torch.empty(B, **i32), n_seg=torch.empty(B, **i32), waypoints=wp,
                                 n_waypoints=n_wp, path=torch.empty((B, int(path_cap), 8), **f64),
                                 path_seg=torch.empty((B, int(path_cap)), **i32), path_len=torch.empty(B, **i32), route=route,
-                                schedule=(order, n_active))
+                                schedule=(order, n_active), map_id=mid)
             if B == 0:
                 return res
             wb = self.lib.trrt_mission_workspace_bytes(B, K)
@@ -1057,7 +1154,7 @@ class Planner:
                                   d_path=res.path.data_ptr(), d_path_seg=res.path_seg.data_ptr(), path_cap=int(path_cap),
                                   d_path_len=res.path_len.data_ptr(), d_work=work.data_ptr(), work_bytes=work.numel())
             _lib.check(self.lib.trrt_mission_batch(C.byref(a), self._stream()), "trrt_mission_batch")
-            res.keep = (nz, rng_d, order_d, mid)
+            res.keep = (nz, rng_d, order_d)
         return res
 
     def _mission_normals(self, n_seg, K, seeds, normals, normal_range, seed_stream):
