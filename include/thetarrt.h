@@ -193,6 +193,68 @@ size_t trrt_validate_tree_workspace_bytes(int64_t n_queries, int32_t K); /* 256 
 int trrt_validate_tree(const trrt_validate_tree_args *args, void *stream);
 
 /* ---------------------------------------------------------------------------
+ * repair_tree.  Tree repair of dynamic RRT replanning after a map edit, on
+ * G / cameFrom (rrt.py:134-201): the nodes whose walk of main.path_nodes to
+ * the start crosses an edge that trrt_validate_tree now fails are removed, the
+ * survivors compacted, and queries whose solution was cut reopened, so that a
+ * trrt_rrt_batch resume grows them on the edited map with the rest of their
+ * sample stream.  Pure tree surgery on the arrays of trrt_rrt_args (d_u
+ * required), updated in place; the map enters only through d_edge_ok, the
+ * output of trrt_validate_tree for the map as it is now.  Per query q, over
+ * its n = n_nodes[q] stored rows:
+ *   - node 0 (the start) is kept, with parent -1 and u NaN x 5 as the
+ *     planning call plants it (a sample that re-hits the start overwrites its
+ *     cameFrom entry, rrt.py:187-188);
+ *   - node i >= 1 is kept when following parent from i reaches node 0 within
+ *     n - 1 steps (the walk of main.path_nodes) and edge_ok is 1 for every
+ *     node the walk leaves before node 0.  The kept set is closed under
+ *     parent; nodes of a parent cycle that never reaches node 0 are dropped;
+ *     on an unedited map nothing is dropped;
+ *   - the kept rows (x, y, theta, parent, u) move together, in their order
+ *     (insertion order, the nearest scan's tie-break), parents remapped
+ *     through d_new_index; n_nodes becomes the kept count; rows at or past it
+ *     are left as they are;
+ *   - a kept sol is remapped and the status kept.  Otherwise sol = -1, and
+ *     TRRT_OK_FOUND becomes TRRT_PAUSED when iters < K-1, TRRT_OK_NOT_FOUND
+ *     otherwise.  iters never changes (a resume continues with sample iters);
+ *     every other status stays;
+ *   - race keys (optional, trrt_rrt_race): each group's key becomes the min of
+ *     (iters << 32) | q over its members with status TRRT_OK_FOUND after the
+ *     repair, UINT64_MAX when there is none.
+ *   d_new_index [n_queries][K]: the new row of old row i, -1 for pruned rows
+ *     and rows >= n; d_n_pruned [n_queries] (may be NULL): rows removed.
+ * Per-iteration logs name old node indices and are not remapped: repair trees
+ * planned without them.  K > 2^30 is TRRT_ERR_INVALID_ARGUMENT (the walk
+ * tables pack a node index and a bit into one int32), as are NULL required
+ * pointers, a race key without groups or groups without a key, and
+ * n_queries >= 2^32 with a race, all before any device work.
+ * ------------------------------------------------------------------------- */
+typedef struct trrt_repair_tree_args {
+    int64_t n_queries;
+    int32_t K;
+    double *d_node_x;            /* [n_queries][K] */
+    double *d_node_y;            /* [n_queries][K] */
+    double *d_node_th;           /* [n_queries][K] */
+    int32_t *d_parent;           /* [n_queries][K] */
+    double *d_u;                 /* [n_queries][K][5] */
+    int32_t *d_n_nodes;          /* [n_queries] */
+    int32_t *d_sol;              /* [n_queries] */
+    int32_t *d_status;           /* [n_queries] */
+    const int32_t *d_iters;      /* [n_queries] */
+    const uint8_t *d_edge_ok;    /* [n_queries][K] of trrt_validate_tree */
+    int32_t *d_new_index;        /* [n_queries][K] */
+    int32_t *d_n_pruned;         /* [n_queries] or NULL */
+    const int32_t *d_race_group; /* [n_queries] or NULL (no race) */
+    int64_t n_race_groups;
+    uint64_t *d_race_key;        /* [n_race_groups] or NULL */
+    void *d_work;                /* 4-byte aligned */
+    size_t work_bytes;
+} trrt_repair_tree_args;
+
+size_t trrt_repair_tree_workspace_bytes(int64_t n_queries, int32_t K); /* 256 + 12 * n_queries * K */
+int trrt_repair_tree(const trrt_repair_tree_args *args, void *stream);
+
+/* ---------------------------------------------------------------------------
  * validate_path.  Planned rows re-checked on the map as it is now, read in
  * place from the padded per-query arrays:
  *   mode 0, Theta* / A* routes of trrt_theta_batch (d_route int32

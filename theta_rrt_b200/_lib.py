@@ -108,6 +108,18 @@ class CValidateTreeArgs(C.Structure):
     ]
 
 
+class CRepairTreeArgs(C.Structure):
+    """struct trrt_repair_tree_args."""
+    _fields_ = [
+        ("n_queries", C.c_int64), ("K", C.c_int32),
+        ("d_node_x", C.c_void_p), ("d_node_y", C.c_void_p), ("d_node_th", C.c_void_p), ("d_parent", C.c_void_p),
+        ("d_u", C.c_void_p), ("d_n_nodes", C.c_void_p), ("d_sol", C.c_void_p), ("d_status", C.c_void_p),
+        ("d_iters", C.c_void_p), ("d_edge_ok", C.c_void_p), ("d_new_index", C.c_void_p), ("d_n_pruned", C.c_void_p),
+        ("d_race_group", C.c_void_p), ("n_race_groups", C.c_int64), ("d_race_key", C.c_void_p),
+        ("d_work", C.c_void_p), ("work_bytes", C.c_size_t),
+    ]
+
+
 class CValidatePathArgs(C.Structure):
     """struct trrt_validate_path_args."""
     _fields_ = [
@@ -137,6 +149,8 @@ SIGNATURES = {
     "trrt_validate_tree_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int32]),
     "trrt_validate_tree": (C.c_int, [C.POINTER(CValidateTreeArgs), C.c_void_p]),
     "trrt_validate_path": (C.c_int, [C.POINTER(CValidatePathArgs), C.c_void_p]),
+    "trrt_repair_tree_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int32]),
+    "trrt_repair_tree": (C.c_int, [C.POINTER(CRepairTreeArgs), C.c_void_p]),
     "trrt_nearest_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int64]),
     "trrt_nearest_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p,
                                      C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),

@@ -17,6 +17,8 @@
 //   grid_edit_kernel / tile_patch_kernel  map edits in place, rows then the strip entries they touch (trrt_edit.cuh)
 //   validate_edges / validate_chain / validate_path kernels: planned trees, routes and mission paths re-checked
 //                             against the map as it is now (trrt_edit.cuh)
+//   repair_tree_kernel / repair_race_kernel  RRT trees pruned to what an edit left reachable, compacted, cut solutions
+//                             reopened, race keys recomputed (trrt_edit.cuh)
 //   legacy_normals_kernel / legacy_normals_fixup_kernel  numpy RandomState(seed).standard_normal streams (trrt_rng.cuh)
 //   rand_conf_kernel<XY>  rrt.rand_conf samples from such streams
 //
@@ -966,6 +968,43 @@ int trrt_validate_tree(const trrt_validate_tree_args *args, void *stream) {
     const unsigned cblocks = (unsigned)std::min<int64_t>(A.n_queries, (int64_t)sm_count() * 64);
     validate_chain_kernel<<<cblocks, 256, 0, st>>>(d);
     CUDA_TRY(cudaGetLastError());
+    return TRRT_OK;
+}
+
+size_t trrt_repair_tree_workspace_bytes(int64_t n_queries, int32_t K) { return trrt_validate_tree_workspace_bytes(n_queries, K); }
+
+int trrt_repair_tree(const trrt_repair_tree_args *args, void *stream) {
+    if (!args) return TRRT_ERR_INVALID_ARGUMENT;
+    const trrt_repair_tree_args &A = *args;
+    // K <= 2^30: the walk tables pack (node index << 1) | bit into an int32; the race key packs q into 32 bits
+    if (A.n_queries < 0 || A.K < 1 || A.K > (1 << 30)) return TRRT_ERR_INVALID_ARGUMENT;
+    // a race needs its key array and at least one group; the group ids may only be absent for an empty batch
+    const bool race = A.d_race_key || A.d_race_group || A.n_race_groups != 0;
+    if (race && (!A.d_race_key || A.n_race_groups < 1 || (A.n_queries > 0 && !A.d_race_group) || A.n_queries > (int64_t)0xffffffffll))
+        return TRRT_ERR_INVALID_ARGUMENT;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (A.n_queries == 0) { // no member holds TRRT_OK_FOUND
+        if (race) CUDA_TRY(cudaMemsetAsync(A.d_race_key, 0xff, (size_t)A.n_race_groups * sizeof(uint64_t), st));
+        return TRRT_OK;
+    }
+    if (!A.d_node_x || !A.d_node_y || !A.d_node_th || !A.d_parent || !A.d_u || !A.d_n_nodes || !A.d_sol || !A.d_status || !A.d_iters ||
+        !A.d_edge_ok || !A.d_new_index || !A.d_work || ((uintptr_t)A.d_work & 3) != 0)
+        return TRRT_ERR_INVALID_ARGUMENT;
+    if (A.work_bytes < trrt_repair_tree_workspace_bytes(A.n_queries, A.K)) return TRRT_ERR_WORKSPACE_TOO_SMALL;
+    RepairDev d;
+    d.nq = A.n_queries; d.K = A.K; d.nx = A.d_node_x; d.ny = A.d_node_y; d.nth = A.d_node_th; d.u = A.d_u; d.parent = A.d_parent;
+    d.n_nodes = A.d_n_nodes; d.sol = A.d_sol; d.status = A.d_status; d.iters = A.d_iters; d.edge_ok = A.d_edge_ok;
+    d.new_index = A.d_new_index; d.n_pruned = A.d_n_pruned; d.work = (int32_t *)A.d_work;
+    const unsigned blocks = (unsigned)std::min<int64_t>(A.n_queries, (int64_t)sm_count() * 64);
+    repair_tree_kernel<<<blocks, REPAIR_THREADS, 0, st>>>(d);
+    CUDA_TRY(cudaGetLastError());
+    if (race) {
+        CUDA_TRY(cudaMemsetAsync(A.d_race_key, 0xff, (size_t)A.n_race_groups * sizeof(uint64_t), st));
+        const unsigned rblocks = (unsigned)std::min<int64_t>((A.n_queries + 255) / 256, (int64_t)sm_count() * 16);
+        repair_race_kernel<<<rblocks, 256, 0, st>>>(A.d_status, A.d_iters, A.d_race_group, A.n_race_groups,
+                                                    (unsigned long long *)A.d_race_key, A.n_queries);
+        CUDA_TRY(cudaGetLastError());
+    }
     return TRRT_OK;
 }
 

@@ -135,60 +135,183 @@ __global__ void __launch_bounds__(128) validate_edges_kernel(const TreeDev a) {
     }
 }
 
+// The walks c_0 = i, c_1 = next(c_0), ... of every node i < n of one query at once, `steps` steps each, by pointer
+// doubling over the whole CTA.  On entry T0[i] = next(i) * 2 | bit(i), with next(i) = -1 where a walk ends, and
+// W[i] = i * 2 | 1.  Table T_k[i] packs (node 2^k steps from i, or -1 where the walk ends first) * 2 | AND of the bits
+// of those 2^k nodes; T_{k+1} composes T_k with itself, and round k folds T_k into W when bit k of `steps` is set.  On
+// exit W[i] = (node `steps` steps from i, or -1 where the walk ended first) * 2 | AND of the bits of the nodes it left.
+// Exact whatever the order of the parents (they may point to higher indices) in ceil(log2(steps + 1)) rounds; the
+// caller's barrier must separate the writes of T0 and W from the call.  K <= 2^30: an index and a bit share an int32.
+__device__ __forceinline__ void chain_walk(int32_t *T0, int32_t *T1, int32_t *W, int n, int steps) {
+    for (int k = 0; k < 31 && steps > 0 && (steps >> k) != 0; k++) {
+        const int32_t *cur = (k & 1) ? T1 : T0;
+        int32_t *nxt = (k & 1) ? T0 : T1;
+        const bool take = (steps >> k) & 1, more = (steps >> (k + 1)) != 0;
+        for (int i = threadIdx.x; i < n; i += blockDim.x) {
+            if (take) {
+                const int32_t s = W[i];
+                const int pos = s >> 1;
+                if (pos >= 0) {
+                    TRRT_CHECK(pos < n);
+                    const int32_t w = cur[pos];
+                    W[i] = (w & ~1) | (s & w & 1);
+                }
+            }
+            if (more) {
+                int32_t w = cur[i];
+                const int j = w >> 1;
+                if (j >= 0) {
+                    TRRT_CHECK(j < n);
+                    const int32_t v = cur[j];
+                    w = (v & ~1) | (w & v & 1);
+                }
+                nxt[i] = w;
+            }
+        }
+        __syncthreads();
+    }
+}
+
 // node_ok of one query per CTA: the AND of edge_ok over the nodes c_0 = i, c_1 = parent[c_0], ... of the walk
 // main.path_nodes does, which follows parent for at most n_nodes - 1 steps and stops at a node without a parent (the
-// cut of trrt_mission.cuh, so parent cycles through an overwritten root are well defined).  Table T_k[i] packs
-// (node 2^k steps from i, or -1 where the walk ends first) << 1 | AND of edge_ok over those 2^k nodes; T_{k+1} composes
-// T_k with itself, and round k folds T_k into the walk of every node when bit k of n_nodes - 1 is set.  Exact whatever the
-// order of the parents (they may point to higher indices) in ceil(log2 n_nodes) rounds.
+// cut of trrt_mission.cuh, so parent cycles through an overwritten root are well defined): chain_walk with next = parent
+// and bit = edge_ok.
 __global__ void __launch_bounds__(256) validate_chain_kernel(const TreeDev a) {
     const int K = a.K;
     for (int64_t q = blockIdx.x; q < a.nq; q += gridDim.x) {
-        int32_t *T0 = a.work + q * 3 * (int64_t)K, *T1 = T0 + K, *P = T1 + K;
+        int32_t *T0 = a.work + q * 3 * (int64_t)K, *T1 = T0 + K, *W = T1 + K;
         const uint8_t *eok = a.edge_ok + q * (int64_t)K;
         uint8_t *nok = a.node_ok + q * (int64_t)K;
-        const int n = min(max(a.n_nodes[q], 0), K), steps = n - 1;
-        for (int i = threadIdx.x; i < K; i += blockDim.x) {
-            if (i < n) {
-                const int p = a.parent[q * K + i];
-                T0[i] = ((p >= 0 && p < n ? p : -1) * 2) | eok[i];
-                P[i] = i;
-            }
-            nok[i] = i < n ? 1 : 0;
+        const int n = min(max(a.n_nodes[q], 0), K);
+        for (int i = threadIdx.x; i < n; i += blockDim.x) {
+            const int p = a.parent[q * K + i];
+            T0[i] = ((p >= 0 && p < n ? p : -1) * 2) | eok[i];
+            W[i] = i * 2 | 1;
         }
         __syncthreads();
-        for (int k = 0; k < 31 && steps > 0 && (steps >> k) != 0; k++) {
-            const int32_t *cur = (k & 1) ? T1 : T0;
-            int32_t *nxt = (k & 1) ? T0 : T1;
-            const bool take = (steps >> k) & 1, more = (steps >> (k + 1)) != 0;
-            for (int i = threadIdx.x; i < n; i += blockDim.x) {
-                if (take) {
-                    const int pos = P[i];
-                    if (pos >= 0) {
-                        TRRT_CHECK(pos < n);
-                        const int32_t w = cur[pos];
-                        nok[i] &= (uint8_t)(w & 1);
-                        P[i] = w >> 1;
-                    }
-                }
-                if (more) {
-                    int32_t w = cur[i];
-                    const int j = w >> 1;
-                    if (j >= 0) {
-                        TRRT_CHECK(j < n);
-                        const int32_t v = cur[j];
-                        w = (v & ~1) | (w & v & 1);
-                    }
-                    nxt[i] = w;
-                }
-            }
-            __syncthreads();
-        }
+        chain_walk(T0, T1, W, n, n - 1);
+        for (int i = threadIdx.x; i < K; i += blockDim.x) nok[i] = i < n ? (uint8_t)(W[i] & 1) : 0;
+        __syncthreads();
         if (threadIdx.x == 0) {
             const int s = a.sol[q];
             a.sol_ok[q] = s < 0 ? (int8_t)-1 : (int8_t)(s < n ? nok[s] : 0);
         }
         __syncthreads(); // the next query of this CTA reuses nothing, but its tables start from a clean barrier
+    }
+}
+
+// ---------------------------------------------------------------------------
+// Tree repair
+// ---------------------------------------------------------------------------
+struct RepairDev {
+    int64_t nq;
+    int K;
+    double *nx, *ny, *nth, *u;
+    int32_t *parent, *n_nodes, *sol, *status;
+    const int32_t *iters;
+    const uint8_t *edge_ok;
+    int32_t *new_index, *n_pruned;
+    int32_t *work; // [nq][3][K]: the walk tables of chain_walk
+};
+
+constexpr int REPAIR_THREADS = 256;
+
+// Exclusive prefix count of `flag` over the CTA, and the CTA's total.  Every thread of the CTA calls it.
+__device__ __forceinline__ int block_count_before(bool flag, int &total, int *warp_count) {
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const unsigned b = __ballot_sync(0xffffffffu, flag);
+    if (lane == 0) warp_count[wid] = __popc(b);
+    __syncthreads();
+    int before = __popc(b & ((1u << lane) - 1u));
+    total = 0;
+    for (int w = 0; w < REPAIR_THREADS / 32; w++) {
+        const int c = warp_count[w];
+        before += w < wid ? c : 0;
+        total += c;
+    }
+    __syncthreads(); // warp_count is written again by the next call
+    return before;
+}
+
+// One query per CTA.  Keep pass: chain_walk with node 0 absorbing (next(0) = 0, bit 1) and every other node stepping to
+// its parent with bit edge_ok, or ending with bit 0 when its parent is outside [0, n) (-1 included): node i is kept
+// when its walk of n - 1 steps stands at node 0 with every bit 1, i.e. it reaches node 0 within n - 1 parent steps over
+// edges that edge_ok passes.  A kept node's parent walks a suffix of the same path, so the kept set is closed under
+// parent.  Compaction: new_index is the exclusive count of kept rows before each row (-1 for pruned rows and rows >= n),
+// in chunks of the CTA; then the rows move in place in increasing chunk order, each chunk read into registers before any
+// of it is written (new <= old, so a chunk's writes land on rows already read), with parents remapped through the
+// complete new_index.  The root leaves with parent -1 and u NaN, as rrt_setup plants it.
+__global__ void __launch_bounds__(REPAIR_THREADS) repair_tree_kernel(const RepairDev a) {
+    __shared__ int warp_count[REPAIR_THREADS / 32];
+    const int K = a.K;
+    for (int64_t q = blockIdx.x; q < a.nq; q += gridDim.x) {
+        int32_t *T0 = a.work + q * 3 * (int64_t)K, *T1 = T0 + K, *W = T1 + K;
+        const int64_t row0 = q * (int64_t)K;
+        const uint8_t *eok = a.edge_ok + row0;
+        int32_t *par = a.parent + row0, *nidx = a.new_index + row0;
+        double *nx = a.nx + row0, *ny = a.ny + row0, *nth = a.nth + row0, *u = a.u + 5 * row0;
+        const int n = min(max(a.n_nodes[q], 0), K);
+        for (int i = threadIdx.x; i < n; i += blockDim.x) {
+            const int p = par[i];
+            T0[i] = i == 0 ? 1 : (p >= 0 && p < n && eok[i] ? p * 2 | 1 : -2);
+            W[i] = i * 2 | 1;
+        }
+        __syncthreads();
+        chain_walk(T0, T1, W, n, n - 1);
+        int kept = 0;
+        for (int base = 0; base < n; base += REPAIR_THREADS) { // new_index
+            const int i = base + threadIdx.x;
+            const bool keep = i < n && W[i] == 1;
+            int total;
+            const int before = block_count_before(keep, total, warp_count);
+            if (i < n) nidx[i] = keep ? kept + before : -1;
+            kept += total;
+        }
+        for (int i = n + threadIdx.x; i < K; i += blockDim.x) nidx[i] = -1;
+        __syncthreads(); // new_index complete before any parent is remapped
+        for (int base = 0; base < n; base += REPAIR_THREADS) { // rows, in place
+            const int i = base + threadIdx.x;
+            const int ni = i < n ? nidx[i] : -1;
+            double x = 0, y = 0, th = 0, uu[5];
+            int p = -1;
+            if (ni >= 0) {
+                TRRT_CHECK(ni <= i && ni < kept && (i == 0 || nidx[i - 1] < 0 || nidx[i - 1] == ni - 1));
+                x = nx[i]; y = ny[i]; th = nth[i];
+                if (i == 0) {
+                    for (int j = 0; j < 5; j++) uu[j] = NAN;
+                } else {
+                    const int op = par[i];
+                    TRRT_CHECK(op >= 0 && op < n && nidx[op] >= 0); // closure: a kept node's parent is kept
+                    p = nidx[op];
+                    for (int j = 0; j < 5; j++) uu[j] = u[5 * i + j];
+                }
+            }
+            __syncthreads(); // the chunk is read before any of it is written
+            if (ni >= 0) {
+                nx[ni] = x; ny[ni] = y; nth[ni] = th; par[ni] = p;
+                for (int j = 0; j < 5; j++) u[5 * ni + j] = uu[j];
+            }
+        }
+        if (threadIdx.x == 0) {
+            const int s = a.sol[q];
+            const int ns = (s >= 0 && s < n) ? nidx[s] : -1;
+            if (ns < 0 && a.status[q] == TRRT_OK_FOUND) a.status[q] = a.iters[q] < K - 1 ? TRRT_PAUSED : TRRT_OK_NOT_FOUND;
+            a.sol[q] = ns;
+            a.n_nodes[q] = kept;
+            if (a.n_pruned) a.n_pruned[q] = n - kept;
+        }
+        __syncthreads(); // the next query of this CTA starts from a clean barrier
+    }
+}
+
+// Race keys after a repair (the launcher fills them with 0xff first): min over the members that still hold
+// TRRT_OK_FOUND of (iters << 32) | q, the key trrt_rrt_race_batch publishes.  Group ids outside [0, n_groups) race nobody.
+__global__ void repair_race_kernel(const int32_t *__restrict__ status, const int32_t *__restrict__ iters,
+                                   const int32_t *__restrict__ group, int64_t n_groups, unsigned long long *key, int64_t nq) {
+    for (int64_t q = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; q < nq; q += (int64_t)gridDim.x * blockDim.x) {
+        const int g = group[q];
+        if (status[q] == TRRT_OK_FOUND && g >= 0 && g < n_groups)
+            atomicMin(key + g, ((unsigned long long)iters[q] << 32) | (unsigned long long)q);
     }
 }
 

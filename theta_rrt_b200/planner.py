@@ -139,7 +139,9 @@ class RrtResult:
 @dataclass
 class RaceResult:
     """Planner.rrt_race output, per problem: winner (query index into result, -1 = no seed reached the goal),
-    winner_seed (int64, -1 = none) and iters (the winner's iterations, -1 = none); result holds every member."""
+    winner_seed (int64, -1 = none) and iters (the winner's iterations, -1 = none); result holds every member.
+    winner, winner_seed and iters are a snapshot of the planning call: Planner.repair_tree and rrt_resume update
+    result.race_key / race_winner / race_iters, not them."""
     result: RrtResult
     winner: torch.Tensor
     winner_seed: torch.Tensor
@@ -232,6 +234,22 @@ class TreeValidity:
 
     def host(self):
         return _host_dict(self)
+
+
+@dataclass
+class TreeRepair:
+    """Planner.repair_tree output: new_index int32 [q, K] (the new row of old row i; -1 for pruned rows and rows at or
+    past the old n_nodes), n_pruned int32 [q] (rows removed), reopened uint8 [q] (1 where an OK_FOUND query lost its
+    solution and became PAUSED) and the TreeValidity the repair followed."""
+    new_index: torch.Tensor
+    n_pruned: torch.Tensor
+    reopened: torch.Tensor
+    validity: TreeValidity
+
+    def host(self):
+        out = _host_dict(self)
+        out["validity"] = self.validity.host()
+        return out
 
 
 @dataclass
@@ -744,7 +762,7 @@ class Planner:
             out = TreeValidity(edge_ok=torch.empty((nq, K), dtype=torch.uint8, device=self.device),
                                node_ok=torch.empty((nq, K), dtype=torch.uint8, device=self.device),
                                sol_ok=torch.empty(nq, dtype=torch.int8, device=self.device))
-            work = self._scratch("validate_tree", self.lib.trrt_validate_tree_workspace_bytes(nq, K))
+            work = self._scratch("tree_walk", self.lib.trrt_validate_tree_workspace_bytes(nq, K))
             a = _lib.CValidateTreeArgs(d_bits=g.bits.data_ptr(), n_maps=g.n_maps, H=g.H, W=g.W,
                                        d_map_id=_ptr(res.launch.map_id), n_queries=nq, K=K, lanes=int(lanes),
                                        d_node_x=res.node_x.data_ptr(), d_node_y=res.node_y.data_ptr(),
@@ -753,6 +771,58 @@ class Planner:
                                        d_node_ok=out.node_ok.data_ptr(), d_sol_ok=out.sol_ok.data_ptr(),
                                        d_work=work.data_ptr(), work_bytes=work.numel())
             _lib.check(self.lib.trrt_validate_tree(C.byref(a), self._stream()), "trrt_validate_tree")
+        return out
+
+    def repair_tree(self, res: RrtResult, validity: TreeValidity | None = None, lanes=0) -> TreeRepair:
+        """Tree repair after a map edit (the pruning step of dynamic RRT replanning), in place on the current stream.
+        validity: validate_tree(res) on the map as it is now (computed here with `lanes` when None).  Per query, node 0
+        (the start) is kept with parent -1 and u NaN; node i >= 1 is kept when following parent from i reaches node 0
+        within n_nodes - 1 steps and every edge it follows passes edge_ok.  The kept rows keep their order (insertion
+        order, the nearest scan's tie-break) and are compacted, parents remapped; n_nodes becomes the kept count.  A
+        query whose solution node was pruned gets sol = -1 and, if it was OK_FOUND, becomes PAUSED (iters < K-1) or
+        OK_NOT_FOUND (no iterations left); iters is unchanged, so rrt_resume(res) then grows the reopened and paused
+        queries on the edited map with the rest of their sample streams.  A raced result gets each group's race_key
+        recomputed from the members still OK_FOUND (race_winner / race_iters decoded again).  Only the edge test of
+        validate_tree is followed: clearance rays and a node's own pixel are not tested again, and the tree is not
+        re-rooted.  Raises ValueError for a result without u, with per-iteration logs (they name old node indices), with
+        packed rows, planned on another grid, or a validity of other shapes."""
+        if res.u is None:
+            raise ValueError("repair_tree needs the edges' u: plan with want_u=True")
+        if res.it_near is not None:
+            raise ValueError("repair_tree does not remap per-iteration logs: plan without logs=True")
+        if res.launch is None or res.launch.grid is not self.grid:
+            raise ValueError("repair_tree repairs a result that Planner.rrt planned on this planner's grid")
+        if res.launch.packed:
+            raise ValueError("repair_tree does not repair packed rows: plan without pack=True")
+        nq, K = res.node_x.shape[0], res.K
+        if validity is not None and (tuple(validity.edge_ok.shape) != (nq, K) or tuple(validity.node_ok.shape) != (nq, K)
+                                     or tuple(validity.sol_ok.shape) != (nq,) or validity.edge_ok.dtype != torch.uint8):
+            raise ValueError(f"validity does not belong to a result of {nq} queries x K = {K}")
+        with torch.cuda.device(self.device):
+            if validity is None:
+                validity = self.validate_tree(res, lanes)
+            edge_ok = validity.edge_ok.to(self.device).contiguous()
+            before = res.status.clone()
+            out = TreeRepair(new_index=torch.empty((nq, K), dtype=torch.int32, device=self.device),
+                             n_pruned=torch.empty(nq, dtype=torch.int32, device=self.device), reopened=None,
+                             validity=validity)
+            # the walk tables of validate_tree, on the same stream: one workspace serves both calls
+            work = self._scratch("tree_walk", self.lib.trrt_repair_tree_workspace_bytes(nq, K))
+            race = res.launch.race
+            a = _lib.CRepairTreeArgs(n_queries=nq, K=K, d_node_x=res.node_x.data_ptr(), d_node_y=res.node_y.data_ptr(),
+                                     d_node_th=res.node_theta.data_ptr(), d_parent=res.parent.data_ptr(),
+                                     d_u=res.u.data_ptr(), d_n_nodes=res.n_nodes.data_ptr(), d_sol=res.sol.data_ptr(),
+                                     d_status=res.status.data_ptr(), d_iters=res.iters.data_ptr(),
+                                     d_edge_ok=edge_ok.data_ptr(), d_new_index=out.new_index.data_ptr(),
+                                     d_n_pruned=out.n_pruned.data_ptr(),
+                                     d_race_group=race[0].data_ptr() if race else None,
+                                     n_race_groups=race[1] if race else 0,
+                                     d_race_key=res.race_key.data_ptr() if race else None,
+                                     d_work=work.data_ptr(), work_bytes=work.numel())
+            _lib.check(self.lib.trrt_repair_tree(C.byref(a), self._stream()), "trrt_repair_tree")
+            if race:
+                res.race_winner, res.race_iters = race_decode(res.race_key)
+            out.reopened = ((before == 0) & (res.status == PAUSED)).to(torch.uint8)
         return out
 
     def validate_path(self, res, lanes=0) -> PathValidity:
